@@ -125,8 +125,10 @@ int zn_decode_verify_batch(zn_ctx* ctx, const uint8_t* blobs_base, const uint64_
  * For each slice i: digest_out[i] = BLAKE3(src), dst_base[dst_off[i] ..] = one frame of `codec` holding src.
  * dst_off has n+1 entries; capacity of slice i is dst_off[i+1]-dst_off[i] and must be >= zn_compress_bound().
  * `level` keeps the meaning of CompressCtx::new(level) (codec.rs:16): higher = more effort.  The zstd match finder
- * has three efforts (levels <= 2, 3..9, >= 10: window of 20 / 40 / 62 KiB); LZ4 has one.  The frame is always
- * decodable by stock libzstd / liblz4.
+ * has four efforts: levels <= 2, 3..9, 10..19 search a window of 20 / 40 / 62 KiB; levels >= 20 (the long effort) find
+ * matches anywhere in the slice up to 8 MiB back, through a candidate index sorted on the device, and take several
+ * times longer.  A match never reaches into another slice, and a frame depends only on its slice's bytes.  LZ4 has
+ * one effort.  The frame is always decodable by stock libzstd / liblz4.
  */
 int zn_compress_batch(zn_ctx* ctx, const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len,
                       uint32_t n, int level, int codec, uint8_t* dst_base, const uint64_t* dst_off,

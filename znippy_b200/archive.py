@@ -442,7 +442,8 @@ class StreamCompressor:
     def __init__(self, output: str, no_skip: bool, level: int = 19, codec_id: int = codec.CODEC_ZSTD,
                  ctx: Ctx | None = None, batch_bytes: int = 256 << 20, native_index: bool = True, native: bool = True,
                  envelope: bool = False):
-        """level defaults to the reference's compression_level = 19 (common_config.rs:37).  envelope=True (native
+        """level defaults to the reference's compression_level = 19 (common_config.rs:37); levels 20-22 select the
+        long effort of the zstd match finder (smaller frames, slower writes; codec.CompressCtx).  envelope=True (native
         writer only): blobs of compressed rows are ZNB1 envelopes, incompressible slices are stored raw inside them."""
         if envelope and not native:
             raise ValueError("the ZNB1 envelope is written by the native pipeline only")
@@ -614,7 +615,8 @@ def compress_dir(input_dir: str, output: str, no_skip: bool = False, level: int 
                  ctx: Ctx | None = None, envelope: bool = False, io_threads: int = 8, slot_bytes: int = 256 << 20) -> CompressionReport:
     """znippy-compress `compress_dir` (walk -> readers -> Magazine slots -> workers -> writer, slot_packer.rs:329-609) in
     one native call: `zn_archive_compress_dir` walks the directory, places every round in a pinned slot, lets
-    `io_threads` readers pread the bytes into place, and runs the same three-stage slot pipeline as compress_stream."""
+    `io_threads` readers pread the bytes into place, and runs the same three-stage slot pipeline as compress_stream.
+    `level` as in compress_stream: 19 by default, 20-22 for the long effort."""
     import ctypes as C
 
     from . import _native as N

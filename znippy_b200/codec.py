@@ -157,7 +157,8 @@ def blake3_hash(data, ctx: Ctx | None = None) -> bytes:
 
 class CompressCtx:
     """codec.rs:8-55.  `level` follows the reference's meaning (higher = more effort); the GPU match finder has
-    three effort settings (window geometries), so levels <= 2, 3..9 and >= 10 map onto them (DESIGN.md §4.3)."""
+    four efforts: three window geometries for levels <= 2, 3..9 and 10..19, and for levels >= 20 (zstd only) the long
+    effort, whose matches reach back anywhere in the slice up to 8 MiB (DESIGN.md §4.3)."""
 
     def __init__(self, compression_level: int, codec: int = CODEC_ZSTD, ctx: Ctx | None = None, envelope: bool = False):
         self.level = int(compression_level)

@@ -382,7 +382,7 @@ struct FseCState {
   ZN_HD void flush(BitWriter& bw, const FseCTable* ct) { bw.add(value, ct->log); }
 };
 
-// packed sequence: ll | ml << 20 | off << 40 (each < 2^20)
+// packed sequence: ll | ml << 20 | off << 40 (ll, ml < 2^20; off < 2^24: the long effort reaches back 8 MiB)
 ZN_HD uint64_t seq_pack(uint32_t ll, uint32_t ml, uint32_t off) { return (uint64_t)ll | ((uint64_t)ml << 20) | ((uint64_t)off << 40); }
 
 // ---- FSE table description (RFC 8878 §4.1.1): the writer mirroring fse_read_ncount of the decoder.
@@ -470,12 +470,14 @@ struct SeqScratch {
   uint32_t sbits[3][32];   // per chunk: FSE state bits of each sequence, value << 8 | count
   int32_t dnb[3][32];      // per chunk: delta_nb / delta_state of each sequence's three codes, fetched by the lanes so
   int32_t dst[3][32];      //            that the serial state chains only wait for the state table itself
-  uint32_t bitbuf[88];     // per chunk: the assembled bitstream (<= 31 carried bits + 32 x 75)
+  uint32_t bitbuf[88];     // per chunk: the assembled bitstream (<= 31 carried bits + 32 x 81: state bits 9 + 8 + 9,
+                           // extra bits 16 + 16 + 23 for an offset value < 2^24), 2 623 of 2 816 bits
 };
 
-// packed sequence after pass 1: ll:17 | ml - 4:17 | offset value:18 | ll code:6 | ml code:6   (ml is 4 .. 131072)
-ZN_HD uint64_t seq_pack2(uint32_t ll, uint32_t ml, uint32_t ofv, uint32_t lc, uint32_t mc) {
-  return (uint64_t)ll | ((uint64_t)(ml - 4u) << 17) | ((uint64_t)ofv << 34) | ((uint64_t)lc << 52) | ((uint64_t)mc << 58);
+// packed sequence after pass 1: ll:17 | ml - 4:17 | offset value:24 | ll code:6   (ml is 4 .. 131072; the ml code is
+// recomputed in pass 2, which leaves room for offset values up to 8 MiB + 3)
+ZN_HD uint64_t seq_pack2(uint32_t ll, uint32_t ml, uint32_t ofv, uint32_t lc) {
+  return (uint64_t)ll | ((uint64_t)(ml - 4u) << 17) | ((uint64_t)ofv << 34) | ((uint64_t)lc << 58);
 }
 
 // Sequences section, called by the whole warp.  Offsets become repeat codes where the history written by THIS block
@@ -537,7 +539,7 @@ ZN_HD uint32_t zstd_encode_sequences(const Warp& w, uint8_t* dst, uint64_t* seqs
     }
     if (k < nseq) {
       const uint32_t lc = len_code(ll, zs::kLLBase, zs::kLLBits, 16, 36), mc = len_code(ml, zs::kMLBase, zs::kMLBits, 32, 53);
-      seqs[k] = seq_pack2(ll, ml, v, lc, mc);
+      seqs[k] = seq_pack2(ll, ml, v, lc);
       w_count(&sc->cnt[0][lc]);
       w_count(&sc->cnt[1][hibit32(v)]);
       w_count(&sc->cnt[2][mc]);
@@ -601,8 +603,8 @@ ZN_HD uint32_t zstd_encode_sequences(const Warp& w, uint8_t* dst, uint64_t* seqs
     const uint32_t here = nseq - base < w.n ? nseq - base : w.n;
     const bool mine = w.lane < here;
     const uint64_t sj = mine ? seqs[base + (here - 1u - w.lane)] : 0ull;  // lane i takes the i-th sequence in coding order
-    const uint32_t ll = (uint32_t)(sj & 0x1FFFF), ml = 4u + (uint32_t)((sj >> 17) & 0x1FFFF), ofv = (uint32_t)((sj >> 34) & 0x3FFFF);
-    const uint32_t lc = (uint32_t)((sj >> 52) & 63), mc = (uint32_t)(sj >> 58);
+    const uint32_t ll = (uint32_t)(sj & 0x1FFFF), ml = 4u + (uint32_t)((sj >> 17) & 0x1FFFF), ofv = (uint32_t)((sj >> 34) & 0xFFFFFF);
+    const uint32_t lc = (uint32_t)(sj >> 58), mc = len_code(ml, zs::kMLBase, zs::kMLBits, 32, 53);
     const uint32_t oc = mine ? (uint32_t)hibit32(ofv) : 0u;
     if (mine) {
       sc->dnb[0][w.lane] = ct[0]->delta_nb[lc]; sc->dst[0][w.lane] = ct[0]->delta_state[lc];
@@ -919,6 +921,48 @@ ZN_HD uint32_t zstd_huf_literals(const Warp& w, const uint8_t* lit, uint32_t nli
   return hdr + comp;
 }
 
+// ------------------------------------------------------------------------------------------------- zstd block payload
+// Literals + sequences sections of one compressed block, whole warp: the block's nlit literals sit at stage + 3 and
+// its nseq sequences in seqs (seq_pack).  scratch = shared memory of >= kPayloadScratch bytes (Huffman tables, then
+// SeqScratch).  Huffman-compressed literals go to region B when that pays, raw literals stay in place (region A).
+// Returns the payload size (the payload starts at stage + *payload_off), or 0 when the block should be stored raw.
+constexpr uint32_t kPayloadScratch = 10240;
+static_assert(sizeof(SeqScratch) <= kPayloadScratch, "SeqScratch outgrew the payload scratch");
+
+ZN_HD uint32_t zstd_block_payload(const Warp& w, uint8_t* stage, uint32_t nlit, uint64_t* seqs, uint32_t nseq, uint32_t n,
+                                  uint32_t* scratch, uint32_t* payload_off) {
+  uint8_t* lit = stage + 3;
+  uint8_t* regB = stage + kZstdHalf;
+  const uint32_t hsz = zstd_huf_literals(w, lit, nlit, regB, scratch);
+  if (hsz) {
+    uint32_t total = 0;
+    if (hsz + 16u < n) {
+      const uint32_t ss = zstd_encode_sequences(w, regB + hsz, seqs, nseq, n - hsz - 16u, reinterpret_cast<SeqScratch*>(scratch));
+      if (ss) total = hsz + ss;
+    }
+    w_sync(w);
+    *payload_off = kZstdHalf;
+    return (total && total < n) ? total : 0u;
+  }
+  // literals section header (raw literals), placed right before the literal bytes
+  const uint32_t hs = nlit < 32 ? 1u : (nlit < 4096 ? 2u : 3u);
+  uint8_t* hp = stage + 3 - hs;
+  uint32_t total = 0;
+  if (w.lane == 0) {
+    if (hs == 1) hp[0] = (uint8_t)(nlit << 3);
+    else if (hs == 2) { hp[0] = (uint8_t)(0x04 | ((nlit & 0xF) << 4)); hp[1] = (uint8_t)(nlit >> 4); }
+    else { hp[0] = (uint8_t)(0x0C | ((nlit & 0xF) << 4)); hp[1] = (uint8_t)(nlit >> 4); hp[2] = (uint8_t)(nlit >> 12); }
+  }
+  // the block must beat its raw form, which also keeps the section inside the slot
+  if (hs + nlit + 16u < n) {
+    const uint32_t ss = zstd_encode_sequences(w, lit + nlit, seqs, nseq, n - (hs + nlit) - 16u, reinterpret_cast<SeqScratch*>(scratch));
+    if (ss) total = hs + nlit + ss;
+  }
+  w_sync(w);
+  *payload_off = 3 - hs;
+  return (total && total < n) ? total : 0u;
+}
+
 // ------------------------------------------------------------------------------------------------- zstd block
 // Compresses slice[bstart .. bstart+n) (n <= 128 KiB) into the payload of one compressed block.
 //   stage   kZstdSlot bytes: literals are written from stage+3, the block payload ends up at stage + *payload_off
@@ -1092,39 +1136,176 @@ ZN_HD uint32_t zstd_compress_block(const Warp& w, const uint8_t* slice, uint32_t
   nlit += rest;
   w_sync(w);
   if (nseq == 0) return 0;  // nothing found: raw block
-  // Huffman-compressed literals into region B when that pays; otherwise raw literals in place (region A)
-  uint8_t* regB = stage + kZstdHalf;
   ZN_CP(6);
-  const uint32_t hsz = zstd_huf_literals(w, lit, nlit, regB, tabw);
-  ZN_CP(7);
-  if (hsz) {
-    uint32_t total = 0;
-    if (hsz + 16u < n) {
-      const uint32_t ss = zstd_encode_sequences(w, regB + hsz, seqs, nseq, n - hsz - 16u, reinterpret_cast<SeqScratch*>(tabw));
-      if (ss) total = hsz + ss;
+  const uint32_t total = zstd_block_payload(w, stage, nlit, seqs, nseq, n, tabw, payload_off);
+  ZN_CP(8);
+  return total;
+}
+
+// ------------------------------------------------------------------------------------------------- zstd long effort
+// Levels >= 20.  The match finder sees the whole slice (up to kLongReach back) through a candidate index built per
+// round of slices:
+//   * every position q of a round (the round's units laid back to back) gets the key bucket << kLongPosBits | q,
+//     bucket = a hash of the kLongK bytes at q; a radix sort of the keys puts the earlier positions with q's bucket
+//     right before q, nearest first, and rank[q] says where q landed;
+//   * a unit is the part of a slice one index covers: slices are parsed in pieces of kLongPiece bytes, each indexed
+//     together with the kLongReach bytes before it, so a round holds whole units and no key reaches another slice;
+//   * one warp parses each 128 KiB block: the best of the kLongD nearest candidates of a position (probes capped at
+//     kLongProbe bytes), the last offset as a repeat candidate, and a two-step lazy rule (zstd's lazy2 gains).
+// The best match of a position depends only on the slice's bytes, and the parse itself is serial code every lane
+// runs alike, so the sequences do not depend on the lane count: the host emulation (one lane) emits the GPU's bytes.
+constexpr uint32_t kLongReach = 8u << 20;                   // largest offset (the reference's slice, libzstd-19's window)
+constexpr uint32_t kLongPiece = 8u << 20;                   // slice bytes parsed per unit (a multiple of kZstdCBlock)
+constexpr uint32_t kLongPosBits = 27;                       // positions per round < 2^27 (units are <= 16 MiB)
+constexpr uint32_t kLongRound = 1u << kLongPosBits;
+constexpr uint32_t kLongHashBits = 29;
+constexpr uint32_t kLongKeyBits = kLongPosBits + kLongHashBits;  // key bits the sort orders
+#ifndef ZN_LONG_K
+#define ZN_LONG_K 5
+#define ZN_LONG_D 16
+#endif
+constexpr uint32_t kLongK = ZN_LONG_K;                      // bytes hashed into a bucket (4 .. 8)
+constexpr uint32_t kLongD = ZN_LONG_D;                      // candidates probed per position
+constexpr uint32_t kLongProbe = 256;                        // bytes a probe measures; a chosen match is extended beyond
+constexpr uint32_t kLongBatch = kOnDevice ? 32u : 4u;       // positions evaluated together (one per lane on the device)
+static_assert(kLongPiece % kZstdCBlock == 0 && kLongK >= 4 && kLongK <= 8, "long effort geometry");
+
+// Slice positions [lo, hi) of a unit occupy round positions [q0, q0 + hi - lo).
+struct LongIndex {
+  const uint64_t* sk;    // the round's keys, sorted
+  const uint32_t* rank;  // rank[q]: index of q's key in sk
+  uint32_t q0, lo;
+};
+
+ZN_HD uint64_t long_key(const uint8_t* slice, uint32_t pos, uint32_t hi, uint32_t q) {
+  uint64_t b = (1ull << kLongHashBits) - 1u;  // the last kLongK - 1 positions share one bucket (matches are verified)
+  if (hi - pos >= kLongK) {
+    uint64_t v = 0;
+    for (uint32_t i = 0; i < kLongK; i++) v |= (uint64_t)slice[pos + i] << (8u * i);
+    b = (v * 0x9E3779B185EBCA87ull) >> (64u - kLongHashBits);
+  }
+  return (b << kLongPosBits) | q;
+}
+
+// unaligned little-endian 32-bit load that touches only the aligned words holding p[0..4)
+ZN_HD uint32_t ld32g(const uint8_t* p) {
+#if defined(__CUDA_ARCH__)
+  const uint32_t* w = reinterpret_cast<const uint32_t*>(reinterpret_cast<uintptr_t>(p) & ~(uintptr_t)3);
+  const uint32_t sh = ((uint32_t)reinterpret_cast<uintptr_t>(p) & 3u) * 8u;
+  return sh ? __funnelshift_r(w[0], w[1], sh) : w[0];
+#else
+  return ld32le(p);
+#endif
+}
+
+// common prefix length of a[0..lim) and b[0..lim), one lane
+ZN_HD uint32_t long_prefix(const uint8_t* a, const uint8_t* b, uint32_t lim) {
+  uint32_t n = 0;
+  for (; n + 4u <= lim; n += 4u) {
+    const uint32_t x = ld32g(a + n) ^ ld32g(b + n);
+    if (x) return n + ((ffs32(x) - 1u) >> 3);
+  }
+  while (n < lim && a[n] == b[n]) n++;
+  return n;
+}
+
+// Longest match for slice position p among its kLongD nearest candidates, measured up to min(kLongProbe, end - p);
+// the nearest candidate wins a tie.  *len = 0 when no candidate matches at all.
+ZN_HD void long_best(const uint8_t* s, const LongIndex& ix, uint32_t p, uint32_t end, uint32_t* len, uint32_t* off) {
+  const uint32_t i = ix.rank[ix.q0 + (p - ix.lo)];
+  const uint64_t bucket = ix.sk[i] >> kLongPosBits;
+  const uint32_t lim = end - p < kLongProbe ? end - p : kLongProbe;
+  uint32_t bl = 0, bo = 0;
+  for (uint32_t d = 1; d <= kLongD && d <= i; d++) {
+    const uint64_t k = ix.sk[i - d];
+    const uint32_t cq = (uint32_t)k & (kLongRound - 1u);
+    if ((k >> kLongPosBits) != bucket || cq < ix.q0) break;  // bucket or unit exhausted
+    const uint32_t c = cq - ix.q0 + ix.lo;
+    if (p - c > kLongReach) break;
+    if (s[c + bl] != s[p + bl]) continue;  // cannot beat the best so far
+    const uint32_t l = long_prefix(s + p, s + c, lim);
+    if (l > bl) {
+      bl = l;
+      bo = p - c;
+      if (l == lim) break;
     }
-    w_sync(w);
-    ZN_CP(8);
-    *payload_off = kZstdHalf;
-    return (total && total < n) ? total : 0u;
   }
-  // literals section header (raw literals), placed right before the literal bytes
-  const uint32_t hs = nlit < 32 ? 1u : (nlit < 4096 ? 2u : 3u);
-  uint8_t* hp = stage + 3 - hs;
-  uint32_t total = 0;
-  if (w.lane == 0) {
-    if (hs == 1) hp[0] = (uint8_t)(nlit << 3);
-    else if (hs == 2) { hp[0] = (uint8_t)(0x04 | ((nlit & 0xF) << 4)); hp[1] = (uint8_t)(nlit >> 4); }
-    else { hp[0] = (uint8_t)(0x0C | ((nlit & 0xF) << 4)); hp[1] = (uint8_t)(nlit >> 4); hp[2] = (uint8_t)(nlit >> 12); }
+  *len = bl;
+  *off = bo;
+}
+
+// lazy2's gain of a match: 4 per byte minus the bits of its offset value (a repeat of the last offset codes as 1)
+ZN_HD int32_t long_gain(uint32_t ml, uint32_t off, uint32_t rep) {
+  return 4 * (int32_t)ml - (int32_t)hibit32(off == rep ? 1u : off + 3u);
+}
+
+// Compresses slice s[bstart .. bstart+n) (n <= 128 KiB) into the payload of one compressed block, whole warp.
+//   ix       the candidate index of the unit holding the block
+//   stage    kZstdSlot bytes: literals are written from stage+3, the payload ends up at stage + *payload_off
+//   seqs     kZstdMaxSeq packed sequences (global scratch)
+//   bl, bo   kLongBatch words each (shared memory): match length / offset of the positions being evaluated
+//   scratch  kPayloadScratch bytes of shared memory for the entropy stages
+// Returns the payload size, or 0 when the block should be stored raw.
+ZN_HD uint32_t zstd_long_block(const Warp& w, const uint8_t* s, const LongIndex& ix, uint32_t bstart, uint32_t n,
+                               uint8_t* stage, uint64_t* seqs, uint32_t* bl, uint32_t* bo, uint32_t* scratch,
+                               uint32_t* payload_off) {
+  const uint32_t bend = bstart + n;
+  uint8_t* lit = stage + 3;
+  uint32_t nlit = 0, nseq = 0, anchor = bstart, pos = bstart, rep = 0;
+  uint32_t base = bend;  // first position of the evaluated batch (none yet)
+  // best match at p: the index's candidates, then the last offset of this block as a repeat candidate
+  auto best = [&](uint32_t p, uint32_t* ml, uint32_t* off) {
+    if (p - base >= kLongBatch) {
+      w_sync(w);
+      for (uint32_t i = w.lane; i < kLongBatch; i += w.n) {
+        uint32_t l = 0, o = 0;
+        if (p + i + 4u <= bend) long_best(s, ix, p + i, bend, &l, &o);
+        bl[i] = l;
+        bo[i] = o;
+      }
+      w_sync(w);
+      base = p;
+    }
+    *ml = bl[p - base];
+    *off = bo[p - base];
+    if (rep && rep <= p) {
+      const uint32_t lim = bend - p < kLongProbe ? bend - p : kLongProbe;
+      const uint32_t rl = long_prefix(s + p, s + p - rep, lim);
+      if (rl >= 4u && (*ml < 4u || long_gain(rl, rep, rep) >= long_gain(*ml, *off, rep))) { *ml = rl; *off = rep; }
+    }
+  };
+  while (pos + 4u <= bend) {
+    uint32_t ml, off;
+    best(pos, &ml, &off);
+    if (ml < 4u) { pos++; continue; }
+    uint32_t start = pos;
+    for (uint32_t ip = pos;;) {  // lazy2: a later start wins when it gains 4 (one step on) or 7 (two steps on) more
+      bool moved = false;
+      for (uint32_t step = 1; step <= 2 && ip + 1u + 4u <= bend; step++) {
+        ip++;
+        uint32_t ml2, off2;
+        best(ip, &ml2, &off2);
+        if (ml2 >= 4u && long_gain(ml2, off2, rep) > long_gain(ml, off, rep) + (step == 1 ? 4 : 7)) {
+          ml = ml2; off = off2; start = ip;
+          moved = true;
+          break;
+        }
+      }
+      if (!moved) break;
+    }
+    if (ml == kLongProbe && start + ml < bend) ml += match_extend(w, s + start + ml, s + start - off + ml, bend - (start + ml));
+    w_copy(w, lit + nlit, s + anchor, start - anchor);
+    if (w.lane == 0) seqs[nseq] = seq_pack(start - anchor, ml, off);
+    nlit += start - anchor;
+    nseq++;
+    rep = off;
+    pos = anchor = start + ml;
   }
-  // the block must beat its raw form, which also keeps the section inside the slot
-  if (hs + nlit + 16u < n) {
-    const uint32_t ss = zstd_encode_sequences(w, lit + nlit, seqs, nseq, n - (hs + nlit) - 16u, reinterpret_cast<SeqScratch*>(tabw));
-    if (ss) total = hs + nlit + ss;
-  }
+  w_copy(w, lit + nlit, s + anchor, bend - anchor);
+  nlit += bend - anchor;
   w_sync(w);
-  *payload_off = 3 - hs;
-  return (total && total < n) ? total : 0u;
+  if (nseq == 0) return 0;
+  return zstd_block_payload(w, stage, nlit, seqs, nseq, n, scratch, payload_off);
 }
 
 // Zstandard frame header: single segment, 8-byte content size (13 bytes); empty content uses the 1-byte form.

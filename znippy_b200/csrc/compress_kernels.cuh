@@ -108,6 +108,62 @@ __global__ void __launch_bounds__(32) k_zstd_blocks(const SliceDesc* __restrict_
   }
 }
 
+// ---- zstd long effort (levels >= 20): candidate index per round of units, then one warp per 128 KiB block
+// A unit: slice positions [lo, hi) indexed, [parse_lo, hi) parsed (cz::zstd_long_block); q0 = round position of lo.
+struct LongUnit {
+  uint64_t src_off;    // slice start in the source
+  uint32_t lo, parse_lo, hi, q0;
+  uint32_t blk_first;  // global block index of the block at parse_lo
+};
+constexpr int kLongCtasPerSm = 8;  // one warp per CTA; bounds the per-CTA sequence scratch
+
+// keys[q] for every position q < n_pos of the round (units ascending in q0)
+__global__ void __launch_bounds__(256) k_long_keys(const LongUnit* __restrict__ units, uint32_t n_units, uint32_t n_pos,
+                                                   const uint8_t* __restrict__ src_base, uint64_t* keys) {
+  for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < n_pos; q += gridDim.x * blockDim.x) {
+    uint32_t lo = 0, hi = n_units;
+    while (hi - lo > 1) {
+      const uint32_t mid = (lo + hi) >> 1;
+      if (units[mid].q0 <= q) lo = mid; else hi = mid;
+    }
+    const LongUnit u = units[lo];
+    keys[q] = cz::long_key(src_base + u.src_off, u.lo + (q - u.q0), u.hi, q);
+  }
+}
+
+// rank[q] = where q's key landed in the sorted order
+__global__ void __launch_bounds__(256) k_long_rank(const uint64_t* __restrict__ sk, uint32_t n_pos, uint32_t* rank) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pos; i += gridDim.x * blockDim.x)
+    rank[(uint32_t)sk[i] & (cz::kLongRound - 1u)] = i;
+}
+
+// blocks [blk0, blk0 + n_blk) of the round (its units ascending in blk_first); meta as k_zstd_blocks writes it
+__global__ void __launch_bounds__(32) k_long_blocks(const LongUnit* __restrict__ units, uint32_t n_units, uint32_t blk0,
+                                                    uint32_t n_blk, const uint8_t* __restrict__ src_base,
+                                                    const uint64_t* __restrict__ sk, const uint32_t* __restrict__ rank,
+                                                    uint8_t* tmp, uint64_t* seq_scratch, uint32_t* meta) {
+  __shared__ __align__(16) uint32_t scratch[cz::kPayloadScratch / 4];
+  __shared__ uint32_t bl[cz::kLongBatch], bo[cz::kLongBatch];
+  const cz::Warp w{threadIdx.x, 32u};
+  uint64_t* seqs = seq_scratch + (size_t)blockIdx.x * cz::kZstdMaxSeq;
+  for (uint32_t j = blk0 + blockIdx.x; j < blk0 + n_blk; j += gridDim.x) {
+    uint32_t lo = 0, hi = n_units;
+    while (hi - lo > 1) {
+      const uint32_t mid = (lo + hi) >> 1;
+      if (units[mid].blk_first <= j) lo = mid; else hi = mid;
+    }
+    const LongUnit u = units[lo];
+    const uint32_t bstart = u.parse_lo + (j - u.blk_first) * cz::kZstdCBlock;
+    const uint32_t n = u.hi - bstart < cz::kZstdCBlock ? u.hi - bstart : cz::kZstdCBlock;
+    const cz::LongIndex ix{sk, rank, u.q0, u.lo};
+    uint32_t poff = 0;
+    const uint32_t c = cz::zstd_long_block(w, src_base + u.src_off, ix, bstart, n, tmp + (size_t)j * cz::kZstdSlot, seqs, bl, bo,
+                                           scratch, &poff);
+    if (w.lane == 0) { meta[2 * j] = poff; meta[2 * j + 1] = c; }
+    __syncwarp();
+  }
+}
+
 __global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
                                                        const uint8_t* tmp, const uint32_t* __restrict__ meta, uint8_t* dst_base,
                                                        uint64_t* dst_len) {

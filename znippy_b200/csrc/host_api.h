@@ -20,17 +20,33 @@ struct CompressScratch {
   size_t seqs_cap = 0;
   void* small = nullptr;  // slices + meta + dst_len
   size_t small_cap = 0;
+  // long effort (levels >= 20): units of the batch, the round's keys (sorted in place between the two buffers; the
+  // buffer the sort leaves free holds the rank array) and the sort's temporary storage
+  void* lunits = nullptr;
+  size_t lunits_cap = 0;
+  uint64_t* lkeys0 = nullptr;
+  size_t lkeys0_cap = 0;
+  uint64_t* lkeys1 = nullptr;
+  size_t lkeys1_cap = 0;
+  void* lsort = nullptr;
+  size_t lsort_cap = 0;
   cudaEvent_t ev[2] = {nullptr, nullptr};
   float last_ms = 0.f;  // device time of the kernels of the last compress_run
   void release() {
     if (tmp) cudaFree(tmp);
     if (seqs) cudaFree(seqs);
     if (small) cudaFree(small);
+    if (lunits) cudaFree(lunits);
+    if (lkeys0) cudaFree(lkeys0);
+    if (lkeys1) cudaFree(lkeys1);
+    if (lsort) cudaFree(lsort);
     if (ev[0]) cudaEventDestroy(ev[0]);
     if (ev[1]) cudaEventDestroy(ev[1]);
     ev[0] = ev[1] = nullptr;
     tmp = nullptr; seqs = nullptr; small = nullptr;
     tmp_cap = seqs_cap = small_cap = 0;
+    lunits = nullptr; lkeys0 = nullptr; lkeys1 = nullptr; lsort = nullptr;
+    lunits_cap = lkeys0_cap = lkeys1_cap = lsort_cap = 0;
   }
 };
 void compress_init_attrs();
