@@ -296,7 +296,7 @@ int zn_plan_pipeline_fallbacks(zn_plan* plan, uint32_t* rows);
 uint32_t zn_plan_launches(const zn_plan* plan);
 /* 1 when the plan decodes and hashes in ONE kernel (batches of large, highly compressible blobs: decode warps feed
  * hash warps through a device-wide tile queue, fused_ws.cuh); the decode stage of zn_plan_last_ms then covers both
- * and the hash stage is empty.  Environment: ZN_FUSE=0 keeps the two kernels apart. */
+ * and the hash stage is empty. */
 int zn_plan_fused(const zn_plan* plan);
 /* device time of the most recent completed run, per stage, in ms (CUDA events on the run's stream):
  * [0] total, [1] decode stage, [2] hash stage (chunks), [3] tree+compare stage.  Synchronises. */

@@ -310,14 +310,12 @@ def test_block_parallel_mixed_batch_with_small_sources(codec, oracle):
         assert out[out_off[i]:out_off[i] + len(c)].tobytes() == c, i
 
 
-@pytest.mark.parametrize("mode", ["ws", "team", "0"])
+@pytest.mark.parametrize("mode", ["ws"])
 def test_fused_decode_hash_kernels(codec, oracle, mode, monkeypatch):
-    """Large, highly compressible blobs through the fused decode+hash kernels (ZN_FUSE: `ws` = warp-specialised K4w, the
-    default; `team` = the interleaved K4; `0` = decode and hash as two kernels): same bytes, same digests, same status
-    rules on all three; a small grid makes every decode team take several blobs."""
+    """Large, highly compressible blobs through the fused decode+hash kernel (`ws` = warp-specialised, k_decode_ws): same
+    bytes, same digests, same status rules as the oracle; a small grid makes every decode team take several blobs."""
     O = oracle
     z, l = O.libzstd(), O.liblz4()
-    monkeypatch.setenv("ZN_FUSE", mode)
     monkeypatch.setenv("ZN_WS_GRID", "3")
     datas = [O.gen_text(8 << 20), O.gen_binary(8 << 20), O.gen_text((1 << 20) + 17), O.gen_binary(700_000),
              np.zeros(3 << 20, np.uint8), O.gen_text(5_000_001), O.gen_binary((4 << 20) - 1), O.gen_text(2 << 20),
@@ -584,3 +582,53 @@ def test_entropy_coded_slices_at_baseline_size(codec, oracle):
     out = d_out.cpu().numpy()
     for k, c in enumerate(contents):
         assert (out[k * (8 << 20): (k + 1) * (8 << 20)] == c).all(), k
+
+
+def test_pipeline_one_pass_sequence_stage(codec, oracle):
+    """Batches of very many small entropy-coded rows take the one-pass sequence stage (k_zseq_g): more blocks than two
+    rounds of phase-1 lanes (2 x SMs x kSeq1Lanes, kSeq1Lanes = 56) and a mean decoded size below 256 KiB.  Real-text rows
+    of 4-12 KiB at levels 1 / 3 / 19: every status, byte and digest equals the oracle's, no row is handed back, and the run
+    launches one kernel less than a 64-row slice of the same rows, which takes the two-phase form (k_zseq1 + k_zseq2)."""
+    import torch
+    from znippy_b200 import Plan
+    O, z = oracle, oracle.libzstd()
+    ctx = codec.default_ctx()
+    n = 2 * torch.cuda.get_device_properties(0).multi_processor_count * 56 + 512
+    rng = np.random.default_rng(17)
+    rt = O.real_text(8 << 20)
+    lens = rng.integers(4096, 12289, n)
+    starts = rng.integers(0, rt.size - 12288, n)
+    contents = [rt[s:s + k].tobytes() for s, k in zip(starts, lens)]
+    blobs = [z.compress(c, (1, 3, 19)[i % 3]) for i, c in enumerate(contents)]
+    offs, cur = [], 0
+    for k, b in enumerate(blobs):
+        cur = (cur + 15) // 16 * 16 + k % 16
+        offs.append(cur)
+        cur += len(b)
+    buf = np.zeros(cur + 16, np.uint8)
+    for o, b in zip(offs, blobs):
+        buf[o:o + len(b)] = np.frombuffer(b, np.uint8)
+    out_len = np.array([len(c) for c in contents], np.uint64)
+    out_off = np.concatenate([[0], np.cumsum((out_len + np.uint64(15)) & ~np.uint64(15))])[:-1].astype(np.uint64)
+    digs = np.frombuffer(b"".join(O.blake3(c) for c in contents), np.uint8)
+    d_in = torch.from_numpy(buf).cuda()
+    d_out = torch.zeros(int(out_off[-1] + out_len[-1]) + 256, dtype=torch.uint8, device="cuda")
+    stream = torch.cuda.current_stream().cuda_stream
+
+    def run(m):
+        plan = Plan.decode_verify(ctx, offs[:m], [len(b) for b in blobs[:m]], [1] * m, out_off[:m], out_len[:m], digs[:m * 32])
+        assert plan.class_counts()[0] == m
+        plan.run(d_in.data_ptr(), d_out.data_ptr(), stream)
+        torch.cuda.synchronize()
+        st, dg = plan.results()
+        assert st.tolist() == [0] * m
+        assert plan.pipeline_fallbacks() == 0
+        assert (dg.reshape(-1) == digs[:m * 32]).all()
+        return plan.launches()
+
+    two_phase = run(64)
+    one_pass = run(n)
+    assert one_pass == two_phase - 1
+    out = d_out.cpu().numpy()
+    for i, c in enumerate(contents):
+        assert out[int(out_off[i]): int(out_off[i]) + len(c)].tobytes() == c, i

@@ -73,7 +73,7 @@ int main(int argc, char** argv) {
 #ifdef TRACE_PAR
     par::k_decode_par<<<nb, par::kParThreads, sizeof(par::ParShared)>>>(d_desc, d_list, nb, d_in, d_out, d_par, d_status, d_prod, d_ctr);
 #else
-    k_decode<TRACE_NT, TRACE_KB, false><<<(nb + TRACE_KB - 1) / TRACE_KB, TRACE_NT>>>(d_desc, d_list, nb, d_in, d_out, d_lit, d_status, d_prod, d_ctr, nullptr, 1u, nullptr, 0u);
+    k_decode<TRACE_NT, TRACE_KB><<<(nb + TRACE_KB - 1) / TRACE_KB, TRACE_NT>>>(d_desc, d_list, nb, d_in, d_out, d_lit, d_status, d_prod, d_ctr, nullptr, 1u, nullptr, 0u);
 #endif
     cudaEventRecord(e1);
     cudaDeviceSynchronize();

@@ -2,7 +2,6 @@
 -DZN_WS_DEBUG copied over znippy_b200/libznippy_cuda.so (tools/bin/variants/lib_wsdebug.so)."""
 import ctypes as C, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-os.environ["ZN_FUSE"] = "ws"
 import numpy as np, torch
 import bench
 from znippy_b200 import Ctx, Plan, _native as N

@@ -3,7 +3,6 @@
 // Replaces the codec call of the reference's read loop (znippy-common/src/decompress.rs:156-166) and of
 // ZnippyArchive::extract_file (archive.rs:159-164) for a whole batch of index rows at once.
 #pragma once
-#include "blake3_kernels.cuh"
 #include "lz4_decode.cuh"
 
 namespace zn {
@@ -18,55 +17,16 @@ ZN_D void warp_stage(uint8_t* dst, const uint8_t* src, uint32_t n, uint32_t lane
   for (uint32_t i = lane; i < n; i += 32) dst[i] = __ldg(src + i);
 }
 
-// K4: decode -> blake3 fusion for large blobs.  The decoding team hashes the chunks of its own output as soon as
-// they are final (below the visibility watermark), in tiles of 32 chunks per warp, while the bulk stores of the
-// following block are still draining: the HBM-bound decode and the ALU-bound hash of different blocks (and of the two
-// CTAs sharing an SM) overlap inside one kernel, with no second pass over the output from HBM.
-struct HashHook {
-  uint8_t* stage;      // nwarps x kB3SmemPerWarp bytes of shared memory
-  const uint8_t* out;  // the blob's output
-  uint32_t* cvs;       // the blob's chaining-value slots
-  uint32_t cap, n_chunks, done, one;
-
-  ZN_D void hash_range(const Team& t, uint32_t c_lo, uint32_t c_hi) {
-    const uint32_t warp = t.tid >> 5, lane = t.tid & 31u, nw = t.n >> 5;
-    for (uint32_t tile = c_lo + warp * 32u; tile < c_hi; tile += nw * 32u) {
-      const uint32_t g = tile + lane;
-      const bool act = g < c_hi;
-      const uint32_t rem = act ? cap - min(cap, g * kChunk) : 0u;
-      uint32_t cv[8];
-      b3_warp_tile(stage + warp * kB3SmemPerWarp, out + (size_t)g * kChunk, rem < kChunk ? rem : kChunk, g, n_chunks == 1, act,
-                   lane, one, cv);
-      if (act) b3::store_cv(cvs + (size_t)g * 8, cv);
-    }
-  }
-  ZN_D void after_block(const Team& t, zs::ExecState& es) {
-    const uint32_t full = min(es.wm, cap) / kChunk;       // complete chunks that are final and visible
-    const uint32_t per_pass = 32u * (t.n >> 5);            // keep every lane of every warp busy
-    if (full >= done + per_pass) {
-      const uint32_t n = (full - done) / per_pass * per_pass;
-      hash_range(t, done, done + n);
-      done += n;
-    }
-  }
-  ZN_D void finish(const Team& t, zs::ExecState& es) {
-    zs::mem_sync(t, es);  // drain bulk stores, make the tail visible
-    if (es.pos == cap) hash_range(t, done, n_chunks);      // a short / long decode is an error anyway
-    done = n_chunks;
-  }
-};
-
 // `only_if` (nullable): word only_if[i * only_stride] != 0 selects list item i; null = every item.
 // NT threads per team; the CTA claims KB work items per atomic and its first KB warps fetch their descriptors (and
 // stage blobs <= kSrcSmall) in parallel, so the three dependent global round trips (counter -> list -> descriptor ->
 // bytes) are paid once per KB blobs instead of once per blob.  This is what bounds the 100 000 x 10 KiB-file corpus.
-template <int NT, int KB, bool FUSE>
+template <int NT, int KB>
 __global__ void __launch_bounds__(NT, NT == 32 ? 16 : 512 / NT) k_decode(const BlobDesc* __restrict__ blobs, const uint32_t* __restrict__ list,
                                                          uint32_t n_list, const uint8_t* blobs_base, uint8_t* out_base,
                                                          uint8_t* lit_scratch, uint32_t* status, uint32_t* produced,
                                                          uint32_t* work_counter, uint32_t* cvs, uint32_t one,
                                                          const uint32_t* only_if, uint32_t only_stride) {
-  extern __shared__ __align__(16) uint8_t hash_stage[];  // FUSE only: (NT / 32) x kB3SmemPerWarp
   __shared__ DecShared sh;
   __shared__ uint32_t s_base;
   __shared__ BlobDesc s_desc[KB];
@@ -119,21 +79,7 @@ __global__ void __launch_bounds__(NT, NT == 32 ? 16 : 512 / NT) k_decode(const B
           __syncthreads();
           src = s_src + 16;
         }
-        if (FUSE) {
-          HashHook hook;
-          hook.stage = hash_stage; hook.out = out_base + d.dst_off; hook.cvs = cvs + d.cv_base * 8;
-          hook.cap = (uint32_t)d.dst_cap; hook.n_chunks = d.n_chunks; hook.done = 0; hook.one = one;
-          if (d.flags & F_LZ4_BLOCK) {
-            st = decode_lz4_block(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, &got);
-            if (st == S_OK) {
-              zs::ExecState es;
-              es.pos = got; es.wm = 0; es.bulk = 1;
-              hook.finish(t, es);
-            }
-          } else {
-            st = decode_blob(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, lit, predef, &got, hook);
-          }
-        } else if (d.flags & F_LZ4_BLOCK) {
+        if (d.flags & F_LZ4_BLOCK) {
           st = decode_lz4_block(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, &got);
         } else {
           st = decode_blob(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, lit, predef, &got);

@@ -101,7 +101,6 @@ struct zn_plan {
   cudaStream_t last_stream = nullptr;
   bool ran = false;
   uint32_t cls_off[DC_COUNT + 1] = {0};  // class c = d_list_dec[cls_off[c] .. cls_off[c + 1]), largest blobs first
-  bool fused_hash = false;   // the DC_BIGPAT rows' chaining values come out of the fused decode kernel
   uint32_t n_hashed = 0;     // rows whose chunks k_b3_chunks may skip
   // device-wide pipeline (DC_PIPE rows)
   zp::ZBlob* d_zb = nullptr;
@@ -113,7 +112,7 @@ struct zn_plan {
 };
 
 static const int kDecodeThreads = 128;
-static const int kDecodeCtasPerSm = 4;  // resident k_decode<128> CTAs per SM (128 regs, 42 KB smem); <256>: half
+static const int kDecodeCtasPerSm = 4;  // resident k_decode<128> CTAs per SM (128 regs, 42 KB smem)
 
 #define ZN_CUDA(ctx, call)                                                              \
   do {                                                                                  \
@@ -195,7 +194,6 @@ extern "C" zn_ctx* zn_ctx_create(int device, size_t staging_bytes) {
   build_predef(&pd);
   if (cudaMemcpyToSymbol(g_predef, &pd, sizeof pd) != cudaSuccess) { zn_ctx_destroy(c); return nullptr; }
   cudaFuncSetAttribute(k_b3_chunks, cudaFuncAttributeMaxDynamicSharedMemorySize, kB3Warps * kB3SmemPerWarp);
-  cudaFuncSetAttribute(k_decode<256, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * kB3SmemPerWarp);
   cudaFuncSetAttribute(k_decode_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWsSmemBytes);
   cudaFuncSetAttribute(par::k_decode_par, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(par::ParShared));
   if (!zp::pipeline_init()) { zn_ctx_destroy(c); return nullptr; }
@@ -313,11 +311,6 @@ extern "C" int zn_plan_set_overlap(zn_plan* p, int groups) {
   return p ? ZN_OK : ZN_E_ARG;
 }
 
-static bool env_off(const char* name) {
-  const char* e = getenv(name);
-  return e && !strcmp(e, "0");
-}
-
 static zn_plan* plan_build(zn_ctx* c, int kind, uint32_t n, const uint64_t* src_off, const uint64_t* src_len,
                            const uint8_t* compressed, const uint64_t* out_off, const uint64_t* out_len,
                            const uint8_t* expect, bool gather_raw) {
@@ -351,7 +344,6 @@ static zn_plan* plan_build(zn_ctx* c, int kind, uint32_t n, const uint64_t* src_
   uint32_t n_lsmall = 0;
   std::vector<uint32_t> llarge, pblob, pidx, cls[DC_COUNT];
   std::vector<uint64_t> magic_off;
-  const bool use_pipe = !env_off("ZN_PIPE"), use_fuse = !env_off("ZN_FUSE");
   uint64_t chunks = 0;
   bool any_status = false;
   for (uint32_t i = 0; i < n; i++) {
@@ -388,7 +380,7 @@ static zn_plan* plan_build(zn_ctx* c, int kind, uint32_t n, const uint64_t* src_
       const bool big = d.dst_cap >= (512u << 10), pat = d.src_len * 64 <= d.dst_cap, lz4b = (d.flags & F_LZ4_BLOCK) != 0;
       int k;
       if (big && pat && !lz4b) k = DC_BIGPAT;
-      else if (use_pipe && !lz4b && !pat && d.src_len < d.dst_cap && d.dst_cap >= 4096 && d.dst_cap < 0xFFFFFFF0ull) k = DC_PIPE;
+      else if (!lz4b && !pat && d.src_len < d.dst_cap && d.dst_cap >= 4096 && d.dst_cap < 0xFFFFFFF0ull) k = DC_PIPE;
       else if (big) k = DC_BIGRAW;
       else if (d.dst_cap <= (64u << 10)) k = DC_SMALL;
       else k = DC_MID;
@@ -413,11 +405,8 @@ static zn_plan* plan_build(zn_ctx* c, int kind, uint32_t n, const uint64_t* src_
   }
   p->cls_off[DC_COUNT] = n_ldec;
   p->n_dec = n_ldec;
-  // Large, highly compressible blobs go through the fused decode+hash kernel (fused_ws.cuh).  ZN_FUSE=0 keeps the two
-  // kernels apart, ZN_FUSE=team selects the older fused kernel in which one team alternates between decoding and hashing.
-  p->fused_hash = use_fuse && !cls[DC_BIGPAT].empty();
-  if (p->fused_hash)
-    for (uint32_t i : cls[DC_BIGPAT]) { descs[i].flags |= F_HASHED; p->ws_tiles += (descs[i].n_chunks + 31u) / 32u; p->n_hashed++; }
+  // Large, highly compressible blobs go through the fused decode+hash kernel (fused_ws.cuh).
+  for (uint32_t i : cls[DC_BIGPAT]) { descs[i].flags |= F_HASHED; p->ws_tiles += (descs[i].n_chunks + 31u) / 32u; p->n_hashed++; }
   // device-wide pipeline: per-blob block-table slots and pool budgets (zpipe.cuh; anything that does not fit is decoded
   // by the one-team kernel instead)
   std::vector<zp::ZBlob> zb(cls[DC_PIPE].size());
@@ -460,7 +449,7 @@ static zn_plan* plan_build(zn_ctx* c, int kind, uint32_t n, const uint64_t* src_
             upload(c, &p->d_digests, (const uint32_t*)nullptr, (size_t)n * 8) &&
             upload(c, &p->d_status, (const uint32_t*)nullptr, n) && upload(c, &p->d_produced, (const uint32_t*)nullptr, n) &&
             upload(c, &p->d_counter, (const uint32_t*)nullptr, 16) &&
-            upload(c, &p->d_wsq, (const uint32_t*)nullptr, p->fused_hash ? 6 + 2 * (size_t)p->ws_tiles : 0) &&
+            upload(c, &p->d_wsq, (const uint32_t*)nullptr, cls[DC_BIGPAT].empty() ? 0 : 6 + 2 * (size_t)p->ws_tiles) &&
             upload(c, &p->d_zb, zb.data(), zb.size());
   if (ok && any_status) ok = upload(c, &p->d_status0, status0, n);
   for (int i = 0; ok && i < 4; i++) ok = cudaEventCreate(&p->ev[i]) == cudaSuccess;
@@ -487,7 +476,7 @@ extern "C" zn_plan* zn_plan_hash(zn_ctx* ctx, uint32_t n, const uint64_t* h_off,
   return plan_build(ctx, PLAN_HASH, n, h_off, h_len, nullptr, nullptr, nullptr, h_expect_digest, false);
 }
 
-extern "C" int zn_plan_fused(const zn_plan* p) { return p && p->fused_hash ? 1 : 0; }
+extern "C" int zn_plan_fused(const zn_plan* p) { return p && p->cls_off[DC_BIGPAT + 1] > p->cls_off[DC_BIGPAT] ? 1 : 0; }
 
 extern "C" int zn_plan_class_counts(const zn_plan* p, uint32_t counts[5]) {
   if (!p || !counts) return ZN_E_ARG;
@@ -566,9 +555,9 @@ static int run_pipeline(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, cuda
   // rows the pipeline handed back (ZBlob.state != 0): the one-team decoder, which also produces their status
   const uint32_t* list = p->d_list_dec + p->cls_off[DC_PIPE];
   const uint32_t grid = std::min<uint32_t>(p->nzb, c->dec_grid);
-  k_decode<kDecodeThreads, 1, false><<<grid, kDecodeThreads, 0, st>>>(p->d_blobs, list, p->nzb, d_blobs, d_out, c->d_lit, p->d_status,
-                                                                   p->d_produced, ctr + 1, nullptr, 1u, &p->d_zb[0].state,
-                                                                   (uint32_t)(sizeof(zp::ZBlob) / 4));
+  k_decode<kDecodeThreads, 1><<<grid, kDecodeThreads, 0, st>>>(p->d_blobs, list, p->nzb, d_blobs, d_out, c->d_lit, p->d_status,
+                                                            p->d_produced, ctr + 1, nullptr, 1u, &p->d_zb[0].state,
+                                                            (uint32_t)(sizeof(zp::ZBlob) / 4));
   if (prof) {
     cudaEventRecord(pe[7], st);
     cudaEventSynchronize(pe[7]);
@@ -624,31 +613,21 @@ extern "C" int zn_plan_run(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, v
     if (rc != ZN_OK) return rc;
   }
   if (const uint32_t nd = cls_n(DC_BIGPAT)) {  // highly compressible large blobs (few, long sequences)
-    const uint32_t* list = cls_list(DC_BIGPAT);
-    uint32_t grid = std::min<uint32_t>(nd, c->dec_grid / 2);
-    if (const char* gs = getenv("ZN_WS_GRID")) grid = std::max(1, std::min<int>((int)grid, atoi(gs)));  // tests: several blobs per CTA
-    const char* fm = getenv("ZN_FUSE");
-    if (p->fused_hash && !(fm && !strcmp(fm, "team"))) {
-      // warp-specialised fused kernel: one CTA per SM, two decode teams each; its tile queue starts empty
-      ZN_CUDA(c, cudaMemsetAsync(p->d_wsq, 0, 24 + 8 * (size_t)p->ws_tiles, st));
-      p->ran_ws = true;
-      // tests (ZN_WS_TEST_STALL=1): announce one tile more than the producers will ever publish, so that a hash warp waits
-      // for an entry that never comes and the watchdog has to end the kernel
-      const uint32_t phantom = getenv("ZN_WS_TEST_STALL") ? 1u : 0u;
-      WsQueue q{p->d_wsq, reinterpret_cast<unsigned long long*>(p->d_wsq + 4), p->ws_tiles + phantom};
-      uint32_t wgrid = (uint32_t)c->sm_count;  // every SM hashes, whether or not one of its teams gets a blob
-      if (const char* gs = getenv("ZN_WS_GRID")) wgrid = std::max(1, std::min<int>((int)wgrid, atoi(gs)));
-      k_decode_ws<<<wgrid, kWsThreads, kWsSmemBytes, st>>>(p->d_blobs, list, nd, d_blobs, d_out, c->d_lit, p->d_status,
-                                                           p->d_produced, p->d_counter + DC_BIGPAT, p->d_cvs, q, 1u);
-    } else if (p->fused_hash)
-      k_decode<256, 1, true><<<grid, 256, 8 * kB3SmemPerWarp, st>>>(p->d_blobs, list, nd, d_blobs, d_out, c->d_lit, p->d_status,
-                                                                   p->d_produced, p->d_counter + DC_BIGPAT, p->d_cvs, 1u, nullptr, 0u);
-    else
-      k_decode<256, 1, false><<<grid, 256, 0, st>>>(p->d_blobs, list, nd, d_blobs, d_out, c->d_lit, p->d_status,
-                                                    p->d_produced, p->d_counter + DC_BIGPAT, nullptr, 1u, nullptr, 0u);
+    // warp-specialised fused kernel: one CTA per SM, two decode teams each; its tile queue starts empty
+    ZN_CUDA(c, cudaMemsetAsync(p->d_wsq, 0, 24 + 8 * (size_t)p->ws_tiles, st));
+    p->ran_ws = true;
+    // tests (ZN_WS_TEST_STALL=1): announce one tile more than the producers will ever publish, so that a hash warp waits
+    // for an entry that never comes and the watchdog has to end the kernel
+    const uint32_t phantom = getenv("ZN_WS_TEST_STALL") ? 1u : 0u;
+    WsQueue q{p->d_wsq, reinterpret_cast<unsigned long long*>(p->d_wsq + 4), p->ws_tiles + phantom};
+    uint32_t wgrid = (uint32_t)c->sm_count;  // every SM hashes, whether or not one of its teams gets a blob
+    // tests (ZN_WS_GRID): a smaller grid, so that every decode team takes several blobs
+    if (const char* gs = getenv("ZN_WS_GRID")) wgrid = std::max(1, std::min<int>((int)wgrid, atoi(gs)));
+    k_decode_ws<<<wgrid, kWsThreads, kWsSmemBytes, st>>>(p->d_blobs, cls_list(DC_BIGPAT), nd, d_blobs, d_out, c->d_lit, p->d_status,
+                                                         p->d_produced, p->d_counter + DC_BIGPAT, p->d_cvs, q, 1u);
     launches++;
   }
-  if (const uint32_t nd = cls_n(DC_BIGRAW)) {  // large raw-block / LZ4 / (pipeline off) entropy-coded blobs: one CTA per SM
+  if (const uint32_t nd = cls_n(DC_BIGRAW)) {  // large raw-block / LZ4 blobs: one CTA per SM
     const uint32_t max_grid = (uint32_t)c->sm_count;
     if (!c->d_par && cudaMalloc(&c->d_par, (size_t)max_grid * par::kParScratchPerCta) != cudaSuccess) {
       c->err = "block-parallel decode scratch allocation failed";
@@ -661,15 +640,15 @@ extern "C" int zn_plan_run(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, v
   }
   if (const uint32_t nd = cls_n(DC_SMALL)) {  // many small blobs: one warp per blob, ~10 blobs in flight per SM
     const uint32_t grid = std::min<uint32_t>((nd + 1) / 2, c->dec_grid_small);
-    k_decode<32, 2, false><<<grid, 32, 0, st>>>(p->d_blobs, cls_list(DC_SMALL), nd, d_blobs, d_out, c->d_lit, p->d_status, p->d_produced,
-                                                p->d_counter + DC_SMALL, nullptr, 1u, nullptr, 0u);
+    k_decode<32, 2><<<grid, 32, 0, st>>>(p->d_blobs, cls_list(DC_SMALL), nd, d_blobs, d_out, c->d_lit, p->d_status, p->d_produced,
+                                         p->d_counter + DC_SMALL, nullptr, 1u, nullptr, 0u);
     launches++;
   }
   if (const uint32_t nd = cls_n(DC_MID)) {
     const uint32_t grid = std::min<uint32_t>((nd + 3) / 4, c->dec_grid);
-    k_decode<kDecodeThreads, 4, false><<<grid, kDecodeThreads, 0, st>>>(p->d_blobs, cls_list(DC_MID), nd, d_blobs, d_out, c->d_lit,
-                                                                     p->d_status, p->d_produced, p->d_counter + DC_MID, nullptr, 1u,
-                                                                     nullptr, 0u);
+    k_decode<kDecodeThreads, 4><<<grid, kDecodeThreads, 0, st>>>(p->d_blobs, cls_list(DC_MID), nd, d_blobs, d_out, c->d_lit,
+                                                              p->d_status, p->d_produced, p->d_counter + DC_MID, nullptr, 1u,
+                                                              nullptr, 0u);
     launches++;
   }
   ZN_CUDA(c, cudaEventRecord(p->ev[1], st));
@@ -682,8 +661,8 @@ extern "C" int zn_plan_run(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, v
     launches++;
   }
   ZN_CUDA(c, cudaEventRecord(p->ev[2], st));
-  // Zstandard content checksums are checked where a row's digest is compared (xxh_verify.cuh); ZN_XXH=0 turns that off
-  const uint8_t* xxh_out = p->n_dec && !env_off("ZN_XXH") ? d_out : nullptr;
+  // Zstandard content checksums are checked where a row's digest is compared (xxh_verify.cuh)
+  const uint8_t* xxh_out = p->n_dec ? d_out : nullptr;
   if (p->n_small) {
     k_b3_tree_small<<<(p->n_small + 127) / 128, 128, 0, st>>>(p->d_blobs, p->d_list_small, p->n_small, p->d_cvs, p->d_digests,
                                                               p->d_expect, p->d_status, 1u, d_blobs, xxh_out);

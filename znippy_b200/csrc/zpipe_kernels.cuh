@@ -5,10 +5,10 @@
 //   k_ztables  warp per block       FSE table descriptions -> fat decoding tables (all lanes, position by position)
 //   k_zseq1    LANE per block       sequence stage, phase 1: the FSE state chain alone (tables + bit stream in shared memory)
 //   k_zseq2    warp per block       sequence stage, phase 2: values, positions, repeat offsets (prefix scans), 16-byte records
-//   k_zseq_g   LANE per block       the one-pass sequence stage (batches of many small blobs); k_zseq / k_zseq1_g: measured variants
+//   k_zseq_g   LANE per block       the one-pass sequence stage (batches of many small blobs)
 //   k_zlit     LANE per stream      Huffman literals, decoding table in shared memory, word stores
 //   k_zchain   thread per blob      output offsets, repeat-offset histories, size checks
-//   k_zexec    CTA per blob         sequence execution in shared memory, group by group
+//   k_zexec2   CTA per blob         sequence execution in shared memory, group by group
 //
 // Every kernel is latency-bound integer work; the design goal is the number of independent dependent-chains in flight
 // (32 per warp in seq / lit, versus one per warp in the one-team-per-blob decoders), not bytes per instruction.
@@ -24,8 +24,6 @@ __device__ FseD g_zpredef[kTabSet];  // decoding tables of the predefined distri
 // shared-memory accesses by 32-bit shared address (no generic-address arithmetic in the byte loops)
 ZN_D uint32_t lds8(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 ZN_D void sts8(uint32_t a, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-ZN_D uint32_t lds32(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
-ZN_D void sts32(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
 // table reads of the sequence decoder: not volatile (the lane's tables never change while it decodes), so the
 // compiler may schedule them early
 ZN_D uint32_t lds32_ro(uint32_t a) { uint32_t v; asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
@@ -167,136 +165,6 @@ __global__ void __launch_bounds__(kTabWarps * 32) k_ztables(ZArgs a) {
 }
 
 // ----------------------------------------------------------------------------------------------------------------- seq
-// One lane per block.  The lane's three decoding tables (5 KiB of 4-byte entries) are copied into shared memory first:
-// with them in global memory the kernel was bound by DRAM latency (16 384 table sets = 168 MB of random 8-byte reads
-// thrashed the L2: 26 GB of DRAM reads, 15 ms); now the state chain runs at shared-memory latency.  kSeqLanes streams
-// per SM (one CTA, two warps) is what 227 KB of shared memory hold.
-constexpr uint32_t kSeqLanes = 44;
-constexpr uint32_t kSeqSmem = kSeqLanes * kTabSet * 4 + (36 + 53) * 4;
-
-struct SmemTabs {
-  uint32_t tab_s, lut_s;  // shared addresses: the lane's table set, the baseline LUTs (LL at 0, ML at 36)
-  ZN_D uint32_t ld(int k, uint32_t i) const { return lds32_ro(tab_s + 4u * ((k == 0 ? kTabOffLL : (k == 1 ? kTabOffOF : kTabOffML)) + i)); }
-  ZN_D uint32_t base(int k, uint32_t sym) const { return lds32_ro(lut_s + 4u * ((k == 0 ? 0u : 36u) + sym)); }
-};
-
-__global__ void __launch_bounds__(64, 1) k_zseq(ZArgs a) {
-  extern __shared__ __align__(16) uint8_t seq_smem[];
-  const uint32_t tid = threadIdx.x;
-  const uint32_t smem_s = (uint32_t)__cvta_generic_to_shared(seq_smem);
-  const uint32_t lut_s = smem_s + kSeqLanes * kTabSet * 4;
-  for (uint32_t i = tid; i < 36; i += 64) sts32(lut_s + 4 * i, zs::kLLBase[i]);
-  for (uint32_t i = tid; i < 53; i += 64) sts32(lut_s + 4 * (36 + i), zs::kMLBase[i]);
-  __syncthreads();
-  if (tid >= kSeqLanes) return;
-  SmemTabs st;
-  st.tab_s = smem_s + tid * kTabSet * 4;
-  st.lut_s = lut_s;
-  const uint32_t n_comp = min(a.pools->comp_used, a.pools->comp_cap);
-  for (uint32_t it = blockIdx.x * kSeqLanes + tid; it < n_comp; it += gridDim.x * kSeqLanes) {
-    const uint32_t slot = a.comp_list[it];
-    if (slot == kNoSlot) continue;
-    ZBlock* b = &a.blocks[slot];
-    if (b->nseq == 0 || b->bits_off == ~0u) continue;
-    const ZBlob z = a.zb[b->pad[0]];
-    const BlobDesc d = a.blobs[z.blob];
-    const uint8_t* src = a.blobs_base + d.src_off;
-    uint32_t logs[3];
-    bool ok = true;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-      const uint32_t offs = k == 0 ? kTabOffLL : (k == 1 ? kTabOffOF : kTabOffML);
-      const uint32_t def = b->seq_def[k];
-      const FseD* t = g_zpredef + offs;
-      logs[k] = k == 1 ? 5u : 6u;
-      if (def == kDefNone) ok = false;
-      else if (def != kDefPredef) {
-        const ZBlock* db = &a.blocks[z.slot0 + def];
-        if (db->bits_off == ~0u || db->tab_slot == kNoSlot) ok = false;
-        else {
-          t = a.tabs + (size_t)db->tab_slot * kTabSet + offs;
-          logs[k] = (db->tlogs >> (8 * k)) & 0xFFu;
-        }
-      }
-      if (ok) {
-        const uint32_t n = 1u << logs[k], dst = st.tab_s + 4u * offs;
-        for (uint32_t i = 0; i < n; i++) sts32(dst + 4 * i, t[i]);
-      }
-    }
-    if (!ok) continue;
-    uint32_t matched, lit_used, rep[3];
-    if (decode_sequences(src, b, st, logs, a.recs + b->seq_base, &matched, &lit_used, rep)) {
-      b->matched = matched;
-      b->lit_used = lit_used;
-      b->rep_fin[0] = rep[0]; b->rep_fin[1] = rep[1]; b->rep_fin[2] = rep[2];
-      b->st_seq = 0;
-    }
-  }
-}
-
-// Variant with the tables left in global memory (4-byte entries: all table sets of a 2 GiB batch are 84 MB and stay
-// L2-resident when the record stores stream past them): every block of the batch is decoded at once, one lane each.
-struct GlobalTabs {
-  const FseD* t[3];
-  uint32_t lut_s;
-  // .cg: the table sets of the lanes of one SM (3.5 warps x 32 lanes x 5 KiB) are several times its L1; left to allocate
-  // there they evict the lanes' bitstream lines, and the refill then waits for L2 as well (ZN_SEQ_LDG=1: the old form)
-  ZN_D uint32_t ld(int k, uint32_t i) const { return cg ? __ldcg(t[k] + i) : __ldg(t[k] + i); }
-  bool cg = true;
-  ZN_D uint32_t base(int k, uint32_t sym) const { return lds32_ro(lut_s + 4u * ((k == 0 ? 0u : 36u) + sym)); }
-};
-
-__global__ void __launch_bounds__(32) k_zseq_g(ZArgs a, int cg) {
-  __shared__ uint32_t s_lut[36 + 53];
-  const uint32_t tid = threadIdx.x;
-  for (uint32_t i = tid; i < 36; i += 32) s_lut[i] = zs::kLLBase[i];
-  for (uint32_t i = tid; i < 53; i += 32) s_lut[36 + i] = zs::kMLBase[i];
-  __syncwarp();
-  GlobalTabs st;
-  st.cg = cg != 0;
-  st.lut_s = (uint32_t)__cvta_generic_to_shared(s_lut);
-  const uint32_t n_comp = min(a.pools->comp_used, a.pools->comp_cap);
-  for (uint32_t it = blockIdx.x * 32 + tid; it < n_comp; it += gridDim.x * 32) {
-    const uint32_t slot = a.comp_list[it];
-    if (slot == kNoSlot) continue;
-    ZBlock* b = &a.blocks[slot];
-    if (b->nseq == 0 || b->bits_off == ~0u) continue;
-    const ZBlob z = a.zb[b->pad[0]];
-    const BlobDesc d = a.blobs[z.blob];
-    const uint8_t* src = a.blobs_base + d.src_off;
-    uint32_t logs[3];
-    bool ok = true;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-      const uint32_t offs = k == 0 ? kTabOffLL : (k == 1 ? kTabOffOF : kTabOffML);
-      const uint32_t def = b->seq_def[k];
-      st.t[k] = g_zpredef + offs;
-      logs[k] = k == 1 ? 5u : 6u;
-      if (def == kDefNone) ok = false;
-      else if (def != kDefPredef) {
-        const ZBlock* db = &a.blocks[z.slot0 + def];
-        if (db->bits_off == ~0u || db->tab_slot == kNoSlot) ok = false;
-        else {
-          st.t[k] = a.tabs + (size_t)db->tab_slot * kTabSet + offs;
-          logs[k] = (db->tlogs >> (8 * k)) & 0xFFu;
-        }
-      }
-    }
-    if (!ok) continue;
-    uint32_t matched, lit_used, rep[3];
-    if (decode_sequences(src, b, st, logs, a.recs + b->seq_base, &matched, &lit_used, rep)) {
-      b->matched = matched;
-      b->lit_used = lit_used;
-      b->rep_fin[0] = rep[0]; b->rep_fin[1] = rep[1]; b->rep_fin[2] = rep[2];
-      b->st_seq = 0;
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------- seq, two-phase form
-// (zpipe.cuh, "seq, two-phase form").  Phase 1 is the state chain alone, one lane per block; phase 2 decodes the values
-// of every sequence independently, a thread per run of consecutive sequences, and writes the final records.
-
 // Where a block's three tables come from (own set, an earlier block's, predefined) and their logs; false = undefined.
 ZN_D bool seq_table_sources(const ZArgs& a, const ZBlock* b, const ZBlob& z, const FseD** t, uint32_t* logs) {
   bool ok = true;
@@ -318,6 +186,50 @@ ZN_D bool seq_table_sources(const ZArgs& a, const ZBlock* b, const ZBlob& z, con
   }
   return ok;
 }
+
+// One-pass form: one lane per block, every block of the batch at once.  The tables stay in global memory (4-byte
+// entries: all table sets of a 2 GiB batch are 84 MB and stay L2-resident when the record stores stream past them).
+struct GlobalTabs {
+  const FseD* t[3];
+  uint32_t lut_s;
+  // .cg: the table sets of the lanes of one SM (3.5 warps x 32 lanes x 5 KiB) are several times its L1; left to allocate
+  // there they evict the lanes' bitstream lines, and the refill then waits for L2 as well
+  ZN_D uint32_t ld(int k, uint32_t i) const { return __ldcg(t[k] + i); }
+  ZN_D uint32_t base(int k, uint32_t sym) const { return lds32_ro(lut_s + 4u * ((k == 0 ? 0u : 36u) + sym)); }
+};
+
+__global__ void __launch_bounds__(32) k_zseq_g(ZArgs a) {
+  __shared__ uint32_t s_lut[36 + 53];
+  const uint32_t tid = threadIdx.x;
+  for (uint32_t i = tid; i < 36; i += 32) s_lut[i] = zs::kLLBase[i];
+  for (uint32_t i = tid; i < 53; i += 32) s_lut[36 + i] = zs::kMLBase[i];
+  __syncwarp();
+  GlobalTabs st;
+  st.lut_s = (uint32_t)__cvta_generic_to_shared(s_lut);
+  const uint32_t n_comp = min(a.pools->comp_used, a.pools->comp_cap);
+  for (uint32_t it = blockIdx.x * 32 + tid; it < n_comp; it += gridDim.x * 32) {
+    const uint32_t slot = a.comp_list[it];
+    if (slot == kNoSlot) continue;
+    ZBlock* b = &a.blocks[slot];
+    if (b->nseq == 0 || b->bits_off == ~0u) continue;
+    const ZBlob z = a.zb[b->pad[0]];
+    const BlobDesc d = a.blobs[z.blob];
+    const uint8_t* src = a.blobs_base + d.src_off;
+    uint32_t logs[3];
+    if (!seq_table_sources(a, b, z, st.t, logs)) continue;
+    uint32_t matched, lit_used, rep[3];
+    if (decode_sequences(src, b, st, logs, a.recs + b->seq_base, &matched, &lit_used, rep)) {
+      b->matched = matched;
+      b->lit_used = lit_used;
+      b->rep_fin[0] = rep[0]; b->rep_fin[1] = rep[1]; b->rep_fin[2] = rep[2];
+      b->st_seq = 0;
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------- seq, two-phase form
+// (zpipe.cuh, "seq, two-phase form").  Phase 1 is the state chain alone, one lane per block; phase 2 decodes the values
+// of every sequence independently, a thread per run of consecutive sequences, and writes the final records.
 
 // phase 1, tables in shared memory in the 3-byte phase-1 format (converted while they are copied in): per lane kTabSet
 // u16 {base | state bits << 10}, then kTabSet u8 {state bits + extra bits}
@@ -364,34 +276,6 @@ __global__ void __launch_bounds__(64, 1) k_zseq1(ZArgs a) {
         sts8(st.tab_s + 2u * kTabSet + e0 + i, fd_nbits(e) + fd_extra(e));
       }
     }
-    if (seq_phase1(sb, a.blobs_base + d.src_off, b, st, logs, a.p1 + b->seq_base)) b->st_seq = 2;
-  }
-}
-
-// phase 1 with the tables left in global memory (every block of the batch at once, one L2 round trip on the chain)
-struct GlobalTabs1 {
-  const FseD* t[3];
-  ZN_D void ld1(int k, uint32_t i, uint32_t* nb, uint32_t* tot) const {
-    const FseD e = __ldcg(t[k] + i);
-    *nb = e & 0x3FFFu; *tot = fd_nbits(e) + fd_extra(e);
-  }
-};
-
-__global__ void __launch_bounds__(32) k_zseq1_g(ZArgs a) {
-  __shared__ __align__(16) uint8_t s_ring[32 * RingBits::kRingBytes];
-  RingBits sb;
-  sb.ring_s = (uint32_t)__cvta_generic_to_shared(s_ring) + threadIdx.x * RingBits::kRingBytes;
-  const uint32_t n_comp = min(a.pools->comp_used, a.pools->comp_cap);
-  for (uint32_t it = blockIdx.x * 32 + threadIdx.x; it < n_comp; it += gridDim.x * 32) {
-    const uint32_t slot = a.comp_list[it];
-    if (slot == kNoSlot) continue;
-    ZBlock* b = &a.blocks[slot];
-    if (b->nseq == 0 || b->bits_off == ~0u) continue;
-    const ZBlob z = a.zb[b->pad[0]];
-    const BlobDesc d = a.blobs[z.blob];
-    GlobalTabs1 st;
-    uint32_t logs[3];
-    if (!seq_table_sources(a, b, z, st.t, logs)) continue;
     if (seq_phase1(sb, a.blobs_base + d.src_off, b, st, logs, a.p1 + b->seq_base)) b->st_seq = 2;
   }
 }
@@ -543,31 +427,33 @@ __global__ void __launch_bounds__(64) k_zchain(ZArgs a) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------- exec
-// One CTA per blob, blocks in order.  A block's sequences are executed in GROUPS: the next <= K * NT
-// sequences whose output spans <= kGroupBytes, assembled in a shared-memory buffer and flushed with one coalesced copy.
+// One CTA per blob, blocks in order.  A block's sequences are executed in GROUPS: the next <= K * NT sequences whose
+// output spans <= GB bytes, assembled in a shared-memory buffer and flushed with one coalesced copy.  A sequence longer
+// than the buffer, raw / RLE blocks and a block's trailing literals are written straight to global memory by the whole
+// team.
 //
 // LZ77 execution is only serial where a match reads bytes that an earlier match of the same neighbourhood produces.
 // Measured on python sources (zstd level 3): the TRUE dependence depth of a 128 KiB block is ~70 matches, while it
-// holds ~10 000 of them — so a group is executed as a WAVEFRONT by all warps at once:
+// holds ~10 000 of them.  So the matches that read bytes of their own group are resolved by POINTER JUMPING over bytes:
 //
-//   setup   every thread owns K sequences (records prefetched a group ahead).  Literal runs come from the
-//           group's staged literals; FAR matches (source entirely before the group: final, read from global memory) are
-//           copied at once; every NEAR match leaves its parameters in shared memory and marks its destination bytes in a
-//           "pending" bitmap (one bit per byte).  Runs longer than 16 bytes become jobs that a whole warp copies;
-//   passes  the pending matches live in a compact list: one lane takes one match, looks at the pending bits of its source
-//           range, and either copies it (shared -> shared, 16 bytes per step) and clears its bits, or puts it on the
-//           next pass's list.  One barrier per pass; a pass executes (at least) one dependence level of the group,
-//           ~20 passes per group, and costs in proportion to the matches still pending;
-//   flush   one coalesced copy of the group to global memory.
+//   setup   every output byte of the group is either KNOWN — a literal, or a match byte whose source lies before the group
+//           (final, in global memory): stored into the buffer at once — or it gets a PARENT: the group-relative position it
+//           copies from (par[], 16 bits per byte; a match with distance < length points every byte into the window before
+//           the match, so it adds one level, not length / distance levels);
+//   rounds  the first round scans par[] (8 entries per 16-byte load) and lists the bytes that are still unknown after it;
+//           later rounds walk that list densely, one lane per unknown byte, compacting it as they go.  An unknown byte
+//           looks at its parent: known -> copy the byte and become known; unknown -> adopt the parent's parent.  Chains
+//           halve every round, so a group whose dependence depth is ~20 matches is done in ~5 rounds of plain loads and
+//           stores: no atomics, no fences — one barrier per round.  "Known" must mean "known before this round's
+//           barrier": a byte resolved in round r is marked with r's parity (kFresh); a reader in a round of the same
+//           parity waits one round (the marker may be this round's), a reader of the other parity copies — so nobody
+//           ever reads a byte that was stored in the same round, and no marker ever needs a second visit;
+//   flush   one coalesced copy of the group to global memory, par[] reset to kKnown.
 //
 // Everything is sized by instruction issue, not bytes: a lone lane that copies costs its warp as much as 32, so the
-// common cases are straight-line predicated code (<= 8 literal bytes, <= 16 match bytes) and the exceptions are
-// compacted into lists that are worked off densely.
-// A sequence longer than the buffer, raw / RLE blocks and a block's trailing literals are written straight to global
-// memory by the whole team.
+// common cases are straight-line predicated code and longer runs become jobs that a whole warp copies.
 constexpr uint32_t kLitLane = 8;     // literal runs up to this length: straight-line code in the owning lane
-constexpr uint32_t kMatchLane = 16;  // far matches up to this length likewise; longer runs become warp jobs
-constexpr uint32_t kNearLane = 64;   // ready near matches up to this length are copied by one lane, longer by a warp
+constexpr uint32_t kMatchLane = 16;  // matches up to this length likewise; longer ones become warp jobs
 
 // development (build with ZN_TRACE_BUILD=1): cycle counters of the exec kernel's phases, summed over the grid
 #ifdef ZP_TRACE
@@ -583,394 +469,6 @@ __device__ unsigned long long g_ztrace[32];
 #define ZT_FLUSH(base, n)
 #endif
 
-
-template <int NT, int K, uint32_t GB>
-struct ExecShared {
-  static constexpr uint32_t kSeqs = K * NT;
-  static constexpr uint32_t kGroupBytes = GB;                       // output bytes of one group (the buffer)
-  static constexpr uint32_t kLitWin = GB < 16384u ? GB : 16384u;    // literal bytes of one group (staged in shared memory)
-  alignas(16) uint8_t buf[kGroupBytes + 16];
-  alignas(16) uint8_t lits[kLitWin + 32];
-  uint32_t bm[kGroupBytes / 32 + 2];           // pending bytes of the group's near matches
-  uint32_t m_a[kSeqs], m_off[kSeqs];  // near matches: (destination - gpos) | (length - 1) << 15, distance
-  uint16_t jobs[kSeqs * 2];           // warp jobs of the setup: sequence (index in the group's thread layout) | kind << 15 (1 = literal run, 0 = far match)
-  uint16_t plist[2][kSeqs];           // pending near matches of this / the next pass (match indices, any order)
-  uint16_t longs[kSeqs];              // ready matches longer than kNearLane: a whole warp copies each at the start of the next pass
-  uint32_t n_pend[3], n_long[3], n_jobs;  // list lengths, rotating over three slots: pass q reads [q % 3], appends to [(q + 1) % 3], clears [(q + 2) % 3]
-  uint32_t pat[kPatWords];
-  SeqRec16 first;                     // record of the group's first candidate sequence
-  uint32_t cnt, gend, lit_hi;
-  uint32_t err, item;
-};
-
-// first word of the pending bitmap at or after bit p0 that has a pending bit in [p0, p1): returns its index and the
-// mask through *mask, or ~0u when the range is clear (p1 > p0)
-ZN_D uint32_t bm_first(uint32_t bm_s, uint32_t p0, uint32_t p1, uint32_t* mask) {
-  const uint32_t w0 = p0 >> 5, w1 = (p1 - 1) >> 5;
-  const uint32_t m0 = 0xFFFFFFFFu << (p0 & 31), m1 = 0xFFFFFFFFu >> (31 - ((p1 - 1) & 31));
-  for (uint32_t w = w0; w <= w1; w++) {
-    const uint32_t m = (w == w0 ? m0 : 0xFFFFFFFFu) & (w == w1 ? m1 : 0xFFFFFFFFu);
-    if (lds32(bm_s + 4 * w) & m) { *mask = m; return w; }
-  }
-  return ~0u;
-}
-template <bool SET>
-ZN_D void bm_mark(uint32_t* bm, uint32_t p0, uint32_t p1) {
-  const uint32_t w0 = p0 >> 5, w1 = (p1 - 1) >> 5;
-  const uint32_t m0 = 0xFFFFFFFFu << (p0 & 31), m1 = 0xFFFFFFFFu >> (31 - ((p1 - 1) & 31));
-  if (w0 == w1) { if (SET) atomicOr(bm + w0, m0 & m1); else atomicAnd(bm + w0, ~(m0 & m1)); return; }
-  if (SET) atomicOr(bm + w0, m0); else atomicAnd(bm + w0, ~m0);
-  for (uint32_t w = w0 + 1; w < w1; w++) bm[w] = SET ? 0xFFFFFFFFu : 0u;  // whole words belong to this match alone
-  if (SET) atomicOr(bm + w1, m1); else atomicAnd(bm + w1, ~m1);
-}
-
-template <int NT, int K, uint32_t GB, int MINB>
-__global__ void __launch_bounds__(NT, MINB) k_zexec(ZArgs a, uint8_t* out_base, uint32_t* produced, uint32_t* work_counter) {
-  extern __shared__ __align__(16) uint8_t exec_smem[];
-  using Sh = ExecShared<NT, K, GB>;
-  Sh* sh = reinterpret_cast<Sh*>(exec_smem);
-  constexpr uint32_t kGroupBytes = Sh::kGroupBytes, kLitWin = Sh::kLitWin;
-  const Team t{threadIdx.x, (uint32_t)NT};
-  const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-  const uint32_t buf_s = (uint32_t)__cvta_generic_to_shared(sh->buf), lits_s = (uint32_t)__cvta_generic_to_shared(sh->lits),
-                 bm_s = (uint32_t)__cvta_generic_to_shared(sh->bm);
-  for (uint32_t i = tid; i < kGroupBytes / 32 + 2; i += NT) sh->bm[i] = 0;
-  for (;;) {
-    if (tid == 0) sh->item = atomicAdd(work_counter, 1u);
-    __syncthreads();
-    const uint32_t item = sh->item;
-    if (tid == 0) { sh->err = 0; sh->cnt = 0; sh->gend = 0; sh->lit_hi = 0; sh->n_jobs = 0; sh->n_pend[0] = sh->n_pend[1] = sh->n_pend[2] = 0; sh->n_long[0] = sh->n_long[1] = sh->n_long[2] = 0; }
-    __syncthreads();
-    if (item >= a.nzb) break;
-    const ZBlob z = a.zb[item];
-    if (z.state) continue;
-    const BlobDesc d = a.blobs[z.blob];
-    const uint8_t* src = a.blobs_base + d.src_off;
-    uint8_t* out = out_base + d.dst_off;
-    bool bad = false;
-    ZT_DECL;
-    for (uint32_t j = 0; j < z.n_blocks && !bad; j++) {
-      const ZBlock* b = &a.blocks[z.slot0 + j];
-      const uint32_t flags = b->flags, type = flags & ZB_TYPE_MASK;
-      const uint32_t blk0 = b->out_base;
-      if (type == 0) { team_copy(t, out + blk0, src + b->src_off, b->len); __syncthreads(); continue; }
-      if (type == 1) { team_fill(t, out + blk0, src[b->src_off], b->len); __syncthreads(); continue; }
-      const uint32_t lt = (flags >> ZB_LIT_SHIFT) & 3u;
-      const uint8_t* lit = lt == 0 ? src + b->lit_off : a.lits + (size_t)b->lit_base16 * 16;
-      const int rle = lt == 1 ? (int)b->lit_off : -1;
-      const SeqRec16* seqs = a.recs + b->seq_base;
-      const uint32_t nseq = b->nseq, frame_start = b->frame_start;
-      const uint32_t r0 = b->rep_in[0], r1 = b->rep_in[1], r2 = b->rep_in[2];
-      uint32_t s0 = 0, gpos = blk0;  // gpos: blob-absolute output position where the next group starts
-      uint32_t lit_next = 0;         // literal position where the next group starts
-      SeqRec16 rn[K];                // prefetched records of sequences s0 + k * NT + tid
-#pragma unroll
-      for (int k = 0; k < K; k++) {
-        rn[k].w0 = rn[k].w1 = rn[k].w2 = rn[k].w3 = 0;
-        if (k * NT + tid < nseq) rn[k] = seqs[k * NT + tid];
-      }
-      while (s0 < nseq) {
-        ZT(0);
-        // ---- the group: the leading sequences that fit the buffer (end positions are monotonic, so "fits" is a prefix)
-        uint32_t inm = 0, my_gend = 0, my_lit_hi = 0;
-        SeqRec16 r[K];
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-          r[k] = rn[k];
-          const bool have = s0 + k * NT + tid < nseq;
-          const uint32_t endp = blk0 + rec_out(r[k]) + rec_ll(r[k]) + rec_ml(r[k]);
-          if (have && endp - gpos <= kGroupBytes && rec_lit(r[k]) + rec_ll(r[k]) - lit_next <= kLitWin) {
-            inm |= 1u << k;
-            my_gend = endp;  // k ascending = sequence index ascending
-            my_lit_hi = rec_lit(r[k]) + rec_ll(r[k]);
-          }
-        }
-        {
-          const uint32_t c = __reduce_add_sync(0xFFFFFFFFu, (uint32_t)__popc(inm));
-          const uint32_t ge = __reduce_max_sync(0xFFFFFFFFu, my_gend), lh = __reduce_max_sync(0xFFFFFFFFu, my_lit_hi);
-          if (lane == 0 && c) { atomicAdd(&sh->cnt, c); atomicMax(&sh->gend, ge); atomicMax(&sh->lit_hi, lh); }
-          if (tid == 0) sh->first = r[0];
-        }
-        __syncthreads();
-        const uint32_t count = sh->cnt, gend = sh->gend, lit_hi = sh->lit_hi;
-        const SeqRec16 q = sh->first;
-        if (count == 0) {
-          // ---- a sequence longer than the buffer: alone, in global memory, by the whole team
-          const uint32_t qo = blk0 + rec_out(q), qll = rec_ll(q), qlr = rec_lit(q), qml = rec_ml(q);
-          if (qll) {
-            if (rle >= 0) team_fill(t, out + qo, (uint32_t)rle, qll);
-            else team_copy(t, out + qo, lit + qlr, qll);
-          }
-          const uint32_t o = sym_resolve(rec_off(q), r0, r1, r2);
-          const uint32_t da = qo + qll;
-          if (qml && (o == 0 || o > da - frame_start)) { bad = true; break; }
-          __syncthreads();
-          if (qml) team_match(t, out + da, o, qml, sh->pat, nullptr);
-          __syncthreads();
-          gpos = da + qml;
-          lit_next = qlr + qll;
-          s0 += 1;
-#pragma unroll
-          for (int k = 0; k < K; k++) {
-            rn[k].w0 = rn[k].w1 = rn[k].w2 = rn[k].w3 = 0;
-            if (s0 + k * NT + tid < nseq) rn[k] = seqs[s0 + k * NT + tid];
-          }
-          continue;
-        }
-        // prefetch the next group's records: their latency hides behind this group's passes
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-          rn[k].w0 = rn[k].w1 = rn[k].w2 = rn[k].w3 = 0;
-          if (s0 + count + k * NT + tid < nseq) rn[k] = seqs[s0 + count + k * NT + tid];
-        }
-        const uint32_t lit_lo = rec_lit(q);
-        if (rle < 0 && lit_hi > lit_lo) team_copy(t, sh->lits, lit + lit_lo, lit_hi - lit_lo);
-        __syncthreads();
-        if (tid == 0) { sh->cnt = 0; sh->gend = 0; sh->lit_hi = 0; }  // (used again only after more barriers)
-        ZT(1);
-        // ---- setup: literal runs, far matches, parameters + pending bits of the near matches
-        // far sources first into L1 (one touch per 32-byte sector), so that the K copy steps below do not each pay a trip to DRAM
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-          if ((inm >> k) & 1u) {
-            const uint32_t ml = rec_ml(r[k]), off = sym_resolve(r[k].w0, r0, r1, r2);
-            const uint32_t dabs = blk0 + rec_out(r[k]) + rec_ll(r[k]);
-            if (ml && off >= ml && off <= dabs && dabs - off + ml <= gpos) {
-              const uint8_t* s = out + (dabs - off);
-              asm volatile("prefetch.global.L1 [%0];" ::"l"(s));
-              if (ml > 1) asm volatile("prefetch.global.L1 [%0];" ::"l"(s + (ml <= kMatchLane ? ml : kMatchLane) - 1));
-            }
-          }
-        }
-#pragma unroll
-        for (int k = 0; k < K; k++) {
-          const bool mine = (inm >> k) & 1u;
-          const uint32_t orl = rec_out(r[k]), ll = mine ? rec_ll(r[k]) : 0u, lr = rec_lit(r[k]);
-          const uint32_t ml = mine ? rec_ml(r[k]) : 0u;
-          const uint32_t oabs = blk0 + orl, dabs = oabs + ll;
-          // literal run: <= kLitLane bytes straight-line, longer ones as a warp job
-          if (ll && ll <= kLitLane) {
-            const uint32_t o = buf_s + (oabs - gpos), ls = lits_s + (lr - lit_lo);
-            uint32_t v[kLitLane];
-#pragma unroll
-            for (int i = 0; i < (int)kLitLane; i++) v[i] = rle >= 0 ? (uint32_t)rle : ((uint32_t)i < ll ? lds8(ls + i) : 0u);
-#pragma unroll
-            for (int i = 0; i < (int)kLitLane; i++) if ((uint32_t)i < ll) sts8(o + i, v[i]);
-          }
-          bool job_lit = ll > kLitLane, job_far = false, near_m = false;
-          uint32_t off = 1;
-          if (ml) {
-            off = sym_resolve(r[k].w0, r0, r1, r2);
-            if (off == 0 || off > dabs - frame_start) sh->err = 1;
-            else {
-              // far: the whole source lies before the group (final, in global memory) and the match does not feed itself
-              const bool far = off >= ml && dabs - off + ml <= gpos;
-              near_m = !far;
-              job_far = far && ml > kMatchLane;
-              if (far && ml <= kMatchLane) {
-                const uint8_t* s = out + (dabs - off);
-                const uint32_t o = buf_s + (dabs - gpos);
-                uint32_t v[kMatchLane];
-#pragma unroll
-                for (int i = 0; i < (int)kMatchLane; i++) if ((uint32_t)i < ml) v[i] = s[i];
-#pragma unroll
-                for (int i = 0; i < (int)kMatchLane; i++) if ((uint32_t)i < ml) sts8(o + i, v[i]);
-              }
-            }
-          }
-          if (near_m) {
-            const uint32_t idx = (uint32_t)k * NT + tid;
-            sh->m_a[idx] = (dabs - gpos) | ((ml - 1u) << 15); sh->m_off[idx] = off;
-            bm_mark<true>(sh->bm, dabs - gpos, dabs - gpos + ml);
-          }
-          {  // pending list of the first pass (order is irrelevant)
-            const uint32_t nb = __ballot_sync(0xFFFFFFFFu, near_m);
-            if (nb) {
-              uint32_t base = 0;
-              if (lane == 0) base = atomicAdd(&sh->n_pend[0], (uint32_t)__popc(nb));
-              base = __shfl_sync(0xFFFFFFFFu, base, 0);
-              if (near_m) sh->plist[0][base + __popc(nb & ((1u << lane) - 1u))] = (uint16_t)((uint32_t)k * NT + tid);
-            }
-          }
-          // jobs: long literal runs and long far matches
-          const uint32_t nj = (job_lit ? 1u : 0u) + (job_far ? 1u : 0u);
-          const uint32_t bj = __ballot_sync(0xFFFFFFFFu, nj != 0);
-          if (bj) {
-            uint32_t pre = nj;  // inclusive prefix sum of nj over the lanes
-#pragma unroll
-            for (int sft = 1; sft < 32; sft <<= 1) { const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, pre, sft); if ((int)lane >= sft) pre += v; }
-            uint32_t base = 0;
-            if (lane == 31) base = atomicAdd(&sh->n_jobs, pre);
-            base = __shfl_sync(0xFFFFFFFFu, base, 31);
-            uint32_t slot = base + pre - nj;
-            const uint32_t idx = (uint32_t)k * NT + tid;
-            if (job_lit) sh->jobs[slot++] = (uint16_t)(idx | 0x8000u);
-            if (job_far) sh->jobs[slot] = (uint16_t)idx;
-          }
-        }
-        __syncthreads();
-        if (sh->err) { bad = true; break; }
-        {  // work off the jobs: one warp per job
-          const uint32_t nj = sh->n_jobs;
-          for (uint32_t i = warp; i < nj; i += NT / 32) {
-            const uint32_t jb = sh->jobs[i], idx = jb & 0x7FFFu;
-            const SeqRec16 rr = seqs[s0 + idx];  // idx = k * NT + tid of the owner = offset from s0 (broadcast load)
-            const uint32_t oabs = blk0 + rec_out(rr), ll = rec_ll(rr);
-            if (jb & 0x8000u) {
-              const uint32_t dd = buf_s + (oabs - gpos), l2 = lits_s + (rec_lit(rr) - lit_lo);
-              for (uint32_t x = lane; x < ll; x += 32) sts8(dd + x, rle >= 0 ? (uint32_t)rle : lds8(l2 + x));
-            } else {
-              const uint32_t dabs = oabs + ll, l = rec_ml(rr);
-              const uint8_t* s = out + (dabs - sym_resolve(rr.w0, r0, r1, r2));
-              const uint32_t dd = buf_s + (dabs - gpos);
-              for (uint32_t x = lane; x < l; x += 32) sts8(dd + x, s[x]);
-            }
-          }
-        }
-        __syncthreads();
-        if (tid == 0) sh->n_jobs = 0;
-        ZT(2);
-        // ---- passes: one dependence level of the group per pass
-        for (uint32_t pass = 0;; pass++) {
-          ZT_CNT(8, tid == 0 ? 1 : 0);
-          const uint32_t par = pass & 1u, c0 = pass % 3u, c1 = (pass + 1u) % 3u, c2 = (pass + 2u) % 3u;
-          const uint32_t np = sh->n_pend[c0], nl = sh->n_long[c0];
-          if (np == 0 && nl == 0) break;
-          if (tid == 0) { sh->n_pend[c2] = 0; sh->n_long[c2] = 0; }  // read a pass ago, appended to a pass from now
-          if (pass > 4u * K * NT) { if (tid == 0) sh->err = 2; break; }  // cannot happen (every pass completes a match): never hang
-          ZT_CNT(10, tid == 0 ? np : 0);
-          // long matches that became ready in the previous pass: one warp each (byte x = window[x mod off])
-          for (uint32_t i = warp; i < nl; i += NT / 32) {
-            const uint32_t idx = sh->longs[i];
-            const uint32_t ma = sh->m_a[idx], oo = sh->m_off[idx];
-            const uint32_t drel = ma & 0x7FFFu, l = (ma >> 15) + 1u, da = gpos + drel;
-            // byte x = window[x mod off]; the phase advances by 32 mod off per step instead of a division per byte
-            uint32_t ph = oo >= l ? lane : lane % oo;
-            const uint32_t step = oo >= l ? 32u : 32u % oo;
-            for (uint32_t x = lane; x < l; x += 32) {
-              const uint32_t p = da - oo + ph;
-              sts8(buf_s + drel + x, p >= gpos ? lds8(buf_s + (p - gpos)) : (uint32_t)out[p]);
-              ph += step;
-              if (oo < l && ph >= oo) ph -= oo;
-            }
-            __syncwarp();
-            if (lane == 0) bm_mark<false>(sh->bm, drel, drel + l);
-          }
-          if (nl) __syncthreads();  // their bytes and cleared bits before anybody checks (uniform: nl is shared)
-          ZT(11);  // pass: counters + long matches
-          for (uint32_t base = warp * 32u; base < np; base += NT) {
-            const uint32_t i = base + lane;
-            const bool act = i < np;
-            uint32_t idx = 0, drel = 0, ml = 1, off = 1;
-            if (act) { idx = sh->plist[par][i]; const uint32_t ma = sh->m_a[idx]; drel = ma & 0x7FFFu; ml = (ma >> 15) + 1u; off = sh->m_off[idx]; }
-            const uint32_t dabs = gpos + drel, sabs = dabs - off;
-            // source bytes the match needs: the window before it, [sabs, min(sabs + ml, dabs)); bytes below gpos are final
-            const uint32_t send = off >= ml ? sabs + ml : dabs;
-            const uint32_t p0 = (sabs > gpos ? sabs : gpos) - gpos, p1 = send - gpos;
-            bool ready = act;
-            if (act && p1 > p0) { uint32_t m; ready = bm_first(bm_s, p0, p1, &m) == ~0u; }
-            const bool lane_copy = ready && ml <= kNearLane;
-            ZT(12);  // pass: list entry + readiness check
-            if (lane_copy) {
-              const uint32_t o = buf_s + drel;
-              if (off >= 16 && sabs >= gpos) {  // 16 loads in flight, then 16 stores
-                const uint32_t sa = buf_s + (sabs - gpos);
-                for (uint32_t c = 0; c < ml; c += 16) {
-                  uint32_t v[16];
-#pragma unroll
-                  for (int x = 0; x < 16; x++) if (c + x < ml) v[x] = lds8(sa + c + x);
-#pragma unroll
-                  for (int x = 0; x < 16; x++) if (c + x < ml) sts8(o + c + x, v[x]);
-                }
-              } else {  // short distance (bytes feed later bytes) or a source that starts before the group
-                for (uint32_t x = 0; x < ml; x++) {
-                  const uint32_t p = sabs + x;
-                  sts8(o + x, p >= gpos ? lds8(buf_s + (p - gpos)) : (uint32_t)out[p]);
-                }
-              }
-            }
-            // same-pass forwarding: the bytes are fenced before the bits are cleared, so a checker that sees clear bits
-            // later in this pass reads final bytes
-            ZT(13);  // pass: copy
-            // same-pass forwarding: the bytes are fenced before the bits are cleared, so a checker that sees clear bits
-            // later in this pass reads final bytes
-            if (__any_sync(0xFFFFFFFFu, lane_copy)) {
-              __threadfence_block();
-              if (lane_copy) bm_mark<false>(sh->bm, drel, drel + ml);
-            }
-            ZT(14);  // pass: clear bits
-            const bool is_long = ready && !lane_copy, again = act && !ready;
-            const uint32_t lb = __ballot_sync(0xFFFFFFFFu, is_long), ab = __ballot_sync(0xFFFFFFFFu, again);
-            if (lb) {
-              uint32_t b0 = 0;
-              if (lane == 0) b0 = atomicAdd(&sh->n_long[c1], (uint32_t)__popc(lb));
-              b0 = __shfl_sync(0xFFFFFFFFu, b0, 0);
-              if (is_long) sh->longs[b0 + __popc(lb & ((1u << lane) - 1u))] = (uint16_t)idx;
-            }
-            if (ab) {
-              uint32_t b0 = 0;
-              if (lane == 0) b0 = atomicAdd(&sh->n_pend[c1], (uint32_t)__popc(ab));
-              b0 = __shfl_sync(0xFFFFFFFFu, b0, 0);
-              if (again) sh->plist[par ^ 1u][b0 + __popc(ab & ((1u << lane) - 1u))] = (uint16_t)idx;
-            }
-            ZT(15);  // pass: appends
-          }
-          __syncthreads();
-          ZT(6);  // pass: barrier
-        }
-        __syncthreads();
-        if (tid == 0) { sh->n_pend[0] = sh->n_pend[1] = sh->n_pend[2] = 0; sh->n_long[0] = sh->n_long[1] = sh->n_long[2] = 0; }
-        ZT(3);
-        if (sh->err) { bad = true; break; }
-        // ---- flush
-        team_copy(t, out + gpos, sh->buf, gend - gpos);
-        __syncthreads();
-        ZT(4);
-        ZT_CNT(9, tid == 0 ? 1 : 0);
-        gpos = gend;
-        lit_next = lit_hi;
-        s0 += count;
-      }
-      if (bad) break;
-      const uint32_t rest = b->lit_regen - b->lit_used;
-      if (rest) {
-        if (rle >= 0) team_fill(t, out + blk0 + b->matched, (uint32_t)rle, rest);
-        else team_copy(t, out + blk0 + b->matched, lit + b->lit_used, rest);
-      }
-      __syncthreads();
-    }
-    if (bad) {  // leave the shared state clean for the next blob
-      __syncthreads();
-      for (uint32_t i = tid; i < kGroupBytes / 32 + 2; i += NT) sh->bm[i] = 0;
-    }
-    if (tid == 0) {
-      if (bad) a.zb[item].state = 1;
-      else produced[z.blob] = (uint32_t)d.dst_cap;
-      ZT(5);
-      ZT_FLUSH(0, 16);
-    }
-  }
-}
-
-
-// ------------------------------------------------------------------------------------------------------- exec, version 2
-// Same contract as k_zexec (one CTA per blob, blocks in order, groups of sequences assembled in shared memory), another
-// way of resolving the matches that read bytes of their own group: POINTER JUMPING over bytes instead of a wavefront
-// over matches.
-//
-//   setup   every output byte of the group is either KNOWN — a literal, or a match byte whose source lies before the group
-//           (final, in global memory): stored into the buffer at once — or it gets a PARENT: the group-relative position it
-//           copies from (par[], 16 bits per byte; a match with distance < length points every byte into the window before
-//           the match, so it adds one level, not length / distance levels);
-//   rounds  the first round scans par[] (8 entries per 16-byte load) and lists the bytes that are still unknown after it;
-//           later rounds walk that list densely, one lane per unknown byte, compacting it as they go.  An unknown byte
-//           looks at its parent: known -> copy the byte and become known; unknown -> adopt the parent's parent.  Chains halve every round, so a group whose
-//           dependence depth is ~20 matches is done in ~5 rounds of plain loads and stores: no pending lists, no bitmap,
-//           no atomics, no fences — one barrier per round.  "Known" must mean "known before this round's barrier": a byte
-//           resolved in round r is marked with r's parity (kFresh); a reader in a round of the same parity waits one round
-//           (the marker may be this round's), a reader of the other parity copies — so nobody ever reads a byte that was
-//           stored in the same round, and no marker ever needs a second visit;
-//   flush   one coalesced copy of the group to global memory, par[] reset to kKnown.
 // bytes per group (template parameter GB) <= 16384: parents are < 2^14, which leaves two flag bits in 16
 constexpr uint32_t kKnown = 0xFFFFu;  // par[] value of a byte whose value is in the buffer (since an earlier round)
 constexpr uint32_t kFresh = 0x8000u;  // | parity << 14: resolved in the round of that parity

@@ -22,17 +22,10 @@ bool pipeline_init() {
   static FseD zset[kTabSet];
   build_predef_set(zset);
   if (cudaMemcpyToSymbol(g_zpredef, zset, sizeof zset) != cudaSuccess) return false;
-  cudaFuncSetAttribute(k_zseq, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSeqSmem);
   cudaFuncSetAttribute(k_zseq1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSeq1Smem);
   cudaFuncSetAttribute(k_zlit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLitSmem);
-  cudaFuncSetAttribute(k_zexec<512, 4, 32768, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ExecShared<512, 4, 32768>));
-  cudaFuncSetAttribute(k_zexec<256, 8, 32768, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ExecShared<256, 8, 32768>));
-  cudaFuncSetAttribute(k_zexec<128, 4, 16384, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ExecShared<128, 4, 16384>));
-#define ZN_A2(NT, K, GB, MINB) ZN_A2L(NT, K, GB, MINB, GB / 4)
-#define ZN_A2L(NT, K, GB, MINB, LC) cudaFuncSetAttribute(k_zexec2<NT, K, GB, MINB, LC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Exec2Shared<NT, K, GB, LC>))
-  ZN_A2(256, 4, 16384, 2); ZN_A2(256, 4, 16384, 3); ZN_A2(512, 4, 16384, 2); ZN_A2(512, 2, 16384, 3); ZN_A2(1024, 2, 16384, 1); ZN_A2(1024, 2, 16384, 2); ZN_A2L(1024, 2, 16384, 2, 8192); ZN_A2L(512, 4, 16384, 2, 8192); ZN_A2(128, 4, 8192, 6); ZN_A2(128, 4, 8192, 4);
-#undef ZN_A2
-#undef ZN_A2L
+  cudaFuncSetAttribute(k_zexec2<512, 4, 16384, 2, 8192>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Exec2Shared<512, 4, 16384, 8192>));
+  cudaFuncSetAttribute(k_zexec2<512, 2, 16384, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Exec2Shared<512, 2, 16384, 4096>));
   return true;
 }
 
@@ -40,16 +33,8 @@ void pipeline_trace_dump() {
 #ifdef ZP_TRACE
   unsigned long long h[32];
   cudaMemcpyFromSymbol(h, g_ztrace, sizeof h);
-  if (!getenv("ZN_EXEC1")) {
-    fprintf(stderr, "zexec2 trace (thread 0 cycles summed over CTAs): other %llu formation %llu lits+prefetch %llu setup %llu jobs %llu rounds %llu flush %llu rest %llu | rounds %llu groups %llu unknown-after-round %llu scan-rounds %llu jobs %llu\n",
-            h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9], h[10], h[11], h[12]);
-    unsigned long long z2[32] = {0};
-    cudaMemcpyToSymbol(g_ztrace, z2, sizeof z2);
-    return;
-  }
-  fprintf(stderr, "zexec trace (thread 0 cycles summed over CTAs): records+extent %llu stage %llu setup %llu passes-other %llu flush %llu rest %llu | passes %llu groups %llu pending-checks %llu\n",
-          h[0], h[1], h[2], h[3], h[4], h[5], h[8], h[9], h[10]);
-  fprintf(stderr, "  per pass: top+long %llu check %llu copy %llu fence+clear %llu append %llu barrier %llu\n", h[11], h[12], h[13], h[14], h[15], h[6]);
+  fprintf(stderr, "zexec2 trace (thread 0 cycles summed over CTAs): other %llu formation %llu lits+prefetch %llu setup %llu jobs %llu rounds %llu flush %llu rest %llu | rounds %llu groups %llu unknown-after-round %llu scan-rounds %llu jobs %llu\n",
+          h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9], h[10], h[11], h[12]);
   unsigned long long z[32] = {0};
   cudaMemcpyToSymbol(g_ztrace, z, sizeof z);
 #endif
@@ -72,56 +57,30 @@ uint32_t pipeline_enqueue(const PipelineLaunch& L, cudaStream_t st, cudaEvent_t*
   // Sequence stage.  The two-phase form runs its state chains ~7x faster per sequence but only kSeq1Lanes blocks per SM at
   // a time; the one-pass form has every block of the batch in flight at once.  So: two-phase when the blocks are long
   // (large blobs: ~10 000 sequences each) or when there are no more of them than two rounds of lanes; one-pass for
-  // batches of very many small blobs (40 000 files of 2-48 KB: 4.2 ms against 6.3).  Development: ZN_SEQ = 0 one-pass /
-  // 1 one-pass with shared-memory tables / 3 two-phase / 4 two-phase with phase-1 tables in global memory.
-  static const int seq_env = getenv("ZN_SEQ") ? atoi(getenv("ZN_SEQ")) : 2;
+  // batches of very many small blobs (40 000 files of 2-48 KB: 4.2 ms against 6.3).
   const uint64_t est_blocks = L.mean_bytes * a.nzb / kZstdBlockMax + a.nzb;
-  const int seq_mode = seq_env == 2 ? ((L.mean_bytes >= (256u << 10) || est_blocks <= 2ull * sms * kSeq1Lanes) ? 3 : 0) : seq_env;
+  const bool large = L.mean_bytes >= (256u << 10);
   uint32_t n_launch = 7;
-  if (seq_mode == 1) k_zseq<<<std::min<uint32_t>((slots + kSeqLanes - 1) / kSeqLanes, sms), 64, kSeqSmem, st>>>(a);
-  else if (seq_mode == 0) k_zseq_g<<<(slots + 31) / 32, 32, 0, st>>>(a, getenv("ZN_SEQ_LDG") ? 0 : 1);
-  else {
-    if (seq_mode == 3) k_zseq1<<<std::min<uint32_t>((slots + kSeq1Lanes - 1) / kSeq1Lanes, sms), 64, kSeq1Smem, st>>>(a);
-    else k_zseq1_g<<<(slots + 31) / 32, 32, 0, st>>>(a);
+  if (large || est_blocks <= 2ull * sms * kSeq1Lanes) {
+    k_zseq1<<<std::min<uint32_t>((slots + kSeq1Lanes - 1) / kSeq1Lanes, sms), 64, kSeq1Smem, st>>>(a);
     if (marks && getenv("ZN_ZPROF_SEQ1")) { cudaEventRecord(marks[8], st); }  // development: end of phase 1
     k_zseq2<<<std::min<uint32_t>((slots + kSeq2Warps - 1) / kSeq2Warps, sms * 16), kSeq2Warps * 32, 0, st>>>(a);
     n_launch = 8;
+  } else {
+    k_zseq_g<<<(slots + 31) / 32, 32, 0, st>>>(a);
   }
   mark();
   k_zlit<<<lit_grid, kLitBlocks * 4, kLitSmem, st>>>(a);
   mark();
   k_zchain<<<(a.nzb + 63) / 64, 64, 0, st>>>(a);
   mark();
-  if (!getenv("ZN_EXEC1")) {  // pointer-jumping exec (ZN_EXEC1=1: the wavefront version)
-    const char* e2 = getenv("ZN_EXEC2");  // development: threads * 10 + CTAs per SM
-    const int shape2 = e2 ? atoi(e2) : (L.mean_bytes >= (256u << 10) ? 5124 : 5123);
-#define ZN_X2(NT, K, GB, MINB) ZN_X2L(NT, K, GB, MINB, GB / 4)
-#define ZN_X2L(NT, K, GB, MINB, LC) k_zexec2<NT, K, GB, MINB, LC><<<std::min<uint32_t>(a.nzb, sms * MINB), NT, sizeof(Exec2Shared<NT, K, GB, LC>), st>>>(a, L.d_out, L.produced, L.exec_counter)
-    switch (shape2) {
-      case 2563: ZN_X2(256, 4, 16384, 3); break;
-      case 5122: ZN_X2(512, 4, 16384, 2); break;
-      case 5123: ZN_X2(512, 2, 16384, 3); break;
-      case 10241: ZN_X2(1024, 2, 16384, 1); break;
-      case 10242: ZN_X2(1024, 2, 16384, 2); break;
-      case 10243: ZN_X2L(1024, 2, 16384, 2, 8192); break;
-      case 5124: ZN_X2L(512, 4, 16384, 2, 8192); break;
-      case 1286: ZN_X2(128, 4, 8192, 6); break;
-      case 1284: ZN_X2(128, 4, 8192, 4); break;
-      default: ZN_X2(256, 4, 16384, 2); break;
-    }
-#undef ZN_X2
-#undef ZN_X2L
-    mark();
-    return n_launch;
-  }
-  const char* ev = getenv("ZN_EXEC");  // development: team shape of the exec kernel
-  const int shape = ev ? atoi(ev) : (L.mean_bytes >= (256u << 10) ? 256 : 128);
-  if (shape == 512)
-    k_zexec<512, 4, 32768, 2><<<std::min<uint32_t>(a.nzb, sms * 2), 512, sizeof(ExecShared<512, 4, 32768>), st>>>(a, L.d_out, L.produced, L.exec_counter);
-  else if (shape == 256)
-    k_zexec<256, 8, 32768, 2><<<std::min<uint32_t>(a.nzb, sms * 2), 256, sizeof(ExecShared<256, 8, 32768>), st>>>(a, L.d_out, L.produced, L.exec_counter);
+  // exec: the team shape follows the mean decoded size, with the same threshold as the sequence stage
+  if (large)
+    k_zexec2<512, 4, 16384, 2, 8192><<<std::min<uint32_t>(a.nzb, sms * 2), 512, sizeof(Exec2Shared<512, 4, 16384, 8192>), st>>>(
+        a, L.d_out, L.produced, L.exec_counter);
   else
-    k_zexec<128, 4, 16384, 4><<<std::min<uint32_t>(a.nzb, sms * 4), 128, sizeof(ExecShared<128, 4, 16384>), st>>>(a, L.d_out, L.produced, L.exec_counter);
+    k_zexec2<512, 2, 16384, 3><<<std::min<uint32_t>(a.nzb, sms * 3), 512, sizeof(Exec2Shared<512, 2, 16384, 4096>), st>>>(
+        a, L.d_out, L.produced, L.exec_counter);
   mark();
   return n_launch;
 }
