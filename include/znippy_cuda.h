@@ -71,14 +71,15 @@ enum {
 enum {
   ZN_CODEC_ZSTD = 1, /* one Zstandard frame per slice */
   ZN_CODEC_LZ4 = 2,  /* one LZ4 frame (independent 64 KiB blocks, content size in header) per slice */
-  /* archive writer only, OR-ed into `codec`: every compressed row's blob is a ZNB1 envelope (see the envelope layer
-   * below) around the frame, or around the raw bytes when the frame did not shrink them (store-if-incompressible);
-   * the index metadata gets znippy_envelope = "ZNB1" and readers resolve such rows through zn_envelope_parse */
+  /* archive writer and compress plans, OR-ed into `codec`: every compressed row's blob is a ZNB1 envelope (see the
+   * envelope layer below) around the frame, or around the raw bytes when the frame did not shrink them
+   * (store-if-incompressible); the index metadata gets znippy_envelope = "ZNB1" and readers resolve such rows through
+   * zn_envelope_parse.  A compress plan makes the same decision on the device and emits the same blob bytes. */
   ZN_CODEC_ENVELOPE = 0x100
 };
 
 typedef struct zn_ctx zn_ctx;   /* one CUDA device + streams + scratch + pinned staging; not thread-safe */
-typedef struct zn_plan zn_plan; /* device-resident descriptors of one decode/verify batch, reusable */
+typedef struct zn_plan zn_plan; /* device-resident descriptors of one decode/verify, hash or compress batch, reusable */
 
 /* ---- library / context ---- */
 int zn_abi_version(void);
@@ -275,7 +276,8 @@ void zn_plan_destroy(zn_plan* plan);
 /* Enqueues the batch on `stream` (cudaStream_t; NULL = the ctx's own stream). Asynchronous.
  * d_out may be NULL only for hash-only plans. */
 int zn_plan_run(zn_plan* plan, const uint8_t* d_blobs, uint8_t* d_out, void* stream);
-/* Waits for the last run and copies results back. status / digests nullable. */
+/* Waits for the last run and copies results back. status / digests nullable.  Compress plans: per-slice statuses, and
+ * the BLAKE3 digests of the source slices when the plan was created with `digests` (otherwise h_digests is untouched). */
 int zn_plan_results(zn_plan* plan, uint32_t* h_status, uint8_t* h_digests);
 /* Kept for ABI stability; has no effect.  (Round 1 offered a stream-overlapped decode/hash schedule here; it measured
  * slower than the stages back to back on every corpus and was replaced by per-row kernel classes.) */
@@ -287,11 +289,11 @@ int zn_plan_set_overlap(zn_plan* plan, int groups);
  *   [2] large raw-block / LZ4 blobs         -> block-parallel team kernel
  *   [3] decoded size <= 64 KiB              -> one-warp teams
  *   [4] the rest                            -> 128-thread teams */
-int zn_plan_class_counts(const zn_plan* plan, uint32_t counts[5]);
+int zn_plan_class_counts(const zn_plan* plan, uint32_t counts[5]); /* ZN_E_STATE on a compress plan */
 /* Rows of class [0] that the device-wide pipeline handed back to the one-team decoder in the last zn_plan_run (anything
  * malformed or beyond the pipeline's budgets; the result is the same, only slower).  Synchronises with the run's
  * stream.  A well-formed batch reports 0 — tests and bench.py check exactly that. */
-int zn_plan_pipeline_fallbacks(zn_plan* plan, uint32_t* rows);
+int zn_plan_pipeline_fallbacks(zn_plan* plan, uint32_t* rows); /* ZN_E_STATE on a compress plan */
 /* kernels launched by one zn_plan_run of this plan */
 uint32_t zn_plan_launches(const zn_plan* plan);
 /* 1 when the plan decodes and hashes in ONE kernel (batches of large, highly compressible blobs: decode warps feed
@@ -299,8 +301,37 @@ uint32_t zn_plan_launches(const zn_plan* plan);
  * and the hash stage is empty. */
 int zn_plan_fused(const zn_plan* plan);
 /* device time of the most recent completed run, per stage, in ms (CUDA events on the run's stream):
- * [0] total, [1] decode stage, [2] hash stage (chunks), [3] tree+compare stage.  Synchronises. */
+ * [0] total, [1] decode stage, [2] hash stage (chunks), [3] tree+compare stage.  Synchronises.
+ * Compress plans: [0] total, [1] compress kernels, [2] hash, [3] sizing and packing. */
 int zn_plan_last_ms(zn_plan* plan, float ms[4]);
+
+/* ---- device-resident compression: the write side of the plan API.  zn_compress_batch copies host slices in, waits for
+ * the frame sizes and copies the frames out; a compress plan takes slices already in HBM (a torch tensor, the output of
+ * a decode plan) and leaves packed blobs in HBM, without waiting.  The frame sizes are only known on the device, so the
+ * layout is made there too: every blob's size from the per-block results, an exclusive scan into offsets, the frames
+ * assembled straight into place.  Blob i is byte for byte the frame zn_compress_batch writes for the same slice, level
+ * and codec when the slice sits at the same 16-byte phase in device memory: the zstd efforts of levels <= 19 stage a
+ * block's window from the 16-byte boundary below it, so their frames depend on that phase (zn_compress_batch keeps a
+ * compact host span's layout from its first byte, and places other batches 16-byte aligned).  With ZN_CODEC_ENVELOPE it is what the archive writer stores for a compressed row: a ZNB1 header and the
+ * frame, or, when the frame is not smaller than the slice, a RAW-payload header and the slice's bytes.
+ * A plan owns its scratch: two plans may run at once on different streams, and zn_compress_batch calls on the same ctx
+ * do not disturb it.  zn_plan_results / zn_plan_launches / zn_plan_last_ms / zn_plan_destroy apply; zn_plan_run on a
+ * compress plan, and zn_plan_run_compress on any other plan, return ZN_E_STATE. ---- */
+
+/* Compress plan over slices that will be resident in HBM: sizes fixed at creation, data supplied per run.  Slice i is
+ * d_src[h_src_off[i] .. + h_src_len[i]) of every run.  `level` and `codec` as for zn_compress_batch; `digests` != 0 also
+ * hashes the source slices (the zn_hash_batch kernels, on the run's stream).  All planning, uploads and allocation
+ * happen here.  NULL, with zn_last_error set, for a slice of 4 GiB or more or a codec other than ZN_CODEC_ZSTD /
+ * ZN_CODEC_LZ4 (optionally | ZN_CODEC_ENVELOPE).  n = 0 is a valid plan. */
+zn_plan* zn_plan_compress(zn_ctx* ctx, uint32_t n, const uint64_t* h_src_off, const uint64_t* h_src_len, int level,
+                          int codec /* ZN_CODEC_ZSTD | ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE */, int digests);
+/* bytes d_dst must hold for any input of these sizes */
+uint64_t zn_plan_compress_capacity(const zn_plan* plan);
+/* Enqueues the batch on `stream` (NULL = ctx stream) and returns without waiting. Blob i lands at
+ * d_dst[d_offsets[i] .. d_offsets[i+1]), back to back with no padding; d_offsets has n+1 entries, written on the
+ * device; d_offsets[n] = total bytes.  d_src offsets and d_dst may have any alignment; d_offsets must be 8-byte aligned
+ * (ZN_E_ARG otherwise).  The call only enqueues kernels: no allocation, no synchronisation. */
+int zn_plan_run_compress(zn_plan* plan, const uint8_t* d_src, uint8_t* d_dst, uint64_t* d_offsets, void* stream);
 
 #ifdef __cplusplus
 }

@@ -13,7 +13,7 @@ from . import build as _build
 ZN_OK, ZN_E_ARG, ZN_E_CUDA, ZN_E_NOMEM, ZN_E_STATE = 0, -1, -2, -3, -4
 S_OK, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_UNSUPPORTED, S_SIZE_MISMATCH = range(6)
 CODEC_ZSTD, CODEC_LZ4 = 1, 2
-CODEC_ENVELOPE = 0x100  # archive writer: wrap compressed rows in ZNB1 (include/znippy_cuda.h)
+CODEC_ENVELOPE = 0x100  # archive writer and compress plans: wrap compressed rows in ZNB1 (include/znippy_cuda.h)
 
 EXPORTS = [
     "zn_abi_version", "zn_device_count", "zn_strerror", "zn_status_name", "zn_ctx_create", "zn_ctx_destroy",
@@ -27,6 +27,7 @@ EXPORTS = [
     "zn_archive_writer_finish", "zn_archive_writer_error", "zn_ctx_pinned_alloc", "zn_ctx_pinned_free",
     "zn_archive_open", "zn_archive_close", "zn_archive_file_count", "zn_archive_file_name", "zn_archive_file_size",
     "zn_archive_extract_files", "zn_archive_set_cache", "zn_archive_cache_stats", "zn_archive_compress_dir", "zn_envelope_parse", "zn_envelope_znb1_header", "zn_envelope_register",
+    "zn_plan_compress", "zn_plan_compress_capacity", "zn_plan_run_compress",
 ]
 
 
@@ -79,6 +80,11 @@ def lib() -> C.CDLL:
     L.zn_plan_destroy.argtypes = [vp]
     L.zn_plan_destroy.restype = None
     L.zn_plan_run.argtypes = [vp, vp, vp, vp]
+    L.zn_plan_compress.argtypes = [vp, u32, vp, vp, C.c_int, C.c_int, C.c_int]
+    L.zn_plan_compress.restype = vp
+    L.zn_plan_compress_capacity.argtypes = [vp]
+    L.zn_plan_compress_capacity.restype = u64
+    L.zn_plan_run_compress.argtypes = [vp, vp, vp, vp, vp]
     L.zn_plan_results.argtypes = [vp, vp, vp]
     L.zn_plan_launches.argtypes = [vp]
     L.zn_plan_launches.restype = u32
@@ -250,6 +256,27 @@ class Plan:
         ex = None if expect is None else u8(expect)
         h = lib().zn_plan_hash(ctx.handle, o.size, ptr(o), ptr(l), ptr(ex))
         return cls(ctx, h, o.size)
+
+    @classmethod
+    def compress(cls, ctx: Ctx, src_off, src_len, level: int = 1, codec: int = CODEC_ZSTD, envelope: bool = False,
+                 digests: bool = True) -> "Plan":
+        """Compress plan over slices resident on the device (zn_plan_compress): slice i = d_src[src_off[i] : + src_len[i]]
+        of every run_compress.  envelope=True: ZNB1 blobs, RAW when the frame does not shrink the slice."""
+        o, l = u64(src_off), u64(src_len)
+        assert l.size == o.size
+        h = lib().zn_plan_compress(ctx.handle, o.size, ptr(o), ptr(l), level, codec | (CODEC_ENVELOPE if envelope else 0),
+                                   1 if digests else 0)
+        return cls(ctx, h, o.size)
+
+    def capacity(self) -> int:
+        """bytes the d_dst of run_compress must hold (zn_plan_compress_capacity)"""
+        return int(lib().zn_plan_compress_capacity(self._h))
+
+    def run_compress(self, d_src_ptr: int, d_dst_ptr: int, d_offsets_ptr: int, stream: int = 0):
+        """Enqueues the compress plan on `stream` (zn_plan_run_compress) and returns at once: blob i lands at
+        d_dst[d_offsets[i] : d_offsets[i + 1]] (n + 1 uint64 offsets, 8-byte aligned)."""
+        self.ctx.check(lib().zn_plan_run_compress(self._h, C.c_void_p(d_src_ptr), C.c_void_p(d_dst_ptr),
+                                                  C.c_void_p(d_offsets_ptr), C.c_void_p(stream)), "zn_plan_run_compress")
 
     def run(self, d_blobs_ptr: int, d_out_ptr: int = 0, stream: int = 0):
         self.ctx.check(lib().zn_plan_run(self._h, C.c_void_p(d_blobs_ptr), C.c_void_p(d_out_ptr), C.c_void_p(stream)),

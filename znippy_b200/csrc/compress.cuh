@@ -1320,5 +1320,47 @@ ZN_HD void zstd_block_header(uint8_t* dst, uint32_t last, uint32_t type, uint32_
   dst[0] = (uint8_t)v; dst[1] = (uint8_t)(v >> 8); dst[2] = (uint8_t)(v >> 16);
 }
 
+// ---- sizes of what the assemble kernels (compress_kernels.cuh) write for a slice of n bytes, from the per-block
+// results alone: a packed layout is computed on the device before any frame byte exists.
+// zstd: meta = the slice's first {payload offset, size} pair (size 0 = raw block); the empty frame is 9 bytes.
+ZN_HD uint64_t zstd_frame_size(uint64_t n, const uint32_t* meta) {
+  if (n == 0) return 9;
+  uint64_t sz = 13;
+  for (uint64_t o = 0, j = 0; o < n; o += kZstdCBlock, j++) {
+    const uint32_t bn = (uint32_t)(n - o < kZstdCBlock ? n - o : kZstdCBlock), c = meta[2 * j + 1];
+    sz += 3 + (c ? c : bn);
+  }
+  return sz;
+}
+// LZ4: csize = the slice's first block size (>= the block's input size means stored); 15-byte header, 4-byte EndMark
+ZN_HD uint64_t lz4_frame_size(uint64_t n, const uint32_t* csize) {
+  uint64_t sz = 15 + 4;
+  for (uint64_t o = 0, j = 0; o < n; o += kLz4Block, j++) {
+    const uint32_t bn = (uint32_t)(n - o < kLz4Block ? n - o : kLz4Block), c = csize[j];
+    sz += 4 + (c < bn ? c : bn);
+  }
+  return sz;
+}
+
+// ZNB1 envelope header (csrc/envelope.cpp, zn_envelope_znb1_header): "ZNB1", payload codec, LEB128 decoded size
+constexpr uint32_t kZnb1Raw = 0, kZnb1Zstd = 1, kZnb1Lz4Frame = 3;  // ZN_PAYLOAD_* of include/znippy_cuda.h
+ZN_HD uint32_t znb1_header_len(uint64_t n) {
+  uint32_t l = 6;
+  for (; n >= 128; n >>= 7) l++;
+  return l;
+}
+ZN_HD uint32_t znb1_header(uint8_t* dst, uint32_t codec, uint64_t n) {
+  dst[0] = 'Z'; dst[1] = 'N'; dst[2] = 'B'; dst[3] = '1';
+  dst[4] = (uint8_t)codec;
+  uint32_t p = 5;
+  do {
+    uint8_t b = (uint8_t)(n & 0x7F);
+    n >>= 7;
+    if (n) b |= 0x80;
+    dst[p++] = b;
+  } while (n);
+  return p;
+}
+
 }  // namespace cz
 }  // namespace zn

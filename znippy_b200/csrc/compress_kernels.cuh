@@ -56,11 +56,10 @@ __global__ void __launch_bounds__(kLz4WarpsPerCta * 32) k_lz4_blocks(const Slice
   }
 }
 
-// ---- LZ4 frame assembly: one CTA per slice
-__global__ void __launch_bounds__(256) k_lz4_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
-                                                      const uint8_t* tmp, const uint32_t* __restrict__ csize, uint8_t* dst_base,
-                                                      uint64_t* dst_len) {
-  const SliceDesc s = slices[blockIdx.x];
+// ---- LZ4 frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_lz4_assemble: one CTA per slice)
+ZN_D void lz4_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base, const uint8_t* tmp,
+                       const uint32_t* __restrict__ csize, uint8_t* dst_base, uint64_t* dst_len) {
+  const SliceDesc s = slices[i];
   uint8_t* dst = dst_base + s.dst_off;
   const Team t{threadIdx.x, blockDim.x};
   if (threadIdx.x == 0) cz::lz4_frame_header(dst, s.src_len);
@@ -81,8 +80,13 @@ __global__ void __launch_bounds__(256) k_lz4_assemble(const SliceDesc* __restric
   }
   if (threadIdx.x == 0) {
     dst[op] = dst[op + 1] = dst[op + 2] = dst[op + 3] = 0;  // EndMark
-    dst_len[blockIdx.x] = op + 4;
+    dst_len[i] = op + 4;
   }
+}
+__global__ void __launch_bounds__(256) k_lz4_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
+                                                      const uint8_t* tmp, const uint32_t* __restrict__ csize, uint8_t* dst_base,
+                                                      uint64_t* dst_len) {
+  lz4_assemble(slices, blockIdx.x, src_base, tmp, csize, dst_base, dst_len);
 }
 
 // ---- zstd: every 128 KiB block of every slice -> staged payload; meta[2j] = payload offset in the slot, meta[2j+1] = size (0 = raw)
@@ -164,17 +168,17 @@ __global__ void __launch_bounds__(32) k_long_blocks(const LongUnit* __restrict__
   }
 }
 
-__global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
-                                                       const uint8_t* tmp, const uint32_t* __restrict__ meta, uint8_t* dst_base,
-                                                       uint64_t* dst_len) {
-  const SliceDesc s = slices[blockIdx.x];
+// ---- zstd frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_zstd_assemble: one CTA per slice)
+ZN_D void zstd_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base, const uint8_t* tmp,
+                        const uint32_t* __restrict__ meta, uint8_t* dst_base, uint64_t* dst_len) {
+  const SliceDesc s = slices[i];
   uint8_t* dst = dst_base + s.dst_off;
   const Team t{threadIdx.x, blockDim.x};
   if (s.src_len == 0) {  // same bytes as libzstd: single-segment, 1-byte content size 0, empty raw last block
     if (threadIdx.x == 0) {
       const uint8_t e[9] = {0x28, 0xB5, 0x2F, 0xFD, 0x20, 0x00, 0x01, 0x00, 0x00};
-      for (int i = 0; i < 9; i++) dst[i] = e[i];
-      dst_len[blockIdx.x] = 9;
+      for (int k = 0; k < 9; k++) dst[k] = e[k];
+      dst_len[i] = 9;
     }
     return;
   }
@@ -196,7 +200,79 @@ __global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restri
       op += 3 + c;
     }
   }
-  if (threadIdx.x == 0) dst_len[blockIdx.x] = op;
+  if (threadIdx.x == 0) dst_len[i] = op;
+}
+__global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
+                                                       const uint8_t* tmp, const uint32_t* __restrict__ meta, uint8_t* dst_base,
+                                                       uint64_t* dst_len) {
+  zstd_assemble(slices, blockIdx.x, src_base, tmp, meta, dst_base, dst_len);
+}
+
+// ---- packed layout (device-resident compress plans): blob i = [ZNB1 header] + frame, or header + the slice's bytes when
+// the envelope stores it RAW; blobs back to back.  One CTA: per tile of slices, every thread sizes one slice from the
+// block results (cz::zstd_frame_size / lz4_frame_size), the CTA scans the sizes, and each thread writes its slice's
+// offset, its frame's destination (past the header) into slices[i].dst_off, the RAW decision and the header.
+constexpr int kLayoutThreads = 1024;
+__global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slices, uint32_t n, const uint32_t* __restrict__ res,
+                                                                uint32_t lz4, uint32_t envelope, uint8_t* dst_base,
+                                                                uint64_t* offsets, uint32_t* raw) {
+  __shared__ uint64_t warp_sum[kLayoutThreads / 32];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  uint64_t carry = 0;  // bytes of the tiles before this one (every thread keeps the same value)
+  for (uint32_t base = 0; base < n; base += kLayoutThreads) {
+    const uint32_t i = base + threadIdx.x;
+    uint64_t sz = 0, len = 0;
+    uint32_t hl = 0, r = 0;
+    if (i < n) {
+      const SliceDesc s = slices[i];
+      len = s.src_len;
+      sz = lz4 ? cz::lz4_frame_size(len, res + s.blk_first) : cz::zstd_frame_size(len, res + 2 * (size_t)s.blk_first);
+      if (envelope) {
+        r = sz >= len;
+        hl = cz::znb1_header_len(len);
+        sz = hl + (r ? len : sz);
+      }
+    }
+    uint64_t incl = sz;  // inclusive scan inside the warp, then over the warps' sums
+#pragma unroll
+    for (uint32_t d = 1; d < 32; d <<= 1) {
+      const uint64_t v = __shfl_up_sync(0xFFFFFFFFu, incl, d);
+      if (lane >= d) incl += v;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    uint64_t before = 0, tile = 0;
+    for (uint32_t k = 0; k < kLayoutThreads / 32; k++) {
+      const uint64_t v = warp_sum[k];
+      before += k < warp ? v : 0;
+      tile += v;
+    }
+    const uint64_t off = carry + before + incl - sz;
+    if (i < n) {
+      offsets[i] = off;
+      slices[i].dst_off = off + hl;
+      raw[i] = r;
+      if (envelope) cz::znb1_header(dst_base + off, r ? cz::kZnb1Raw : (lz4 ? cz::kZnb1Lz4Frame : cz::kZnb1Zstd), len);
+    }
+    carry += tile;
+    __syncthreads();  // warp_sum is rewritten by the next tile
+  }
+  if (threadIdx.x == 0) offsets[n] = carry;
+}
+
+// Frames straight into the packed layout (one CTA per slice); a RAW row gets the slice's bytes instead of its frame.
+// dst_len receives the frame lengths, as from k_zstd_assemble / k_lz4_assemble.
+template <bool LZ4>
+__global__ void __launch_bounds__(256) k_assemble_packed(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
+                                                         const uint8_t* tmp, const uint32_t* __restrict__ res,
+                                                         const uint32_t* __restrict__ raw, uint8_t* dst_base, uint64_t* dst_len) {
+  if (raw[blockIdx.x]) {
+    const SliceDesc s = slices[blockIdx.x];
+    team_copy(Team{threadIdx.x, blockDim.x}, dst_base + s.dst_off, src_base + s.src_off, (uint32_t)s.src_len);
+    return;
+  }
+  if (LZ4) lz4_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
+  else zstd_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
 }
 
 }  // namespace zn

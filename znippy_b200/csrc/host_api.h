@@ -7,6 +7,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <string>
+#include <vector>
 
 #include "zpipe.cuh"
 
@@ -51,6 +52,33 @@ struct CompressScratch {
 };
 void compress_init_attrs();
 size_t compress_bound(size_t n, int codec);  // zn_compress_bound: raw-block fallback makes this exact
+struct SliceDesc;
+// What compress_prepare works out from the slice sizes alone: the effort, the grid, the device descriptors (inside the
+// scratch), and for the long effort the rounds of units, each with its block range and the kernels of its key sort.
+struct CompressPrep {
+  bool lz4 = false;
+  int effort = 0;
+  uint32_t n = 0, nb = 0, grid = 0, sm_count = 0;
+  SliceDesc* d_sl = nullptr;   // n slice descriptors
+  uint32_t* d_meta = nullptr;  // per-block results: zstd {payload offset, size} pairs, LZ4 sizes
+  uint64_t* d_len = nullptr;   // n frame lengths
+  uint32_t* d_raw = nullptr;   // n RAW decisions of the packed layout
+  std::vector<uint32_t> round_first{0}, round_pos, round_blk0, round_nblk, round_sort_launches;
+  uint32_t long_grid = 0;
+  size_t sort_temp = 0;
+  uint32_t launches = 0;  // kernels compress_enqueue launches
+};
+// Plans a batch: grows `cs` to fit, uploads the descriptors on `st` (dst_off[i]: where slice i's frame goes; nullable
+// for a packed layout, which places the frames on the device).  No kernel runs.
+int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const uint64_t* src_off, const uint64_t* src_len,
+                     uint32_t n, int level, int codec, const uint64_t* dst_off, CompressPrep* P, uint32_t* status,
+                     std::string* err);
+// Enqueues the block kernels of a prepared batch on `st` (P.launches kernels): fills the per-block results.
+int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, std::string* err);
+// Enqueues the packed layout and the frame assembly after compress_enqueue (2 kernels; none when P.n == 0):
+// d_offsets[0..n] (exclusive prefix sum of the blob sizes), ZNB1 headers when `envelope`, and every blob in place.
+void compress_pack(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, uint8_t* d_dst,
+                   uint64_t* d_offsets, bool envelope);
 // Compresses n slices resident on the device into frames at d_dst + dst_off[i]; synchronises `st` before returning.
 int compress_run(CompressScratch* cs, cudaStream_t st, int sm_count, const uint8_t* d_src, const uint64_t* src_off,
                  const uint64_t* src_len, uint32_t n, int level, int codec, uint8_t* d_dst, const uint64_t* dst_off,

@@ -2,7 +2,8 @@
 //
 // A zn_ctx owns one device, one stream, device staging buffers and the decode scratch; a zn_plan owns the device
 // descriptor tables of one batch (the index rows blob_offset/blob_size/compressed/uncompressed_size/checksum of
-// znippy-common/src/index.rs:45-52) and can be run any number of times on resident data.  The host-buffer entry
+// znippy-common/src/index.rs:45-52) and can be run any number of times on resident data; a compress plan also owns its
+// compressor scratch, so that it runs on any stream beside other plans and the ctx's own calls.  The host-buffer entry
 // points are the plan API wrapped in one H2D copy before and one D2H copy after.
 #include <cuda_runtime.h>
 
@@ -68,7 +69,7 @@ struct zn_ctx {
   std::string err;
 };
 
-enum PlanKind { PLAN_DECODE_VERIFY = 1, PLAN_HASH = 2 };
+enum PlanKind { PLAN_DECODE_VERIFY = 1, PLAN_HASH = 2, PLAN_COMPRESS = 3 };
 
 // decode classes: every compressed row of a batch is routed by its own sizes (index columns only, no device feedback)
 enum DecClass {
@@ -109,6 +110,14 @@ struct zn_plan {
   uint64_t z_mean = 0;       // mean decoded size of the pipeline rows (picks the exec team size)
   bool uploads_synced = false;  // the plan's arrays (uploaded on the ctx stream) are known to have landed
   uint32_t launches_per_run = 0;
+  // compress plans: their own scratch and descriptors (compress_prepare), the hash plan of the source slices (digests),
+  // ZNB1 packing, the d_dst bytes any input of these sizes may need, and the statuses the planner gave
+  CompressScratch cs;
+  CompressPrep cp;
+  zn_plan* hp = nullptr;
+  bool envelope = false;
+  uint64_t capacity = 0;
+  std::vector<uint32_t> h_status;
 };
 
 static const int kDecodeThreads = 128;
@@ -480,12 +489,14 @@ extern "C" int zn_plan_fused(const zn_plan* p) { return p && p->cls_off[DC_BIGPA
 
 extern "C" int zn_plan_class_counts(const zn_plan* p, uint32_t counts[5]) {
   if (!p || !counts) return ZN_E_ARG;
+  if (p->kind == PLAN_COMPRESS) return ZN_E_STATE;
   for (int k = 0; k < DC_COUNT; k++) counts[k] = p->cls_off[k + 1] - p->cls_off[k];
   return ZN_OK;
 }
 
 extern "C" int zn_plan_pipeline_fallbacks(zn_plan* p, uint32_t* rows) {
   if (!p || !rows) return ZN_E_ARG;
+  if (p->kind == PLAN_COMPRESS) return ZN_E_STATE;
   *rows = 0;
   if (!p->nzb || !p->ran) return ZN_OK;
   cudaSetDevice(p->ctx->device);
@@ -507,6 +518,8 @@ extern "C" void zn_plan_destroy(zn_plan* p) {
     if (q) cudaFreeAsync(q, p->ctx->stream);
   for (auto& e : p->ev)
     if (e) cudaEventDestroy(e);
+  if (p->hp) zn_plan_destroy(p->hp);
+  p->cs.release();
   delete p;
 }
 
@@ -581,6 +594,7 @@ static int run_pipeline(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, cuda
 
 extern "C" int zn_plan_run(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, void* stream_v) {
   if (!p) return ZN_E_ARG;
+  if (p->kind == PLAN_COMPRESS) return ZN_E_STATE;
   zn_ctx* c = p->ctx;
   cudaSetDevice(c->device);
   cudaStream_t st = stream_v ? (cudaStream_t)stream_v : c->stream;
@@ -687,6 +701,11 @@ extern "C" int zn_plan_results(zn_plan* p, uint32_t* h_status, uint8_t* h_digest
   if (!p->ran) return ZN_E_STATE;
   zn_ctx* c = p->ctx;
   cudaSetDevice(c->device);
+  if (p->kind == PLAN_COMPRESS) {
+    ZN_CUDA(c, cudaStreamSynchronize(p->last_stream));
+    if (h_status && p->n) memcpy(h_status, p->h_status.data(), (size_t)p->n * 4);
+    return h_digests && p->hp ? zn_plan_results(p->hp, nullptr, h_digests) : ZN_OK;
+  }
   if (h_status && p->n) ZN_CUDA(c, cudaMemcpyAsync(h_status, p->d_status, (size_t)p->n * 4, cudaMemcpyDeviceToHost, p->last_stream));
   if (h_digests && p->n) ZN_CUDA(c, cudaMemcpyAsync(h_digests, p->d_digests, (size_t)p->n * 32, cudaMemcpyDeviceToHost, p->last_stream));
   uint32_t stall = 0;
@@ -708,6 +727,85 @@ extern "C" int zn_plan_last_ms(zn_plan* p, float ms[4]) {
   ZN_CUDA(c, cudaEventElapsedTime(&ms[1], p->ev[0], p->ev[1]));
   ZN_CUDA(c, cudaEventElapsedTime(&ms[2], p->ev[1], p->ev[2]));
   ZN_CUDA(c, cudaEventElapsedTime(&ms[3], p->ev[2], p->ev[3]));
+  return ZN_OK;
+}
+
+// --------------------------------------------------------------------------------------------- compress plans
+extern "C" zn_plan* zn_plan_compress(zn_ctx* c, uint32_t n, const uint64_t* h_src_off, const uint64_t* h_src_len, int level,
+                                     int codec, int digests) {
+  if (!c) return nullptr;
+  const int base = codec & ~ZN_CODEC_ENVELOPE;
+  if (base != ZN_CODEC_ZSTD && base != ZN_CODEC_LZ4) {
+    c->err = "zn_plan_compress: codec must be ZN_CODEC_ZSTD or ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE";
+    return nullptr;
+  }
+  if (n && (!h_src_off || !h_src_len)) { c->err = "zn_plan_compress: null size arrays"; return nullptr; }
+  cudaSetDevice(c->device);
+  zn_plan* p = new zn_plan();
+  p->ctx = c;
+  p->kind = PLAN_COMPRESS;
+  p->n = n;
+  p->envelope = (codec & ZN_CODEC_ENVELOPE) != 0;
+  p->h_status.assign(n, 0);
+  for (uint32_t i = 0; i < n; i++) {
+    uint8_t hdr[ZN_ENVELOPE_ZNB1_MAX_HEADER];
+    p->capacity += p->envelope ? zn_envelope_znb1_header(ZN_PAYLOAD_RAW, h_src_len[i], hdr, sizeof hdr) + h_src_len[i]
+                               : compress_bound(h_src_len[i], base);
+  }
+  std::string err;
+  if (compress_prepare(&p->cs, c->stream, c->sm_count, h_src_off, h_src_len, n, level, base, nullptr, &p->cp, p->h_status.data(),
+                       &err) != 0) {
+    c->err = "zn_plan_compress: " + err;
+    zn_plan_destroy(p);
+    return nullptr;
+  }
+  if (digests && n && !(p->hp = zn_plan_hash(c, n, h_src_off, h_src_len, nullptr))) {  // c->err says why
+    zn_plan_destroy(p);
+    return nullptr;
+  }
+  bool ok = true;
+  for (int i = 0; ok && i < 4; i++) ok = cudaEventCreate(&p->ev[i]) == cudaSuccess;
+  if (ok) ok = cudaStreamSynchronize(c->stream) == cudaSuccess;  // descriptors and units have landed
+  if (!ok) {
+    c->err = std::string("zn_plan_compress: ") + cudaGetErrorString(cudaGetLastError());
+    zn_plan_destroy(p);
+    return nullptr;
+  }
+  p->uploads_synced = true;
+  return p;
+}
+
+extern "C" uint64_t zn_plan_compress_capacity(const zn_plan* p) { return p && p->kind == PLAN_COMPRESS ? p->capacity : 0; }
+
+extern "C" int zn_plan_run_compress(zn_plan* p, const uint8_t* d_src, uint8_t* d_dst, uint64_t* d_offsets, void* stream_v) {
+  if (!p) return ZN_E_ARG;
+  if (p->kind != PLAN_COMPRESS) return ZN_E_STATE;
+  zn_ctx* c = p->ctx;
+  if (!d_offsets || ((uintptr_t)d_offsets & 7) || (p->n && (!d_src || !d_dst))) {
+    c->err = "zn_plan_run_compress: null pointer or d_offsets not 8-byte aligned";
+    return ZN_E_ARG;
+  }
+  cudaSetDevice(c->device);
+  cudaStream_t st = stream_v ? (cudaStream_t)stream_v : c->stream;
+  ZN_CUDA(c, cudaEventRecord(p->ev[0], st));
+  if (compress_enqueue(&p->cs, p->cp, st, d_src, &c->err) != 0) return ZN_E_CUDA;
+  ZN_CUDA(c, cudaEventRecord(p->ev[1], st));
+  uint32_t hash_launches = 0;
+  if (p->hp) {  // digests of the source slices: the hash plan's kernels, on the same stream
+    const int rc = zn_plan_run(p->hp, d_src, nullptr, st);
+    if (rc != ZN_OK) return rc;
+    hash_launches = p->hp->launches_per_run;
+  }
+  ZN_CUDA(c, cudaEventRecord(p->ev[2], st));
+  if (p->n) compress_pack(&p->cs, p->cp, st, d_src, d_dst, d_offsets, p->envelope);
+  else ZN_CUDA(c, cudaMemsetAsync(d_offsets, 0, 8, st));
+  ZN_CUDA(c, cudaEventRecord(p->ev[3], st));
+  ZN_CUDA(c, cudaGetLastError());
+  const uint32_t launches = p->cp.launches + (p->n ? 2u : 0u);
+  c->launches += launches;  // zn_plan_run counted the hash kernels
+  p->launches_per_run = launches + hash_launches;
+  p->last_stream = st;
+  p->ran = true;
   return ZN_OK;
 }
 
