@@ -232,6 +232,31 @@ const char* zn_archive_file_name(const zn_archive* a, uint64_t i, uint64_t* size
 int zn_archive_file_size(const zn_archive* a, const char* path, uint64_t* size); /* 1 = present */
 int zn_archive_extract_files(zn_ctx* ctx, zn_archive* a, const char* const* paths, uint32_t n, uint8_t* out_base,
                              const uint64_t* out_off, uint32_t* file_status);
+/* Byte ranges of files (HTTP Range requests, the zip central directory at the end of a jar or wheel).  Request i asks
+ * for bytes [offset[i], offset[i] + length[i]) of file paths[i], clamped at the file's end as pread clamps: an offset at
+ * or past the end, or a zero length, gives got[i] = 0 with status 0.  The bytes go to out_base + out_off[i] ..; got[i] =
+ * bytes written, and out_base is written only inside [out_off[i], out_off[i] + got[i]).  file_status[i] as
+ * zn_archive_extract_files (2 | (blob status << 16) for the first failing chunk of the request, which then gets got = 0).
+ * All requests of a call are one batch:
+ *   - only the chunks a range touches are read; a chunk several requests touch is decoded once;
+ *   - a chunk covered in full is decoded and checked exactly as extract_files decodes it (no digest compare);
+ *   - a chunk covered in part is decoded only up to the end of the block that holds the furthest byte any request of the
+ *     call needs from it (at most one 128 KiB zstd block or one LZ4 frame block more).  Only that prefix is checked:
+ *     damage past the block where decoding stopped goes unseen, and the content checksum is not checked.  A frame that
+ *     ends before that point gives ZN_S_SIZE_MISMATCH.  A raw LZ4 block chunk is one block and decodes whole;
+ *   - store-as-is chunks and ZNB1 chunks with a RAW payload never reach the GPU: only the requested bytes are pread,
+ *     straight into out_base.  A call whose ranges lie only in such chunks launches no kernel;
+ *   - with the LRU on, cached chunks are copied from it, chunks decoded in full are inserted, partial chunks never.
+ * stats (nullable) counts what the call did. */
+typedef struct {
+  uint64_t rows_decoded;    /* distinct index rows run through a decoder in this call */
+  uint64_t bytes_decoded;   /* bytes those decoders produced (whole rows + edge-row prefixes) */
+  uint64_t blob_bytes_read; /* bytes pread from the archive */
+  uint64_t rows_from_cache; /* rows answered by the LRU of decoded slices */
+} zn_range_stats;
+int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* const* paths, const uint64_t* offset,
+                           const uint64_t* length, uint32_t n, uint8_t* out_base, const uint64_t* out_off, uint64_t* got,
+                           uint32_t* file_status, zn_range_stats* stats /* nullable */);
 /* LRU of decoded slices for a serving process (SURVEY §8f-2): with a non-zero budget, every slice extract_files decodes is
  * kept in host memory (keyed by index row, evicted least-recently-used first) and later requests for it skip pread, H2D
  * and the decode.  0 (the default) turns it off and drops what is cached.  stats: hits, misses, evictions, bytes, slices. */

@@ -26,7 +26,7 @@ EXPORTS = [
     "zn_index_writer_finish", "zn_archive_decompress", "zn_archive_writer_create", "zn_archive_writer_add",
     "zn_archive_writer_finish", "zn_archive_writer_error", "zn_ctx_pinned_alloc", "zn_ctx_pinned_free",
     "zn_archive_open", "zn_archive_close", "zn_archive_file_count", "zn_archive_file_name", "zn_archive_file_size",
-    "zn_archive_extract_files", "zn_archive_set_cache", "zn_archive_cache_stats", "zn_archive_compress_dir", "zn_envelope_parse", "zn_envelope_znb1_header", "zn_envelope_register",
+    "zn_archive_extract_files", "zn_archive_read_ranges", "zn_archive_set_cache", "zn_archive_cache_stats", "zn_archive_compress_dir", "zn_envelope_parse", "zn_envelope_znb1_header", "zn_envelope_register",
     "zn_plan_compress", "zn_plan_compress_capacity", "zn_plan_run_compress",
 ]
 
@@ -136,6 +136,7 @@ def lib() -> C.CDLL:
     L.zn_archive_file_name.restype = C.c_char_p
     L.zn_archive_file_size.argtypes = [vp, C.c_char_p, C.POINTER(u64)]
     L.zn_archive_extract_files.argtypes = [vp, vp, vp, u32, vp, vp, vp]
+    L.zn_archive_read_ranges.argtypes = [vp, vp, vp, vp, vp, u32, vp, vp, vp, vp, vp]
     L.zn_archive_writer_create.argtypes = [vp, C.c_char_p, C.c_int, C.c_int, C.c_int, sz]
     L.zn_archive_writer_create.restype = vp
     L.zn_archive_writer_add.argtypes = [vp, C.c_char_p, vp, u64, C.c_int, C.c_int8, C.c_char_p]

@@ -413,6 +413,53 @@ class ZnippyArchive:
                 res.append(out[int(offs[i]): int(offs[i]) + sizes[i]].tobytes())
         return res
 
+    def read_range(self, relative_path: str, offset: int, length: int) -> bytes:
+        """Bytes [offset, offset + length) of one file, clamped at its end like pread; raises as extract_file does."""
+        r = self.read_ranges([(relative_path, offset, length)])[0]
+        if isinstance(r, Exception):
+            raise r
+        return r
+
+    def read_ranges(self, requests, stats: bool = False):
+        """One batch of (path, offset, length) byte ranges (zn_archive_read_ranges): only the chunks a range touches are
+        read, and an edge chunk is decoded only up to the block that holds the range's end.  Returns a list of
+        bytes | Exception (KeyError: no such file, CodecError: a chunk failed), and with stats=True also the counters
+        {rows_decoded, bytes_decoded, blob_bytes_read, rows_from_cache} of the call."""
+        import ctypes as C
+
+        from . import _native as N
+        ctx = self.ctx or default_ctx()
+        n = len(requests)
+        off = np.array([int(r[1]) for r in requests] or [0], np.uint64)
+        length = np.array([int(r[2]) for r in requests] or [0], np.uint64)
+        sizes = [self.file_size(r[0]) for r in requests]
+        outs = np.zeros(max(n, 1), np.uint64)
+        cur = 0
+        for i, sz in enumerate(sizes):  # room for the clamped length only
+            outs[i] = cur
+            if sz is not None and int(off[i]) < sz:
+                cur += min(int(length[i]), sz - int(off[i]))
+        out = np.zeros(max(cur, 1), np.uint8)
+        got = np.zeros(max(n, 1), np.uint64)
+        st = np.zeros(max(n, 1), np.uint32)
+        counters = np.zeros(4, np.uint64)
+        arr = (C.c_char_p * max(n, 1))(*[r[0].encode() for r in requests])
+        ctx.check(N.lib().zn_archive_read_ranges(ctx.handle, self._h, arr, N.ptr(off), N.ptr(length), n, N.ptr(out),
+                                                 N.ptr(outs), N.ptr(got), N.ptr(st), N.ptr(counters)),
+                  "zn_archive_read_ranges")
+        res = []
+        for i, r in enumerate(requests):
+            if st[i] == 1:
+                res.append(KeyError(f"file not found in archive: {r[0]}"))
+            elif st[i] != 0:
+                res.append(codec.CodecError(int(st[i]) >> 16, f"decompress chunk of {r[0]}"))
+            else:
+                res.append(out[int(outs[i]): int(outs[i]) + int(got[i])].tobytes())
+        if stats:
+            return res, dict(zip(("rows_decoded", "bytes_decoded", "blob_bytes_read", "rows_from_cache"),
+                                 (int(x) for x in counters)))
+        return res
+
 
 # --------------------------------------------------------------------------------------------- write side
 

@@ -1664,3 +1664,251 @@ extern "C" int zn_archive_extract_files(zn_ctx* ctx, zn_archive* a, const char* 
   zn_ctx_pinned_free(stage);
   return rc;
 }
+
+// Windowed decode of znippy_cuda.cu (declared in host_api.h, which needs the CUDA headers this file is built without).
+extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                 uint8_t* pack, uint32_t* status, uint64_t* produced);
+
+namespace {
+struct PinnedBuf {  // pinned host buffer from the process-wide cache, returned on scope exit
+  uint8_t* p = nullptr;
+  ~PinnedBuf() { if (p) zn_ctx_pinned_free(p); }
+};
+bool pread_all(int fd, uint8_t* dst, uint64_t len, uint64_t off) {
+  uint64_t done = 0;
+  while (done < len) {
+    const ssize_t r = pread(fd, dst + done, len - done, (off_t)(off + done));
+    if (r <= 0) return false;
+    done += (uint64_t)r;
+  }
+  return true;
+}
+}  // namespace
+
+// Byte ranges (include/znippy_cuda.h): each request is cut into pieces, one per index row it overlaps; the distinct rows
+// are answered from the LRU, pread in part (store-as-is rows, RAW payloads) or decoded, full rows in full and edge rows
+// up to the furthest byte any piece needs (zn_decode_windows).  Pieces are written only once every row of their request
+// is known to be good.
+extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* const* paths, const uint64_t* offset,
+                                      const uint64_t* length, uint32_t n, uint8_t* out_base, const uint64_t* out_off,
+                                      uint64_t* got, uint32_t* file_status, zn_range_stats* stats) {
+  if (!ctx || !a || (n && (!paths || !offset || !length || !out_base || !out_off || !got || !file_status))) return ZN_E_ARG;
+  zn_range_stats S;
+  memset(&S, 0, sizeof S);
+  const IndexImpl& I = a->index->ix;
+  struct Piece {
+    uint32_t req, row;     // row: index into `rows` below
+    uint64_t s, e, dst;    // bytes [s, e) of the row go to out_base + dst
+    uint64_t at;           // where the bytes wait: offset in `cached` or in the decode pack
+  };
+  struct Row {
+    uint64_t r, need = 0;  // index row; bytes [0, need) of it are needed
+    int kind = 0;          // 0 decode, 1 pread (store-as-is or RAW payload), 2 cache, 3 failed before any decode
+    uint64_t raw_off = 0;  // kind 1: archive offset of the row's first content byte
+    uint32_t status = 0, flag = 0;
+    uint64_t payload_off = 0, payload_len = 0;
+  };
+  std::vector<Piece> pieces;
+  std::vector<Row> rows;
+  std::unordered_map<uint64_t, uint32_t> row_at;
+  for (uint32_t k = 0; k < n; k++) {
+    got[k] = 0;
+    file_status[k] = 0;
+    auto it = a->files.find(paths[k]);
+    if (it == a->files.end()) { file_status[k] = 1; continue; }
+    const zn_archive::FileEntry& F = it->second;
+    if (length[k] == 0 || offset[k] >= F.size) continue;
+    const uint64_t lo = offset[k], hi = lo + std::min(length[k], F.size - lo);
+    got[k] = hi - lo;
+    // the last row starting at or before lo, then forward while rows start before hi
+    auto rit = std::upper_bound(F.rows.begin(), F.rows.end(), lo, [&](uint64_t v, uint64_t r) { return v < I.col[2][r]; });
+    if (rit != F.rows.begin()) --rit;
+    for (; rit != F.rows.end() && I.col[2][*rit] < hi; ++rit) {
+      const uint64_t r = *rit, fo = I.col[2][r], s = std::max(lo, fo), e = std::min(hi, fo + I.col[3][r]);
+      if (s >= e) continue;
+      auto ins = row_at.emplace(r, (uint32_t)rows.size());
+      if (ins.second) { rows.emplace_back(); rows.back().r = r; }
+      Row& R = rows[ins.first->second];
+      R.need = std::max(R.need, e - fo);
+      pieces.push_back({k, ins.first->second, s - fo, e - fo, out_off[k] + (s - lo), 0});
+    }
+  }
+  // cached rows: the bytes of their pieces are copied out under the lock (a later insertion may evict the row)
+  std::vector<uint8_t> cached;
+  zn_archive::Cache& K = a->cache;
+  if (K.budget && !rows.empty()) {
+    std::lock_guard<std::mutex> g(K.mu);
+    for (Row& R : rows) {
+      auto c = K.at.find(R.r);
+      if (c == K.at.end()) { K.misses++; continue; }
+      K.lru.splice(K.lru.begin(), K.lru, c->second);
+      K.hits++;
+      R.kind = 2;
+      S.rows_from_cache++;
+    }
+    for (Piece& P : pieces) {
+      if (rows[P.row].kind != 2) continue;
+      const std::vector<uint8_t>& v = K.at[rows[P.row].r]->second;
+      P.at = cached.size();
+      cached.insert(cached.end(), v.begin() + (long)P.s, v.begin() + (long)P.e);
+    }
+  }
+  // envelopes and store-as-is rows: which rows reach a decoder, and with which payload
+  static const uint8_t flag_of[5] = {0, 1, 3, 1, 2};  // ZN_PAYLOAD_* -> compressed value of a bare payload
+  for (Row& R : rows) {
+    if (R.kind == 2) continue;
+    const uint64_t bo = I.col[0][R.r], bl = I.col[1][R.r], ul = I.col[3][R.r];
+    const uint8_t ce = I.comp_eff[R.r];
+    R.payload_off = 0;
+    R.payload_len = bl;
+    R.flag = ce;
+    if (ce == 4) {
+      // ZNB1 and bare frames are parsed from their first bytes (the parser reads no further for them, so it is told
+      // the blob's full length); a foreign envelope gets the whole blob
+      std::vector<uint8_t> head((size_t)std::min<uint64_t>(bl, 64));
+      if (!pread_all(a->fd, head.data(), head.size(), bo)) return ZN_E_ARG;
+      S.blob_bytes_read += head.size();
+      uint32_t magic = 0;
+      if (head.size() >= 4) memcpy(&magic, head.data(), 4);
+      const bool header_only = magic == 0x31424E5Au /* "ZNB1" */ || magic == 0xFD2FB528u || magic == 0x184D2204u ||
+                               (magic & 0xFFFFFFF0u) == 0x184D2A50u;
+      if (!header_only && head.size() < bl) {
+        head.resize(bl);
+        if (!pread_all(a->fd, head.data(), bl, bo)) return ZN_E_ARG;
+        S.blob_bytes_read += bl;
+      }
+      zn_envelope e;
+      const int erc = zn_envelope_parse(head.data(), header_only ? bl : head.size(), &e);
+      if (erc != ZN_OK || (e.out_len != ~0ull && e.out_len != ul)) {
+        R.kind = 3;
+        R.status = erc != ZN_OK ? ZN_S_UNSUPPORTED : ZN_S_SIZE_MISMATCH;
+        continue;
+      }
+      R.payload_off = e.payload_off;
+      R.payload_len = e.payload_len;
+      R.flag = flag_of[e.codec];
+    }
+    if (R.flag == 0) {
+      if (R.payload_len != ul) { R.kind = 3; R.status = ZN_S_SIZE_MISMATCH; continue; }  // as zn_decode_verify_batch
+      R.kind = 1;
+      R.raw_off = bo + R.payload_off;
+    }
+  }
+  // decode rows: whole blobs into pinned staging, 16 bytes apart (room for the magic of a magicless zstd payload)
+  std::vector<uint32_t> dec;
+  uint64_t in_cur = 0;
+  for (uint32_t j = 0; j < (uint32_t)rows.size(); j++)
+    if (rows[j].kind == 0) { dec.push_back(j); in_cur += 16 + ((I.col[1][rows[j].r] + 15) & ~15ull); }
+  std::vector<uint8_t> full_row(rows.size(), 0);  // decoded in full (and so a candidate for the cache)
+  PinnedBuf pack;  // the decoded bytes of every piece of a decode row
+  if (!dec.empty()) {
+    const uint32_t nd = (uint32_t)dec.size();
+    std::vector<uint64_t> bo(nd), bl(nd), ol(nd), stop(nd), prod(nd), w_off, w_len;
+    std::vector<uint8_t> cf(nd);
+    std::vector<uint32_t> st(nd), w_row, dec_at(rows.size(), 0);
+    PinnedBuf stage_buf;
+    uint8_t* stage = stage_buf.p = (uint8_t*)zn_ctx_pinned_alloc(in_cur + 4096);
+    if (!stage) return ZN_E_NOMEM;
+    uint64_t cur = 0;
+    for (uint32_t j = 0; j < nd; j++) {
+      Row& R = rows[dec[j]];
+      dec_at[dec[j]] = j;
+      bo[j] = cur + 16 + R.payload_off;
+      bl[j] = R.payload_len;
+      cf[j] = (uint8_t)R.flag;
+      ol[j] = I.col[3][R.r];
+      stop[j] = R.need;
+      full_row[dec[j]] = R.need >= ol[j] || R.flag == 2;
+      cur += 16 + ((I.col[1][R.r] + 15) & ~15ull);
+    }
+    {
+      std::atomic<size_t> next{0};
+      std::atomic<int> io_err{0};
+      auto body = [&] {
+        for (size_t j; (j = next.fetch_add(1)) < nd;) {
+          const Row& R = rows[dec[j]];
+          if (!pread_all(a->fd, stage + bo[j] - R.payload_off, I.col[1][R.r], I.col[0][R.r])) io_err = 1;
+        }
+      };
+      std::vector<std::thread> ts;
+      for (int t = 1; t < (nd >= 16 ? 4 : 1); t++) ts.emplace_back(body);
+      body();
+      for (auto& t : ts) t.join();
+      if (io_err) return ZN_E_ARG;
+    }
+    for (uint32_t j = 0; j < nd; j++) {
+      S.blob_bytes_read += I.col[1][rows[dec[j]].r];
+      if (cf[j] == 3) {  // magicless zstd payload: decoded as magic + payload
+        static const uint8_t magic[4] = {0x28, 0xB5, 0x2F, 0xFD};
+        bo[j] -= 4;
+        bl[j] += 4;
+        memcpy(stage + bo[j], magic, 4);
+        cf[j] = 1;
+      }
+    }
+    // windows: one per piece, plus the whole row where a full row goes into the cache
+    uint64_t packed = 0;
+    for (Piece& P : pieces) {
+      if (rows[P.row].kind != 0) continue;
+      w_row.push_back(dec_at[P.row]); w_off.push_back(P.s); w_len.push_back(P.e - P.s);
+      P.at = packed;
+      packed += P.e - P.s;
+    }
+    std::vector<uint64_t> whole_at(nd, ~0ull);
+    if (K.budget)
+      for (uint32_t j = 0; j < nd; j++)
+        if (full_row[dec[j]] && ol[j] <= K.budget) {
+          w_row.push_back(j); w_off.push_back(0); w_len.push_back(ol[j]);
+          whole_at[j] = packed;
+          packed += ol[j];
+        }
+    if (!(pack.p = (uint8_t*)zn_ctx_pinned_alloc(packed + 64))) return ZN_E_NOMEM;
+    const int rc = zn_decode_windows(ctx, stage, bo.data(), bl.data(), cf.data(), ol.data(), stop.data(), nd, w_row.data(),
+                                     w_off.data(), w_len.data(), (uint32_t)w_row.size(), pack.p, st.data(), prod.data());
+    if (rc != ZN_OK) return rc;
+    for (uint32_t j = 0; j < nd; j++) {
+      rows[dec[j]].status = st[j];
+      S.rows_decoded++;
+      S.bytes_decoded += prod[j];
+    }
+    if (K.budget) {
+      std::lock_guard<std::mutex> g(K.mu);
+      for (uint32_t j = 0; j < nd; j++) {
+        const uint64_t r = rows[dec[j]].r;
+        if (whole_at[j] == ~0ull || st[j] != ZN_S_OK || K.at.count(r)) continue;
+        while (K.used + ol[j] > K.budget && !K.lru.empty()) {  // evict from the cold end
+          K.used -= K.lru.back().second.size();
+          K.at.erase(K.lru.back().first);
+          K.lru.pop_back();
+          K.evictions++;
+        }
+        K.lru.emplace_front(r, std::vector<uint8_t>(pack.p + whole_at[j], pack.p + whole_at[j] + ol[j]));
+        K.at[r] = K.lru.begin();
+        K.used += ol[j];
+      }
+    }
+  }
+  // request statuses: the first failing row of each request, in file order
+  for (const Piece& P : pieces) {
+    const Row& R = rows[P.row];
+    if (R.status != ZN_S_OK && file_status[P.req] == 0) {
+      file_status[P.req] = 2u | (R.status << 16);
+      got[P.req] = 0;
+    }
+  }
+  // the bytes of good requests: decoded and cached pieces, and store-as-is / RAW bytes pread straight into place
+  for (const Piece& P : pieces) {
+    if (file_status[P.req] != 0) continue;
+    const Row& R = rows[P.row];
+    if (R.kind == 0) memcpy(out_base + P.dst, pack.p + P.at, P.e - P.s);
+    if (R.kind == 2) memcpy(out_base + P.dst, cached.data() + P.at, P.e - P.s);
+    if (R.kind == 1) {
+      if (!pread_all(a->fd, out_base + P.dst, P.e - P.s, R.raw_off + P.s)) return ZN_E_ARG;
+      S.blob_bytes_read += P.e - P.s;
+    }
+  }
+  if (stats) *stats = S;
+  return ZN_OK;
+}

@@ -21,12 +21,15 @@ ZN_D void warp_stage(uint8_t* dst, const uint8_t* src, uint32_t n, uint32_t lane
 // NT threads per team; the CTA claims KB work items per atomic and its first KB warps fetch their descriptors (and
 // stage blobs <= kSrcSmall) in parallel, so the three dependent global round trips (counter -> list -> descriptor ->
 // bytes) are paid once per KB blobs instead of once per blob.  This is what bounds the 100 000 x 10 KiB-file corpus.
-template <int NT, int KB>
+// kStop (range reads): blob i is decoded only up to the block that reaches stop[i] (zs::StopAt) into its full-size
+// output; it fails with S_SIZE_MISMATCH when its frames end before stop[i].
+template <int NT, int KB, bool kStop = false>
 __global__ void __launch_bounds__(NT, NT == 32 ? 16 : 512 / NT) k_decode(const BlobDesc* __restrict__ blobs, const uint32_t* __restrict__ list,
                                                          uint32_t n_list, const uint8_t* blobs_base, uint8_t* out_base,
                                                          uint8_t* lit_scratch, uint32_t* status, uint32_t* produced,
                                                          uint32_t* work_counter, uint32_t* cvs, uint32_t one,
-                                                         const uint32_t* only_if, uint32_t only_stride) {
+                                                         const uint32_t* only_if, uint32_t only_stride,
+                                                         const uint32_t* __restrict__ stop = nullptr) {
   __shared__ DecShared sh;
   __shared__ uint32_t s_base;
   __shared__ BlobDesc s_desc[KB];
@@ -79,12 +82,17 @@ __global__ void __launch_bounds__(NT, NT == 32 ? 16 : 512 / NT) k_decode(const B
           __syncthreads();
           src = s_src + 16;
         }
-        if (d.flags & F_LZ4_BLOCK) {
+        if (kStop) {
+          zs::StopAt h;
+          h.stop = stop[blob];
+          st = decode_blob(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, lit, predef, &got, h);
+          if (st == S_OK && got < h.stop) st = S_SIZE_MISMATCH;
+        } else if (d.flags & F_LZ4_BLOCK) {
           st = decode_lz4_block(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, &got);
         } else {
           st = decode_blob(t, &sh, src, (uint32_t)d.src_len, out_base + d.dst_off, (uint32_t)d.dst_cap, lit, predef, &got);
         }
-        if (st == S_OK && got != (uint32_t)d.dst_cap) st = S_SIZE_MISMATCH;
+        if (!kStop && st == S_OK && got != (uint32_t)d.dst_cap) st = S_SIZE_MISMATCH;
       }
       ZN_TP(22);
       if (kWide && threadIdx.x < kBulkIssuers) bulk_wait_all();  // bulk stores read the tile: drain before it is reused

@@ -104,3 +104,17 @@ void pipeline_trace_dump();  // development builds (ZN_TRACE_BUILD=1): prints an
 }  // namespace zp
 
 }  // namespace zn
+
+// ---------------------------------------------------------------------------------------------- znippy_cuda.cu
+// Windowed host-buffer decode behind zn_archive_read_ranges (container.cpp declares it too: it is compiled without the
+// CUDA headers).  Row i (compressed[i]: 1 = frame, 2 = raw LZ4 block) decodes into device scratch of out_len[i] bytes:
+//   stop[i] < out_len[i] and a frame: only up to the block that reaches stop[i] (k_decode<.., true>), no digest tree and
+//                                     no content checksum; S_SIZE_MISMATCH when the frames end before stop[i];
+//   otherwise:                        in full, through the plan of zn_decode_verify_batch (no expected digests).
+// Then only the n_win windows come back: win_len[w] bytes at offset win_off[w] of row win_row[w], packed back to back
+// into `pack` (host memory, pinned for speed).  status[i] as zn_decode_verify_batch; produced[i] = bytes decoded.
+struct zn_ctx;
+extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                 uint8_t* pack, uint32_t* status, uint64_t* produced);

@@ -114,8 +114,11 @@ ZN_HD uint32_t decode_block(const Team& t, DecShared* sh, const uint8_t* p, uint
   return S_OK;
 }
 
+// `hook` only decides where to stop (zs::stop_here): after the data block that reaches a StopAt's stop, S_OK without
+// the content-size comparison.
+template <class Hook>
 ZN_HD uint32_t decode_frame(const Team& t, DecShared* sh, const uint8_t* src, uint32_t src_len, uint8_t* out,
-                            uint32_t cap, uint32_t* produced) {
+                            uint32_t cap, uint32_t* produced, const Hook& hook) {
   *produced = 0;
   if (src_len < 7) return S_DECODE_ERROR;
   if (ld32le(src) != 0x184D2204u) return S_UNSUPPORTED;
@@ -157,6 +160,7 @@ ZN_HD uint32_t decode_frame(const Team& t, DecShared* sh, const uint8_t* src, ui
       if (rc != S_OK) return rc;
     }
     *produced = es.pos;
+    if (zs::stop_here(hook, es.pos)) return S_OK;
     ip += n;
     if (bchk) {
       if (src_len - ip < 4) return S_DECODE_ERROR;
@@ -171,6 +175,10 @@ ZN_HD uint32_t decode_frame(const Team& t, DecShared* sh, const uint8_t* src, ui
   if (has_csize && csize != (uint64_t)es.pos) return S_SIZE_MISMATCH;
   return S_OK;
 }
+ZN_HD uint32_t decode_frame(const Team& t, DecShared* sh, const uint8_t* src, uint32_t src_len, uint8_t* out,
+                            uint32_t cap, uint32_t* produced) {
+  return decode_frame(t, sh, src, src_len, out, cap, produced, zs::NoHook{});
+}
 
 }  // namespace lz
 
@@ -182,7 +190,7 @@ ZN_HD uint32_t decode_blob(const Team& t, DecShared* sh, const uint8_t* src, uin
                            uint32_t cap, uint8_t* lit_scratch, uint32_t& predef, uint32_t* produced, Hook& hook) {
   *produced = 0;
   if (src_len >= 4 && ld32le(src) == 0x184D2204u) {
-    const uint32_t rc = lz::decode_frame(t, sh, src, src_len, out, cap, produced);
+    const uint32_t rc = lz::decode_frame(t, sh, src, src_len, out, cap, produced, hook);
     if (rc == S_OK) {  // the LZ4 path has no per-block hook: everything is hashed at the end
       zs::ExecState es;
       es.pos = *produced; es.wm = 0; es.bulk = 1;  // force a full memory barrier (and bulk drain) in finish()

@@ -1015,6 +1015,146 @@ extern "C" int zn_decode_verify_batch(zn_ctx* c, const uint8_t* blobs_base, cons
   return rc;
 }
 
+extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                 uint8_t* pack, uint32_t* status, uint64_t* produced) {
+  if (!c || (n && (!blobs_base || !blob_off || !blob_len || !compressed || !out_len || !stop || !status || !produced))) return ZN_E_ARG;
+  if (n_win && (!win_row || !win_off || !win_len || !pack)) return ZN_E_ARG;
+  if (n == 0) return ZN_OK;
+  cudaSetDevice(c->device);
+  // every row decodes into scratch of its full size, so the block a prefix row writes past its stop lands in its own space
+  std::vector<uint64_t> dev_out(n);
+  std::vector<uint32_t> full, part;
+  uint64_t cur = 0;
+  for (uint32_t i = 0; i < n; i++) {
+    if (out_len[i] >= 0xFFFFFFF0ull || (compressed[i] != 1 && compressed[i] != 2)) return ZN_E_ARG;
+    dev_out[i] = cur;
+    cur += (out_len[i] + 15) & ~15ull;
+    (compressed[i] == 1 && stop[i] < out_len[i] ? part : full).push_back(i);
+  }
+  std::vector<uint64_t> gtab(3 * (size_t)n_win);  // gather table: source offset, length, offset in `pack`
+  uint64_t packed = 0;
+  for (uint32_t w = 0; w < n_win; w++) {
+    const uint32_t r = win_row[w];
+    if (r >= n || win_off[w] > out_len[r] || win_len[w] > out_len[r] - win_off[w]) return ZN_E_ARG;
+    gtab[w] = dev_out[r] + win_off[w];
+    gtab[n_win + w] = win_len[w];
+    gtab[2 * (size_t)n_win + w] = packed;
+    packed += win_len[w];
+  }
+  Layout Li = make_layout(blob_off, blob_len, n);
+  int rc = ensure(c, &c->d_in, &c->d_in_cap, Li.total);
+  if (rc) return rc;
+  rc = ensure(c, &c->d_out, &c->d_out_cap, cur);
+  if (rc) return rc;
+  rc = copy_in(c, c->d_in, blobs_base, blob_off, blob_len, n, Li);
+  if (rc) return rc;
+  // prefix rows: the team kernels with a stop, one-warp teams up to 64 KiB, 128-thread teams above; largest first
+  const uint32_t np = (uint32_t)part.size();
+  std::sort(part.begin(), part.end(), [&](uint32_t x, uint32_t y) {
+    const bool sx = stop[x] <= (64u << 10), sy = stop[y] <= (64u << 10);
+    return sx != sy ? sx : stop[x] > stop[y];
+  });
+  uint32_t n_small = 0;
+  while (n_small < np && stop[part[n_small]] <= (64u << 10)) n_small++;
+  // one device block: descriptors, stops, list, statuses, produced, 2 work counters, gather table
+  const size_t o_stop = sizeof(BlobDesc) * np, o_list = o_stop + 4ull * np, o_st = o_list + 4ull * np, o_pr = o_st + 4ull * np,
+               o_ctr = o_pr + 4ull * np, o_tab = (o_ctr + 8 + 7) & ~(size_t)7, o_end = o_tab + 8 * gtab.size();
+  std::vector<uint8_t> h(o_end, 0);
+  {
+    BlobDesc* d = reinterpret_cast<BlobDesc*>(h.data());
+    uint32_t* s = reinterpret_cast<uint32_t*>(h.data() + o_stop);
+    uint32_t* l = reinterpret_cast<uint32_t*>(h.data() + o_list);
+    for (uint32_t j = 0; j < np; j++) {
+      const uint32_t i = part[j];
+      d[j].src_off = Li.dev_off[i]; d[j].src_len = blob_len[i]; d[j].dst_off = dev_out[i]; d[j].dst_cap = out_len[i];
+      d[j].n_chunks = 0; d[j].cv_base = 0; d[j].flags = F_COMPRESSED;
+      s[j] = (uint32_t)stop[i];
+      l[j] = j;
+    }
+    if (!gtab.empty()) memcpy(h.data() + o_tab, gtab.data(), 8 * gtab.size());
+  }
+  uint8_t* dm = nullptr;
+  uint8_t* d_pack = nullptr;
+  if (cudaMallocAsync((void**)&dm, o_end + 16, c->stream) != cudaSuccess ||
+      (packed && cudaMallocAsync((void**)&d_pack, packed + 64, c->stream) != cudaSuccess) ||
+      cudaMemcpyAsync(dm, h.data(), o_end, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
+    c->err = std::string("range decode allocation failed: ") + cudaGetErrorString(cudaGetLastError());
+    if (dm) cudaFreeAsync(dm, c->stream);
+    if (d_pack) cudaFreeAsync(d_pack, c->stream);
+    return ZN_E_NOMEM;
+  }
+  // rows needed in full: the plan of zn_decode_verify_batch (decode classes, digest tree, content checksums)
+  zn_plan* p = nullptr;
+  if (!full.empty()) {
+    const size_t nf = full.size();
+    std::vector<uint64_t> fo(nf), fl(nf), fd(nf), fol(nf);
+    std::vector<uint8_t> fc(nf);
+    for (size_t j = 0; j < nf; j++) {
+      const uint32_t i = full[j];
+      fo[j] = Li.dev_off[i]; fl[j] = blob_len[i]; fc[j] = compressed[i]; fd[j] = dev_out[i]; fol[j] = out_len[i];
+    }
+    p = plan_build(c, PLAN_DECODE_VERIFY, (uint32_t)nf, fo.data(), fl.data(), fc.data(), fd.data(), fol.data(), nullptr, false);
+    if (p) rc = zn_plan_run(p, c->d_in, c->d_out, nullptr);
+    if (!p || rc != ZN_OK) {
+      if (p) zn_plan_destroy(p);
+      cudaFreeAsync(dm, c->stream);
+      if (d_pack) cudaFreeAsync(d_pack, c->stream);
+      return p ? rc : ZN_E_NOMEM;
+    }
+  }
+  const BlobDesc* d_desc = reinterpret_cast<const BlobDesc*>(dm);
+  const uint32_t* d_stop = reinterpret_cast<const uint32_t*>(dm + o_stop);
+  const uint32_t* d_list = reinterpret_cast<const uint32_t*>(dm + o_list);
+  uint32_t* d_st = reinterpret_cast<uint32_t*>(dm + o_st);
+  uint32_t* d_pr = reinterpret_cast<uint32_t*>(dm + o_pr);
+  uint32_t* d_ctr = reinterpret_cast<uint32_t*>(dm + o_ctr);
+  const uint64_t* d_tab = reinterpret_cast<const uint64_t*>(dm + o_tab);
+  uint32_t launches = 0;
+  if (n_small) {
+    const uint32_t grid = std::min<uint32_t>((n_small + 1) / 2, c->dec_grid_small);
+    k_decode<32, 2, true><<<grid, 32, 0, c->stream>>>(d_desc, d_list, n_small, c->d_in, c->d_out, c->d_lit, d_st, d_pr, d_ctr,
+                                                      nullptr, 1u, nullptr, 0u, d_stop);
+    launches++;
+  }
+  if (const uint32_t nm = np - n_small) {
+    const uint32_t grid = std::min<uint32_t>((nm + 3) / 4, c->dec_grid);
+    k_decode<kDecodeThreads, 4, true><<<grid, kDecodeThreads, 0, c->stream>>>(d_desc, d_list + n_small, nm, c->d_in, c->d_out,
+                                                                              c->d_lit, d_st, d_pr, d_ctr + 1, nullptr, 1u,
+                                                                              nullptr, 0u, d_stop);
+    launches++;
+  }
+  // the windows, packed back to back on the device and returned with one copy
+  if (packed) {
+    k_pack_frames<<<std::min<uint32_t>((n_win + 7) / 8, (uint32_t)c->sm_count * 8u), 256, 0, c->stream>>>(
+        c->d_out, d_tab, d_tab + n_win, d_tab + 2 * (size_t)n_win, n_win, d_pack);
+    launches++;
+  }
+  c->launches += launches;
+  std::vector<uint32_t> pst(np), ppr(np);
+  rc = cudaGetLastError() == cudaSuccess ? ZN_OK : ZN_E_CUDA;
+  if (rc == ZN_OK && packed && cudaMemcpyAsync(pack, d_pack, packed, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = ZN_E_CUDA;
+  if (rc == ZN_OK && np &&
+      (cudaMemcpyAsync(pst.data(), d_st, 4ull * np, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
+       cudaMemcpyAsync(ppr.data(), d_pr, 4ull * np, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess))
+    rc = ZN_E_CUDA;
+  if (rc != ZN_OK) c->err = std::string("range decode: ") + cudaGetErrorString(cudaGetLastError());
+  std::vector<uint32_t> fst(full.size());
+  if (p) {
+    const int prc = zn_plan_results(p, fst.data(), nullptr);  // synchronises the stream
+    if (rc == ZN_OK) rc = prc;
+    zn_plan_destroy(p);
+  }
+  if (rc == ZN_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) { c->err = cudaGetErrorString(cudaGetLastError()); rc = ZN_E_CUDA; }
+  cudaFreeAsync(dm, c->stream);
+  if (d_pack) cudaFreeAsync(d_pack, c->stream);
+  if (rc != ZN_OK) return rc;
+  for (size_t j = 0; j < full.size(); j++) { status[full[j]] = fst[j]; produced[full[j]] = out_len[full[j]]; }
+  for (uint32_t j = 0; j < np; j++) { status[part[j]] = pst[j]; produced[part[j]] = ppr[j]; }
+  return ZN_OK;
+}
+
 extern "C" int zn_frame_content_size(const uint8_t* blob, size_t len, uint64_t* size_out) {
   if (!blob || !size_out) return ZN_E_ARG;
   *size_out = 0;

@@ -441,8 +441,18 @@ struct NoHook {
   ZN_HD void finish(const Team&, ExecState&) {}
 };
 
+// Range reads: ends the decode after the first block whose end reaches `stop` (block-granular, so at most one block is
+// written past it).  Every other hook decodes to the end; stop_here is then a constant false and compiles away.
+struct StopAt : NoHook {
+  uint32_t stop;
+};
+template <class Hook>
+ZN_HD bool stop_here(const Hook&, uint32_t) { return false; }
+ZN_HD bool stop_here(const StopAt& h, uint32_t pos) { return pos >= h.stop; }
+
 // All concatenated frames of one blob (skippable frames are skipped).  Team-uniform.
-// Returns the blob's status; *produced = bytes written to out.
+// Returns the blob's status; *produced = bytes written to out.  With a StopAt hook the decode returns S_OK as soon as a
+// block ends at or past the stop, without the frame-content-size comparison or the checksum of that frame.
 template <class Hook>
 ZN_HD uint32_t decode_frames(const Team& t, DecShared* sh, const uint8_t* src, uint32_t src_len, uint8_t* out,
                              uint32_t cap, uint8_t* lit_scratch, uint32_t& predef, uint32_t* produced, Hook& hook) {
@@ -528,6 +538,7 @@ ZN_HD uint32_t decode_frames(const Team& t, DecShared* sh, const uint8_t* src, u
       }
       *produced = es.pos;
       hook.after_block(t, es);
+      if (stop_here(hook, es.pos)) return S_OK;
       if (last) break;
     }
     if (fb != 0 && (uint64_t)(es.pos - frame_start) != fcs) return S_SIZE_MISMATCH;
