@@ -254,7 +254,81 @@ class _Zstd:
         z.ZSTD_CCtx_setParameter.restype = C.c_size_t
         z.ZSTD_compress2.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t]
         z.ZSTD_compress2.restype = C.c_size_t
+        z.ZSTD_compressSequences.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p,
+                                             C.c_size_t]
+        z.ZSTD_compressSequences.restype = C.c_size_t
+        z.ZSTD_CCtx_refPrefix.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        z.ZSTD_CCtx_refPrefix.restype = C.c_size_t
+        z.ZSTD_writeSkippableFrame.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_uint]
+        z.ZSTD_writeSkippableFrame.restype = C.c_size_t
         self.z = z
+
+    # Experimental parameter ids of zstd.h 1.5.5 (ZSTD_c_experimentalParam5 / 11 / 12 / 19); the ids move between releases.
+    C_LITERAL_COMPRESSION_MODE = 1002    # ZSTD_ps_enable = 1 (Huffman), ZSTD_ps_disable = 2 (raw literals)
+    C_BLOCK_DELIMITERS = 1008            # ZSTD_sf_explicitBlockDelimiters = 1
+    C_VALIDATE_SEQUENCES = 1009          # checks offsets against the content only: a frame with a prefix needs it off
+    C_SEARCH_EXTERNAL_REPCODES = 1016    # below level 10 libzstd would otherwise never turn a given offset into a repeat code
+
+    class _Seq(C.Structure):  # ZSTD_Sequence
+        _fields_ = [("offset", C.c_uint), ("litLength", C.c_uint), ("matchLength", C.c_uint), ("rep", C.c_uint)]
+
+    def _check(self, r):
+        if self.z.ZSTD_isError(r):
+            raise RuntimeError(self.z.ZSTD_getErrorName(r).decode())
+        return r
+
+    def compress_sequences(self, blocks, literals, level: int = 3, params: dict | None = None, prefix=None):
+        """One frame whose blocks carry exactly the given LZ77 parse (ZSTD_compressSequences; libzstd chooses the entropy
+        coding, repeat codes included).  `blocks`: one list of (ll, ml, off) per block; a last tuple with ml == 0 holds
+        the block's trailing literals.  Literal bytes are taken from `literals` in order.  `prefix`: content the frame
+        may reference before its start (ZSTD_CCtx_refPrefix); a decoder needs the same prefix.
+        Returns (content, frame); content excludes the prefix."""
+        lit = bytes(_buf(literals))
+        pre = bytes(_buf(prefix)) if prefix is not None else b""
+        out, li, arr = bytearray(pre), 0, []
+        for block in blocks:
+            for k, (ll, ml, off) in enumerate(block):
+                if li + ll > len(lit):
+                    raise ValueError("literal source too short")
+                out += lit[li:li + ll]
+                li += ll
+                if ml == 0:
+                    if k != len(block) - 1:
+                        raise ValueError("only a block's last tuple may have no match")
+                    break
+                s = len(out) - off
+                if off <= 0 or s < 0:
+                    raise ValueError(f"offset {off} reaches before the content")
+                out += out[s:s + ml] if off >= ml else (out[s:] * (ml // off + 1))[:ml]
+                arr.append((off, ll, ml, 0))
+            last = block[-1] if block else (0, 0, 0)
+            arr.append((0, last[0] if last[1] == 0 else 0, 0, 0))  # block delimiter carrying the trailing literals
+        content = bytes(out[len(pre):])
+        seqs = (self._Seq * len(arr))(*[self._Seq(*a) for a in arr])
+        cap = self.z.ZSTD_compressBound(len(content)) + 64 * len(blocks)
+        dst = np.empty(cap, np.uint8)
+        src = np.frombuffer(content, np.uint8) if content else np.zeros(1, np.uint8)
+        cctx = self.z.ZSTD_createCCtx()
+        try:
+            settings = {100: level, self.C_BLOCK_DELIMITERS: 1, self.C_VALIDATE_SEQUENCES: 1,  # 100: compressionLevel
+                        self.C_SEARCH_EXTERNAL_REPCODES: 1}
+            settings.update(params or {})
+            for k, v in settings.items():
+                self._check(self.z.ZSTD_CCtx_setParameter(cctx, int(k), int(v)))
+            pbuf = np.frombuffer(pre, np.uint8) if pre else None
+            if pre:
+                self._check(self.z.ZSTD_CCtx_refPrefix(cctx, _ptr(pbuf), len(pre)))
+            r = self._check(self.z.ZSTD_compressSequences(cctx, _ptr(dst), cap, seqs, len(arr), _ptr(src), len(content)))
+        finally:
+            self.z.ZSTD_freeCCtx(cctx)
+        return content, dst[:r].tobytes()
+
+    def skippable_frame(self, payload: bytes, variant: int = 0) -> bytes:
+        """ZSTD_writeSkippableFrame: magic 0x184D2A50 + variant, size, payload."""
+        src = np.frombuffer(payload, np.uint8) if payload else np.zeros(1, np.uint8)
+        dst = np.empty(len(payload) + 8, np.uint8)
+        r = self._check(self.z.ZSTD_writeSkippableFrame(_ptr(dst), dst.size, _ptr(src), len(payload), variant))
+        return dst[:r].tobytes()
 
     def version(self) -> int:
         return int(self.z.ZSTD_versionNumber())

@@ -45,6 +45,14 @@ def _run(codec, blobs, comp, contents, expect=True, want_out=True, align=1, lead
     return st, dg, out, out_off
 
 
+def _classes(codec, blobs, contents):
+    """rows per decode class plan_build gives these rows (zn_plan_class_counts; the plan is not run)"""
+    from znippy_b200 import Plan
+    lens = [len(c) for c in contents]
+    return Plan.decode_verify(codec.default_ctx(), np.cumsum([0] + [len(b) for b in blobs])[:-1], [len(b) for b in blobs],
+                              [1] * len(blobs), np.cumsum([0] + lens)[:-1], lens).class_counts()
+
+
 def test_blake3_kats(codec, oracle):
     O = oracle
     kats = json.load(open(os.path.join(GOLD, "blake3_kat.json")))
@@ -94,6 +102,9 @@ def test_zstd_entropy_paths_vs_oracle(codec, oracle, level):
                 O.gen_text(3 << 20).tobytes(), O.gen_binary(1 << 20).tobytes(), O.gen_random(200_000).tobytes(), b"",
                 bytes([7]) * 70000 + O.real_text(3000).tobytes() + bytes([9]) * 200000]
     blobs = [z.compress(c, level) for c in contents]
+    # the last row, runs around real text, is compressed to under 1/64 and is below 512 KiB: it takes k_decode<128,4>,
+    # not the device-wide pipeline
+    assert _classes(codec, blobs[-1:], contents[-1:]) == [0, 0, 0, 0, 1]
     for b, c in zip(blobs, contents):  # the oracle agrees with libzstd on these frames
         rc, o = O.zstd_decompress(b, len(c))
         assert rc == 0 and o == c
@@ -231,9 +242,10 @@ def test_codec_rs_unit_tests(codec, oracle):
 
 
 def test_block_parallel_path_levels_and_fuzz(codec, oracle):
-    """Large entropy-coded blobs take the block-parallel kernel (walker, symbolic repeat offsets, lane-parallel
-    executor).  All levels (treeless literals / repeat-mode tables appear at >= 7), multi-frame blobs, and injected
-    corruption: the verdict must match the oracle's and nothing may hang."""
+    """Large entropy-coded blobs (compressed above 1/64 of their content) take the device-wide pipeline, whatever the
+    name says: k_decode_par only gets rows whose frame is at least as large as their content.  All levels (treeless
+    literals / repeat-mode tables appear at >= 7), multi-frame blobs, and injected corruption: the verdict must match the
+    oracle's and nothing may hang."""
     O = oracle
     z = O.libzstd()
     rt = O.real_text(3_000_000)
@@ -243,6 +255,7 @@ def test_block_parallel_path_levels_and_fuzz(codec, oracle):
     contents.append(O.gen_rle_literals().tobytes() * 4); blobs.append(z.compress(contents[-1], 19))
     two = rt[:1_200_000].tobytes()
     contents.append(two + two[:700_000]); blobs.append(z.compress(two, 3) + z.compress(two[:700_000], 19))
+    assert _classes(codec, blobs, contents) == [len(blobs), 0, 0, 0, 0]
     st, dg, out, out_off = _run(codec, blobs, [1] * len(blobs), contents)
     assert st.tolist() == [0] * len(blobs)
     for i, c in enumerate(contents):
@@ -294,8 +307,9 @@ def test_raw_lz4_blocks(codec, oracle):
 
 
 def test_block_parallel_mixed_batch_with_small_sources(codec, oracle):
-    """A big-blob batch (block-parallel kernel) that also holds blobs whose COMPRESSED form is small enough to be staged
-    in shared memory, with short-sequence blocks (lane executor) and long-match blocks (team executor) interleaved."""
+    """A big-blob batch that also holds blobs whose compressed form is small, with short-sequence blocks and long-match
+    blocks interleaved.  Every row is entropy-coded above 1/64 and at least 4 KiB, so the device-wide pipeline takes them
+    all (not the block-parallel kernel the name recalls)."""
     O = oracle
     z = O.libzstd()
     rt = O.real_text(2_500_000)
@@ -304,6 +318,7 @@ def test_block_parallel_mixed_batch_with_small_sources(codec, oracle):
     contents = [rt.tobytes(), small_real.tobytes(), mix.tobytes(), rt[:1_000_000].tobytes(), small_real[:5000].tobytes(),
                 rt[100:2_200_100].tobytes()]
     blobs = [z.compress(c, 3) for c in contents]
+    assert _classes(codec, blobs, contents) == [len(blobs), 0, 0, 0, 0]
     st, dg, out, out_off = _run(codec, blobs, [1] * len(blobs), contents)
     assert st.tolist() == [0] * len(blobs)
     for i, c in enumerate(contents):

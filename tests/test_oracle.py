@@ -248,3 +248,26 @@ def test_cpu_pipeline_counters_follow_reference_rules(oracle):
     blobs2, dig = O.compress_slices(np.concatenate(slices), np.cumsum([0] + usz)[:-1], usz, 3, 2)
     for s, b, d in zip(slices, blobs2, dig):
         assert z.decompress(b, len(s)) == s.tobytes() and d.tobytes() == O.blake3_official(s)
+
+
+def test_frames_from_chosen_sequences(oracle):
+    """compress_sequences: libzstd writes a frame carrying exactly the given parse (explicit block delimiters, validated
+    sequences), which libzstd and the oracle decode to the expanded content, with one sequence per tuple given; repeated
+    distances become repeat codes; an invalid tuple is refused."""
+    O, z = oracle, oracle.libzstd()
+    rt = O.real_text(400_000)
+    blocks = [[(5000, 100_000, 1), (2000, 20_000, 3)],
+              [(100, 40, 7)] * 600 + [(10, 30_000, 17_000), (55, 0, 0)],
+              [(3, 5, 4)] * 5000]
+    content, frame = z.compress_sequences(blocks, rt)
+    assert len(content) == 127_000 + 600 * 140 + 30_010 + 55 + 5000 * 8
+    assert content[:5000] == rt[:5000].tobytes() and content[5000:105_000] == content[4999:5000] * 100_000
+    assert z.decompress(frame, len(content)) == content
+    rc, out, st = O.zstd_decompress(frame, len(content), want_stats=True)
+    assert rc == 0 and out == content
+    assert st["sequences"] == sum(1 for b in blocks for t in b if t[1]) and st["blocks_compressed"] == 3
+    assert st["repcode_uses"] >= 5000
+    with pytest.raises(RuntimeError):
+        z.compress_sequences([[(10, 2, 5)]], rt)  # shorter than the minimum match
+    with pytest.raises(ValueError):
+        z.compress_sequences([[(10, 5, 11)]], rt)  # reaches before the content
