@@ -75,7 +75,16 @@ enum {
    * envelope layer below) around the frame, or around the raw bytes when the frame did not shrink them
    * (store-if-incompressible); the index metadata gets znippy_envelope = "ZNB1" and readers resolve such rows through
    * zn_envelope_parse.  A compress plan makes the same decision on the device and emits the same blob bytes. */
-  ZN_CODEC_ENVELOPE = 0x100
+  ZN_CODEC_ENVELOPE = 0x100,
+  /* OR-ed into ZN_CODEC_ZSTD at levels <= 19 (zn_compress_batch, compress plans, archive writer): the Zstandard seekable
+   * format.  Every 128 KiB block of a slice is an independent frame (13-byte header, one last block, no history from
+   * the block before), followed by a skippable frame holding the seek table {compressed size, decompressed size, low 32
+   * bits of XXH64(content)} per frame and the footer {N, 0x80, 0x8F92EAB1}.  Every zstd decoder reads such a blob as the
+   * concatenated frames and skips the table; archive range reads use the table to decode only the frames a range
+   * touches.  An empty slice is the 9-byte empty frame and a one-entry table.  The archive writer records
+   * znippy_seekable = "zstd" in the index metadata.  LZ4 and levels >= 20 (whose matches reach up to 8 MiB back) are
+   * refused. */
+  ZN_CODEC_SEEKABLE = 0x400 /* 0x200 | ZN_CODEC_ZSTD stays an unknown codec */
 };
 
 typedef struct zn_ctx zn_ctx;   /* one CUDA device + streams + scratch + pinned staging; not thread-safe */
@@ -130,16 +139,22 @@ int zn_decode_verify_batch(zn_ctx* ctx, const uint8_t* blobs_base, const uint64_
  * matches anywhere in the slice up to 8 MiB back, through a candidate index sorted on the device, and take several
  * times longer.  A match never reaches into another slice, and a frame depends only on its slice's bytes.  LZ4 has
  * one effort.  The frame is always decodable by stock libzstd / liblz4.
+ * codec ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE (levels <= 19): the blob is the seekable layout described at the codec enum;
+ * ZN_E_ARG for LZ4 or a level >= 20 with the flag.
  */
 int zn_compress_batch(zn_ctx* ctx, const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len,
                       uint32_t n, int level, int codec, uint8_t* dst_base, const uint64_t* dst_off,
                       uint64_t* dst_len_out, uint8_t* digest_out /* nullable */, uint32_t* status);
 
+/* ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE: exact, per 128 KiB block 13 + 3 + the block's bytes + 12, plus 17 for the seek
+ * table; 38 for an empty slice. */
 size_t zn_compress_bound(size_t src_len, int codec);
 /* device time (ms, CUDA events) of the compression kernels of the most recent zn_compress_batch on this ctx */
 float zn_ctx_last_compress_ms(const zn_ctx* ctx);
 
-/* decoded size announced by the frame header. returns ZN_OK, 1 when the frame carries no size, <0 on error */
+/* decoded size announced by the frame header. returns ZN_OK, 1 when the frame carries no size, <0 on error.  Only the
+ * first frame is read: the decoded size of a blob of concatenated frames with a seek table (ZN_CODEC_SEEKABLE) is what
+ * zn_envelope_parse reports. */
 int zn_frame_content_size(const uint8_t* blob, size_t len, uint64_t* size_out);
 
 /* ---- envelope layer (csrc/envelope.cpp): what the reference's zl_get_decompressed_size / zl_decompress pair does
@@ -159,7 +174,8 @@ typedef struct {
   uint64_t payload_len;
   uint64_t out_len;     /* decoded size the envelope announces; UINT64_MAX when it carries none */
 } zn_envelope;
-/* ZN_OK; 1 = not a recognised / well-formed envelope (the row gets ZN_S_UNSUPPORTED); < 0 bad arguments */
+/* ZN_OK; 1 = not a recognised / well-formed envelope (the row gets ZN_S_UNSUPPORTED); < 0 bad arguments.  A bare zstd
+ * blob that ends in a valid seek table (ZN_CODEC_SEEKABLE) announces the sum of the table's decompressed sizes. */
 int zn_envelope_parse(const uint8_t* blob, size_t len, zn_envelope* out);
 /* Writes the ZNB1 header for a payload of `codec` decoding to out_len bytes; returns its length (0 on bad arguments). */
 size_t zn_envelope_znb1_header(uint32_t codec, uint64_t out_len, uint8_t* hdr, size_t cap);
@@ -244,6 +260,11 @@ int zn_archive_extract_files(zn_ctx* ctx, zn_archive* a, const char* const* path
  *     call needs from it (at most one 128 KiB zstd block or one LZ4 frame block more).  Only that prefix is checked:
  *     damage past the block where decoding stopped goes unseen, and the content checksum is not checked.  A frame that
  *     ends before that point gives ZN_S_SIZE_MISMATCH.  A raw LZ4 block chunk is one block and decodes whole;
+ *   - in seekable archives (index metadata znippy_seekable = "zstd", ZN_CODEC_SEEKABLE), a zstd chunk covered in part
+ *     is served from its seek table instead: only the 128 KiB frames the requests touch are read, each run of adjacent
+ *     ones is decoded whole, and every decoded frame is checked against the table's XXH64 (a mismatch is
+ *     ZN_S_DECODE_ERROR).  A table that is missing or inconsistent with the chunk sends it down the prefix path above.
+ *     The counters then count the frames' output and the table + frame bytes read;
  *   - store-as-is chunks and ZNB1 chunks with a RAW payload never reach the GPU: only the requested bytes are pread,
  *     straight into out_base.  A call whose ranges lie only in such chunks launches no kernel;
  *   - with the LRU on, cached chunks are copied from it, chunks decoded in full are inserted, partial chunks never.
@@ -280,7 +301,10 @@ const char* zn_archive_writer_error(const zn_archive_writer* w);
 /* The writer is a three-stage pipeline over three pinned slots (the Magazine, slotpool.rs:93-227): filling slot k+2,
  * compressing slot k+1 on the GPU and pwriting slot k overlap; `ctx` belongs to the writer until finish().
  * compress_dir (slot_packer.rs:329-609): walks input_dir (sorted), cuts every file into rounds placed in the slots and
- * lets io_threads readers pread the bytes into place — the whole directory in one call. */
+ * lets io_threads readers pread the bytes into place — the whole directory in one call.
+ * codec ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE (levels <= 19) writes seekable blobs and the index metadata
+ * znippy_seekable = "zstd"; with LZ4 or a level >= 20 zn_archive_writer_create returns NULL and zn_archive_compress_dir
+ * returns ZN_E_ARG with a message. */
 int zn_archive_compress_dir(zn_ctx* ctx, const char* input_dir, const char* output_path, int no_skip, int level, int codec,
                             size_t slot_bytes, int io_threads, zn_compression_report* report, char* err, size_t errcap);
 /* pinned host memory (cudaHostAlloc) for callers that stage their own buffers */
@@ -346,10 +370,13 @@ int zn_plan_last_ms(zn_plan* plan, float ms[4]);
 /* Compress plan over slices that will be resident in HBM: sizes fixed at creation, data supplied per run.  Slice i is
  * d_src[h_src_off[i] .. + h_src_len[i]) of every run.  `level` and `codec` as for zn_compress_batch; `digests` != 0 also
  * hashes the source slices (the zn_hash_batch kernels, on the run's stream).  All planning, uploads and allocation
- * happen here.  NULL, with zn_last_error set, for a slice of 4 GiB or more or a codec other than ZN_CODEC_ZSTD /
- * ZN_CODEC_LZ4 (optionally | ZN_CODEC_ENVELOPE).  n = 0 is a valid plan. */
+ * happen here.  NULL, with zn_last_error set, for a slice of 4 GiB or more, a codec other than ZN_CODEC_ZSTD
+ * (optionally | ZN_CODEC_SEEKABLE) / ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE, or ZN_CODEC_SEEKABLE at a level
+ * >= 20.  Seekable plans also run the frame checksum kernel, counted in stage [1] of zn_plan_last_ms.  n = 0 is a valid
+ * plan. */
 zn_plan* zn_plan_compress(zn_ctx* ctx, uint32_t n, const uint64_t* h_src_off, const uint64_t* h_src_len, int level,
-                          int codec /* ZN_CODEC_ZSTD | ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE */, int digests);
+                          int codec /* ZN_CODEC_ZSTD [| ZN_CODEC_SEEKABLE] | ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE */,
+                          int digests);
 /* bytes d_dst must hold for any input of these sizes */
 uint64_t zn_plan_compress_capacity(const zn_plan* plan);
 /* Enqueues the batch on `stream` (NULL = ctx stream) and returns without waiting. Blob i lands at

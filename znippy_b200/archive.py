@@ -488,13 +488,20 @@ class StreamCompressor:
 
     def __init__(self, output: str, no_skip: bool, level: int = 19, codec_id: int = codec.CODEC_ZSTD,
                  ctx: Ctx | None = None, batch_bytes: int = 256 << 20, native_index: bool = True, native: bool = True,
-                 envelope: bool = False):
+                 envelope: bool = False, seekable: bool = False):
         """level defaults to the reference's compression_level = 19 (common_config.rs:37); levels 20-22 select the
         long effort of the zstd match finder (smaller frames, slower writes; codec.CompressCtx).  envelope=True (native
-        writer only): blobs of compressed rows are ZNB1 envelopes, incompressible slices are stored raw inside them."""
+        writer only): blobs of compressed rows are ZNB1 envelopes, incompressible slices are stored raw inside them.
+        seekable=True (native writer, zstd at levels <= 19): compressed rows are seekable blobs, and range reads decode
+        only the 128 KiB frames they touch."""
         if envelope and not native:
             raise ValueError("the ZNB1 envelope is written by the native pipeline only")
+        if seekable and not native:
+            raise ValueError("seekable archives are written by the native pipeline only")
+        if seekable and (codec_id != codec.CODEC_ZSTD or level >= 20):
+            raise ValueError("seekable archives need the zstd codec at a level <= 19")
         self.envelope = envelope
+        self.seekable = seekable
         self.native_index = native_index
         self.native = native
         self._w = None
@@ -507,7 +514,8 @@ class StreamCompressor:
         if self._w is None:
             self._ctx = self.ctx or default_ctx()
             self._w = N.lib().zn_archive_writer_create(self._ctx.handle, self.output.encode(), int(self.no_skip), self.level,
-                                                       self.codec_id | (N.CODEC_ENVELOPE if self.envelope else 0), self.batch_bytes)
+                                                       self.codec_id | (N.CODEC_ENVELOPE if self.envelope else 0) |
+                                                       (N.CODEC_SEEKABLE if self.seekable else 0), self.batch_bytes)
             if not self._w:
                 raise IOError(f"cannot create {self.output}")
         return self._w
@@ -659,11 +667,12 @@ def compress_stream(output: str, no_skip: bool, **kw) -> StreamCompressor:
 
 
 def compress_dir(input_dir: str, output: str, no_skip: bool = False, level: int = 19, codec_id: int = codec.CODEC_ZSTD,
-                 ctx: Ctx | None = None, envelope: bool = False, io_threads: int = 8, slot_bytes: int = 256 << 20) -> CompressionReport:
+                 ctx: Ctx | None = None, envelope: bool = False, io_threads: int = 8, slot_bytes: int = 256 << 20,
+                 seekable: bool = False) -> CompressionReport:
     """znippy-compress `compress_dir` (walk -> readers -> Magazine slots -> workers -> writer, slot_packer.rs:329-609) in
     one native call: `zn_archive_compress_dir` walks the directory, places every round in a pinned slot, lets
     `io_threads` readers pread the bytes into place, and runs the same three-stage slot pipeline as compress_stream.
-    `level` as in compress_stream: 19 by default, 20-22 for the long effort."""
+    `level` as in compress_stream: 19 by default, 20-22 for the long effort; `seekable` as in compress_stream."""
     import ctypes as C
 
     from . import _native as N
@@ -672,7 +681,8 @@ def compress_dir(input_dir: str, output: str, no_skip: bool = False, level: int 
     rep8 = (C.c_uint64 * 8)()
     err = C.create_string_buffer(512)
     rc = N.lib().zn_archive_compress_dir(ctx.handle, input_dir.encode(), out.encode(), int(no_skip), level,
-                                         codec_id | (N.CODEC_ENVELOPE if envelope else 0), slot_bytes, io_threads, C.byref(rep8), err, 512)
+                                         codec_id | (N.CODEC_ENVELOPE if envelope else 0) | (N.CODEC_SEEKABLE if seekable else 0),
+                                         slot_bytes, io_threads, C.byref(rep8), err, 512)
     if rc != 0:
         raise N.NativeError(f"zn_archive_compress_dir: {err.value.decode(errors='replace')}")
     return CompressionReport(*[int(x) for x in rep8])

@@ -19,7 +19,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
-from ._native import (CODEC_LZ4, CODEC_ZSTD, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_OK,  # noqa: F401
+from ._native import (CODEC_LZ4, CODEC_SEEKABLE, CODEC_ZSTD, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_OK,  # noqa: F401
                       S_SIZE_MISMATCH, S_UNSUPPORTED, Ctx, NativeError, default_ctx)
 
 
@@ -105,8 +105,13 @@ def compress_batch(src, src_off, src_len, level: int = 1, codec: int = CODEC_ZST
 
 
 def frame_content_size(blob) -> int | None:
-    """zl_get_decompressed_size (codec.rs:69): decoded size announced by the frame header, None when absent."""
+    """zl_get_decompressed_size (codec.rs:69): decoded size announced by the frame header, None when absent.  A bare zstd
+    blob that ends in a seek table (CODEC_SEEKABLE) holds several frames: its size is the table's sum
+    (zn_envelope_parse)."""
     b = N.u8(blob)
+    env = envelope_parse(b) if b[:4].tobytes() == b"\x28\xb5\x2f\xfd" else None
+    if env is not None and env[4] is not None:
+        return env[4]
     v = C.c_uint64(0)
     rc = N.lib().zn_frame_content_size(N.ptr(b) if b.size else None, b.size, C.byref(v))
     if rc < 0:
@@ -158,11 +163,13 @@ def blake3_hash(data, ctx: Ctx | None = None) -> bytes:
 class CompressCtx:
     """codec.rs:8-55.  `level` follows the reference's meaning (higher = more effort); the GPU match finder has
     four efforts: three window geometries for levels <= 2, 3..9 and 10..19, and for levels >= 20 (zstd only) the long
-    effort, whose matches reach back anywhere in the slice up to 8 MiB (DESIGN.md §4.3)."""
+    effort, whose matches reach back anywhere in the slice up to 8 MiB (DESIGN.md §4.3).  seekable=True (zstd, levels
+    <= 19): one independent frame per 128 KiB block and a seek table (CODEC_SEEKABLE, DESIGN.md §4.3)."""
 
-    def __init__(self, compression_level: int, codec: int = CODEC_ZSTD, ctx: Ctx | None = None, envelope: bool = False):
+    def __init__(self, compression_level: int, codec: int = CODEC_ZSTD, ctx: Ctx | None = None, envelope: bool = False,
+                 seekable: bool = False):
         self.level = int(compression_level)
-        self.codec = codec
+        self.codec = codec | (CODEC_SEEKABLE if seekable else 0)
         self.ctx = ctx or default_ctx()
         self.envelope = envelope  # wrap every frame in ZNB1; incompressible input is then stored RAW (size + 6..10 bytes)
 
@@ -178,7 +185,7 @@ class CompressCtx:
         if self.envelope:
             if len(blobs[0]) >= b.size:
                 return envelope_wrap(PAYLOAD_RAW, b.size, b.tobytes())
-            return envelope_wrap(PAYLOAD_ZSTD if self.codec == CODEC_ZSTD else PAYLOAD_LZ4_FRAME, b.size, blobs[0])
+            return envelope_wrap(PAYLOAD_LZ4_FRAME if self.codec == CODEC_LZ4 else PAYLOAD_ZSTD, b.size, blobs[0])
         return blobs[0]
 
     def compress_into(self, data, out: bytearray) -> int:

@@ -11,7 +11,8 @@
 //     first lane with a verified 4-byte match, and the match is extended 128 bytes per step across the warp;
 //   * zstd blocks carry raw literals and sequences coded with the PREDEFINED FSE tables (modes byte 0), never a
 //     repeat-offset code, so blocks do not depend on each other and stock libzstd decodes the frame;
-//     the match window of a block is primed with the tail of the previous block (the window is the whole slice);
+//     the match window of a block is primed with the tail of the previous block (the window is the whole slice),
+//     except in seekable slices, where every block is a frame of its own and starts without history;
 //   * every block lands in a scratch slot; a second kernel lays the blocks out back to back behind the frame header.
 //
 // Everything here is warp-uniform code over a `Warp` abstraction (32 lanes on the device, 1 lane on the host) so the
@@ -1332,6 +1333,53 @@ ZN_HD uint64_t zstd_frame_size(uint64_t n, const uint32_t* meta) {
   }
   return sz;
 }
+// The empty frame, as libzstd writes it: single segment, 1-byte content size 0, empty raw last block (9 bytes).
+ZN_HD uint32_t zstd_empty_frame(uint8_t* dst) {
+  const uint8_t e[9] = {0x28, 0xB5, 0x2F, 0xFD, 0x20, 0x00, 0x01, 0x00, 0x00};
+  for (int k = 0; k < 9; k++) dst[k] = e[k];
+  return 9;
+}
+
+// ---- seekable layout (ZN_CODEC_SEEKABLE): every kZstdCBlock block of the slice is a frame of its own (the 13-byte
+// header, one last block), then the seek table of the Zstandard seekable format (contrib/seekable_format in the zstd
+// tree): a skippable frame, magic 0x184D2A5E and Frame_Size = 12 N + 9, holding per frame {compressed size, decompressed
+// size, low 32 bits of XXH64(content, 0)}, then the footer {N, descriptor 0x80 = checksums present, 0x8F92EAB1}, all
+// little-endian.  An empty slice is the empty frame and a table with one entry.
+constexpr uint32_t kSeekEntry = 12, kSeekFixed = 17;  // bytes per entry; skippable header (8) + footer (9)
+constexpr uint32_t kSeekSkipMagic = 0x184D2A5Eu, kSeekFooterMagic = 0x8F92EAB1u, kSeekChecksums = 0x80u;
+constexpr uint32_t kXxhEmpty = 0x51D8E999u;  // low 32 bits of XXH64("", 0)
+ZN_HD void put_le32(uint8_t* d, uint32_t v) { d[0] = (uint8_t)v; d[1] = (uint8_t)(v >> 8); d[2] = (uint8_t)(v >> 16); d[3] = (uint8_t)(v >> 24); }
+// meta as for zstd_frame_size
+ZN_HD uint64_t zstd_seekable_size(uint64_t n, const uint32_t* meta) {
+  if (n == 0) return 9 + kSeekEntry + kSeekFixed;
+  uint64_t sz = kSeekFixed;
+  for (uint64_t o = 0, j = 0; o < n; o += kZstdCBlock, j++) {
+    const uint32_t bn = (uint32_t)(n - o < kZstdCBlock ? n - o : kZstdCBlock), c = meta[2 * j + 1];
+    sz += 13 + 3 + (c ? c : bn) + kSeekEntry;
+  }
+  return sz;
+}
+// The seek table of a slice of n bytes at dst; returns its length.  meta as for zstd_frame_size, xxh = the checksum of
+// the slice's first frame (unused when n == 0).
+ZN_HD uint32_t zstd_seek_table(uint8_t* dst, uint64_t n, const uint32_t* meta, const uint32_t* xxh) {
+  const uint32_t nf = n ? (uint32_t)((n + kZstdCBlock - 1) / kZstdCBlock) : 1u;
+  put_le32(dst, kSeekSkipMagic);
+  put_le32(dst + 4, kSeekEntry * nf + 9);
+  uint8_t* e = dst + 8;
+  if (n == 0) {
+    put_le32(e, 9); put_le32(e + 4, 0); put_le32(e + 8, kXxhEmpty);
+    e += kSeekEntry;
+  }
+  for (uint64_t o = 0, j = 0; o < n; o += kZstdCBlock, j++, e += kSeekEntry) {
+    const uint32_t bn = (uint32_t)(n - o < kZstdCBlock ? n - o : kZstdCBlock), c = meta[2 * j + 1];
+    put_le32(e, 13 + 3 + (c ? c : bn)); put_le32(e + 4, bn); put_le32(e + 8, xxh[j]);
+  }
+  put_le32(e, nf);
+  e[4] = (uint8_t)kSeekChecksums;
+  put_le32(e + 5, kSeekFooterMagic);
+  return kSeekFixed + kSeekEntry * nf;
+}
+
 // LZ4: csize = the slice's first block size (>= the block's input size means stored); 15-byte header, 4-byte EndMark
 ZN_HD uint64_t lz4_frame_size(uint64_t n, const uint32_t* csize) {
   uint64_t sz = 15 + 4;

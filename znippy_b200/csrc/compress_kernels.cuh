@@ -9,6 +9,7 @@
 
 #include "compress.cuh"
 #include "coop.cuh"
+#include "xxh_verify.cuh"
 
 namespace zn {
 
@@ -90,7 +91,8 @@ __global__ void __launch_bounds__(256) k_lz4_assemble(const SliceDesc* __restric
 }
 
 // ---- zstd: every 128 KiB block of every slice -> staged payload; meta[2j] = payload offset in the slot, meta[2j+1] = size (0 = raw)
-template <class WN>
+// kFrames (seekable slices): every block is a frame of its own, so its match finder starts without history.
+template <class WN, bool kFrames = false>
 __global__ void __launch_bounds__(32) k_zstd_blocks(const SliceDesc* __restrict__ slices, uint32_t n_slices, uint32_t total_blocks,
                                                     const uint8_t* __restrict__ src_base, uint8_t* tmp, uint64_t* seq_scratch,
                                                     uint32_t* meta) {
@@ -105,8 +107,9 @@ __global__ void __launch_bounds__(32) k_zstd_blocks(const SliceDesc* __restrict_
     const uint64_t o = (uint64_t)(j - s.blk_first) * cz::kZstdCBlock;
     const uint32_t n = (uint32_t)(s.src_len - o < cz::kZstdCBlock ? s.src_len - o : cz::kZstdCBlock);
     uint32_t poff = 0;
-    const uint32_t c = cz::zstd_compress_block<WN>(w, src_base + s.src_off, (uint32_t)o, n, tmp + (size_t)j * cz::kZstdSlot, seqs, D, tab,
-                                               &poff);
+    const uint64_t base = kFrames ? s.src_off + o : s.src_off;
+    const uint32_t bstart = kFrames ? 0u : (uint32_t)o;
+    const uint32_t c = cz::zstd_compress_block<WN>(w, src_base + base, bstart, n, tmp + (size_t)j * cz::kZstdSlot, seqs, D, tab, &poff);
     if (w.lane == 0) { meta[2 * j] = poff; meta[2 * j + 1] = c; }
     __syncwarp();
   }
@@ -174,12 +177,8 @@ ZN_D void zstd_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const 
   const SliceDesc s = slices[i];
   uint8_t* dst = dst_base + s.dst_off;
   const Team t{threadIdx.x, blockDim.x};
-  if (s.src_len == 0) {  // same bytes as libzstd: single-segment, 1-byte content size 0, empty raw last block
-    if (threadIdx.x == 0) {
-      const uint8_t e[9] = {0x28, 0xB5, 0x2F, 0xFD, 0x20, 0x00, 0x01, 0x00, 0x00};
-      for (int k = 0; k < 9; k++) dst[k] = e[k];
-      dst_len[i] = 9;
-    }
+  if (s.src_len == 0) {
+    if (threadIdx.x == 0) dst_len[i] = cz::zstd_empty_frame(dst);
     return;
   }
   if (threadIdx.x == 0) cz::zstd_frame_header(dst, s.src_len);
@@ -202,20 +201,59 @@ ZN_D void zstd_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const 
   }
   if (threadIdx.x == 0) dst_len[i] = op;
 }
+// Seekable slice (cz::zstd_seek_table): one frame per block, then the seek table; xxh[j] = checksum of global block j.
+ZN_D void zstd_seekable_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base,
+                                 const uint8_t* tmp, const uint32_t* __restrict__ meta, const uint32_t* __restrict__ xxh,
+                                 uint8_t* dst_base, uint64_t* dst_len) {
+  const SliceDesc s = slices[i];
+  uint8_t* dst = dst_base + s.dst_off;
+  const Team t{threadIdx.x, blockDim.x};
+  uint64_t op = s.src_len ? 0 : 9;
+  if (s.src_len == 0 && threadIdx.x == 0) cz::zstd_empty_frame(dst);
+  for (uint32_t b = 0; b < s.n_blocks; b++) {
+    const uint32_t j = s.blk_first + b;
+    const uint64_t o = (uint64_t)b * cz::kZstdCBlock;
+    const uint32_t n = (uint32_t)(s.src_len - o < cz::kZstdCBlock ? s.src_len - o : cz::kZstdCBlock);
+    const uint32_t poff = meta[2 * j], c = meta[2 * j + 1];
+    if (threadIdx.x == 0) {
+      cz::zstd_frame_header(dst + op, n);
+      cz::zstd_block_header(dst + op + 13, 1, c ? 2 : 0, c ? c : n);
+    }
+    team_copy(t, dst + op + 16, c ? tmp + (size_t)j * cz::kZstdSlot + poff : src_base + s.src_off + o, c ? c : n);
+    op += 16 + (c ? c : n);
+  }
+  if (threadIdx.x == 0) dst_len[i] = op + cz::zstd_seek_table(dst + op, s.src_len, meta + 2 * (size_t)s.blk_first, xxh + s.blk_first);
+}
+// xxh: nullptr, or the block checksums of a seekable batch (k_block_xxh)
 __global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
-                                                       const uint8_t* tmp, const uint32_t* __restrict__ meta, uint8_t* dst_base,
-                                                       uint64_t* dst_len) {
-  zstd_assemble(slices, blockIdx.x, src_base, tmp, meta, dst_base, dst_len);
+                                                       const uint8_t* tmp, const uint32_t* __restrict__ meta,
+                                                       const uint32_t* __restrict__ xxh, uint8_t* dst_base, uint64_t* dst_len) {
+  if (xxh) zstd_seekable_assemble(slices, blockIdx.x, src_base, tmp, meta, xxh, dst_base, dst_len);
+  else zstd_assemble(slices, blockIdx.x, src_base, tmp, meta, dst_base, dst_len);
+}
+
+// ---- seekable batches: xxh[j] = low 32 bits of XXH64 of global block j's source bytes (one thread per block: XXH64 is
+// serial along a block, and blocks are independent)
+constexpr int kXxhThreads = 32;  // few threads per CTA: the blocks spread over every SM
+__global__ void __launch_bounds__(kXxhThreads) k_block_xxh(const SliceDesc* __restrict__ slices, uint32_t n_slices,
+                                                           uint32_t total_blocks, const uint8_t* __restrict__ src_base,
+                                                           uint32_t* xxh) {
+  for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < total_blocks; j += gridDim.x * blockDim.x) {
+    const SliceDesc s = slices[slice_of_block(slices, n_slices, j)];
+    const uint64_t o = (uint64_t)(j - s.blk_first) * cz::kZstdCBlock;
+    const uint32_t n = (uint32_t)(s.src_len - o < cz::kZstdCBlock ? s.src_len - o : cz::kZstdCBlock);
+    xxh[j] = (uint32_t)xxh64_1(src_base + s.src_off + o, n);
+  }
 }
 
 // ---- packed layout (device-resident compress plans): blob i = [ZNB1 header] + frame, or header + the slice's bytes when
 // the envelope stores it RAW; blobs back to back.  One CTA: per tile of slices, every thread sizes one slice from the
-// block results (cz::zstd_frame_size / lz4_frame_size), the CTA scans the sizes, and each thread writes its slice's
+// block results (cz::zstd_frame_size / zstd_seekable_size / lz4_frame_size), the CTA scans the sizes, and each thread writes its slice's
 // offset, its frame's destination (past the header) into slices[i].dst_off, the RAW decision and the header.
 constexpr int kLayoutThreads = 1024;
 __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slices, uint32_t n, const uint32_t* __restrict__ res,
-                                                                uint32_t lz4, uint32_t envelope, uint8_t* dst_base,
-                                                                uint64_t* offsets, uint32_t* raw) {
+                                                                uint32_t lz4, uint32_t seekable, uint32_t envelope,
+                                                                uint8_t* dst_base, uint64_t* offsets, uint32_t* raw) {
   __shared__ uint64_t warp_sum[kLayoutThreads / 32];
   const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
   uint64_t carry = 0;  // bytes of the tiles before this one (every thread keeps the same value)
@@ -226,7 +264,9 @@ __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slice
     if (i < n) {
       const SliceDesc s = slices[i];
       len = s.src_len;
-      sz = lz4 ? cz::lz4_frame_size(len, res + s.blk_first) : cz::zstd_frame_size(len, res + 2 * (size_t)s.blk_first);
+      sz = lz4        ? cz::lz4_frame_size(len, res + s.blk_first)
+           : seekable ? cz::zstd_seekable_size(len, res + 2 * (size_t)s.blk_first)
+                      : cz::zstd_frame_size(len, res + 2 * (size_t)s.blk_first);
       if (envelope) {
         r = sz >= len;
         hl = cz::znb1_header_len(len);
@@ -261,17 +301,19 @@ __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slice
 }
 
 // Frames straight into the packed layout (one CTA per slice); a RAW row gets the slice's bytes instead of its frame.
-// dst_len receives the frame lengths, as from k_zstd_assemble / k_lz4_assemble.
+// dst_len receives the frame lengths, as from k_zstd_assemble / k_lz4_assemble; xxh as for k_zstd_assemble.
 template <bool LZ4>
 __global__ void __launch_bounds__(256) k_assemble_packed(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
                                                          const uint8_t* tmp, const uint32_t* __restrict__ res,
-                                                         const uint32_t* __restrict__ raw, uint8_t* dst_base, uint64_t* dst_len) {
+                                                         const uint32_t* __restrict__ xxh, const uint32_t* __restrict__ raw,
+                                                         uint8_t* dst_base, uint64_t* dst_len) {
   if (raw[blockIdx.x]) {
     const SliceDesc s = slices[blockIdx.x];
     team_copy(Team{threadIdx.x, blockDim.x}, dst_base + s.dst_off, src_base + s.src_off, (uint32_t)s.src_len);
     return;
   }
   if (LZ4) lz4_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
+  else if (xxh) zstd_seekable_assemble(slices, blockIdx.x, src_base, tmp, res, xxh, dst_base, dst_len);
   else zstd_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
 }
 

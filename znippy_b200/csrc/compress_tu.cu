@@ -13,11 +13,17 @@ void compress_init_attrs() {
   cudaFuncSetAttribute(k_zstd_blocks<cz::WinFast>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinFast>::kSmemBytes);
   cudaFuncSetAttribute(k_zstd_blocks<cz::WinMid>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinMid>::kSmemBytes);
   cudaFuncSetAttribute(k_zstd_blocks<cz::WinHigh>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinHigh>::kSmemBytes);
+  cudaFuncSetAttribute(k_zstd_blocks<cz::WinFast, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinFast>::kSmemBytes);
+  cudaFuncSetAttribute(k_zstd_blocks<cz::WinMid, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinMid>::kSmemBytes);
+  cudaFuncSetAttribute(k_zstd_blocks<cz::WinHigh, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZstdLaunch<cz::WinHigh>::kSmemBytes);
 }
 
 size_t compress_bound(size_t n, int codec) {
+  const size_t nb = (n + cz::kZstdCBlock - 1) / cz::kZstdCBlock;
+  if (codec & kCodecSeekable)  // exact: every block stored raw in a frame of its own (cz::zstd_seekable_size)
+    return n ? n + (13 + 3 + cz::kSeekEntry) * nb + cz::kSeekFixed : 9 + cz::kSeekEntry + cz::kSeekFixed;
   if (codec == 2) return n + 4 * ((n + cz::kLz4Block - 1) / cz::kLz4Block) + 32;
-  return n + 3 * ((n + cz::kZstdCBlock - 1) / cz::kZstdCBlock) + 32;
+  return n + 3 * nb + 32;
 }
 
 template <typename T>
@@ -141,7 +147,12 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   // zstd: the level picks the match finder: three window geometries, then (levels >= 20) the whole-slice long effort;
   // LZ4 has one effort
   const int effort = level <= 2 ? 0 : (level <= 9 ? 1 : (level <= 19 ? 2 : 3));
-  const bool lz4 = codec == 2;
+  const bool seekable = (codec & kCodecSeekable) != 0;
+  const bool lz4 = (codec & ~kCodecSeekable) == 2;
+  if (seekable && (lz4 || effort == 3)) {  // the long effort reaches up to 8 MiB back, which a one-block frame rules out
+    *err = "seekable frames need the zstd codec at a level <= 19";
+    return -1;
+  }
   const uint64_t bsz = lz4 ? cz::kLz4Block : cz::kZstdCBlock;
   std::vector<SliceDesc> sl(n);
   uint64_t total_blocks = 0;
@@ -162,7 +173,8 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   const uint32_t grid = std::max<uint32_t>(1, std::min<uint32_t>((nb + wpc - 1) / wpc, (uint32_t)sm_count * (lz4 ? 6u : (effort == 0 ? ZstdLaunch<cz::WinFast>::kCtasPerSm
                                                                   : effort == 1 ? ZstdLaunch<cz::WinMid>::kCtasPerSm
                                                                                 : ZstdLaunch<cz::WinHigh>::kCtasPerSm))));
-  const size_t small_bytes = (size_t)n * sizeof(SliceDesc) + (size_t)nb * 8 + (size_t)n * 8 + (size_t)n * 4 + 64;
+  const size_t small_bytes = (size_t)n * sizeof(SliceDesc) + (size_t)nb * 8 + (size_t)n * 8 + (size_t)n * 4 + 64 +
+                             (seekable ? (size_t)nb * 4 : 0);
   if (!grow(&cs->tmp, &cs->tmp_cap, std::max<size_t>(1, (size_t)nb * slot)) ||
       !grow((uint8_t**)&cs->small, &cs->small_cap, small_bytes) ||
       (!lz4 && effort < 3 && !grow(&cs->seqs, &cs->seqs_cap, (size_t)grid * wpc * cz::kZstdMaxSeq * 8))) {
@@ -171,6 +183,7 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   }
   *P = CompressPrep();
   P->lz4 = lz4;
+  P->seekable = seekable;
   P->effort = effort;
   P->n = n;
   P->nb = nb;
@@ -181,12 +194,13 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   uint64_t* d_len = (uint64_t*)((uint8_t*)P->d_meta + (size_t)nb * 8);
   P->d_len = (uint64_t*)(((uintptr_t)d_len + 7) & ~(uintptr_t)7);
   P->d_raw = (uint32_t*)(P->d_len + n);
+  if (seekable) P->d_xxh = P->d_raw + n;
   if (cudaMemcpyAsync(P->d_sl, sl.data(), (size_t)n * sizeof(SliceDesc), cudaMemcpyHostToDevice, st) != cudaSuccess) {
     *err = "compress H2D failed";
     return -2;
   }
   if (nb && !lz4 && effort == 3) return long_prepare(cs, st, sm_count, sl, P, err);
-  if (nb) P->launches = 1;
+  if (nb) P->launches = seekable ? 2 : 1;
   return 0;
 }
 
@@ -214,6 +228,16 @@ int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st
     return 0;
   }
   const uint32_t n = P.n, nb = P.nb, grid = P.grid;
+  if (P.seekable) {
+    k_block_xxh<<<(nb + kXxhThreads - 1) / kXxhThreads, kXxhThreads, 0, st>>>(P.d_sl, n, nb, d_src, P.d_xxh);
+    if (P.effort == 0)
+      k_zstd_blocks<cz::WinFast, true><<<grid, 32, ZstdLaunch<cz::WinFast>::kSmemBytes, st>>>(P.d_sl, n, nb, d_src, cs->tmp, cs->seqs, P.d_meta);
+    else if (P.effort == 1)
+      k_zstd_blocks<cz::WinMid, true><<<grid, 32, ZstdLaunch<cz::WinMid>::kSmemBytes, st>>>(P.d_sl, n, nb, d_src, cs->tmp, cs->seqs, P.d_meta);
+    else
+      k_zstd_blocks<cz::WinHigh, true><<<grid, 32, ZstdLaunch<cz::WinHigh>::kSmemBytes, st>>>(P.d_sl, n, nb, d_src, cs->tmp, cs->seqs, P.d_meta);
+    return 0;
+  }
   if (P.lz4) k_lz4_blocks<<<grid, kLz4WarpsPerCta * 32, 0, st>>>(P.d_sl, n, nb, d_src, cs->tmp, P.d_meta);
   else if (P.effort == 0)
     k_zstd_blocks<cz::WinFast><<<grid, 32, ZstdLaunch<cz::WinFast>::kSmemBytes, st>>>(P.d_sl, n, nb, d_src, cs->tmp, cs->seqs, P.d_meta);
@@ -227,9 +251,10 @@ int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st
 void compress_pack(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, uint8_t* d_dst,
                    uint64_t* d_offsets, bool envelope) {
   if (!P.n) return;
-  k_pack_layout<<<1, kLayoutThreads, 0, st>>>(P.d_sl, P.n, P.d_meta, P.lz4 ? 1u : 0u, envelope ? 1u : 0u, d_dst, d_offsets, P.d_raw);
-  if (P.lz4) k_assemble_packed<true><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_raw, d_dst, P.d_len);
-  else k_assemble_packed<false><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_raw, d_dst, P.d_len);
+  k_pack_layout<<<1, kLayoutThreads, 0, st>>>(P.d_sl, P.n, P.d_meta, P.lz4 ? 1u : 0u, P.seekable ? 1u : 0u, envelope ? 1u : 0u, d_dst,
+                                              d_offsets, P.d_raw);
+  if (P.lz4) k_assemble_packed<true><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, nullptr, P.d_raw, d_dst, P.d_len);
+  else k_assemble_packed<false><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, P.d_raw, d_dst, P.d_len);
 }
 
 // Compresses n slices resident on the device into frames at d_dst + dst_off[i]; synchronises `st` before returning.
@@ -246,7 +271,7 @@ int compress_run(CompressScratch* cs, cudaStream_t st, int sm_count, const uint8
   if (rc) return rc;
   *launches = P.launches;
   if (P.lz4) k_lz4_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, d_dst, P.d_len);
-  else k_zstd_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, d_dst, P.d_len);
+  else k_zstd_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, d_dst, P.d_len);
   (*launches)++;
   cudaEventRecord(cs->ev[1], st);
   if (cudaMemcpyAsync(out_len, P.d_len, (size_t)n * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||

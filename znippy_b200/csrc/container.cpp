@@ -110,6 +110,7 @@ struct IndexImpl {
   std::vector<uint32_t> chunk_seq;
   std::vector<uint8_t> compressed;
   std::vector<uint8_t> comp_eff;  // what the batch calls get: 4 (enveloped) instead of 1 when the archive declares an envelope
+  bool seekable = false;          // znippy_seekable = "zstd": zstd payloads may end in a seek table (ZN_CODEC_SEEKABLE)
   std::vector<uint8_t> checksums;
   std::vector<uint64_t> path_off;  // rows + 1
   std::string paths;
@@ -630,6 +631,11 @@ static zn_index* index_open_range(const char* path, uint64_t want_lo, uint64_t w
         if (it->second != "ZNB1") throw std::string("archive declares an unknown blob envelope: " + it->second);
         for (auto& c : h->ix.comp_eff) c = c ? 4 : 0;
       }
+      it = h->ix.metadata.find("znippy_seekable");
+      if (it != h->ix.metadata.end()) {
+        if (it->second != "zstd") throw std::string("archive declares an unknown seekable format: " + it->second);
+        h->ix.seekable = true;
+      }
     }
     uint64_t payload_end = moff;
     for (auto& g : h->ix.groups) payload_end = std::min(payload_end, g.index_offset);
@@ -1060,7 +1066,7 @@ struct zn_archive_writer {
   zn_ctx* ctx;
   int fd;
   bool no_skip;
-  int level, codec;
+  int level, codec;       // codec: ZN_CODEC_ZSTD [| ZN_CODEC_SEEKABLE] or ZN_CODEC_LZ4, as zn_compress_batch takes it
   bool envelope = false;  // ZN_CODEC_ENVELOPE: blobs of compressed rows are ZNB1 envelopes (store-if-incompressible)
   uint64_t slot_bytes, out_cursor = 0;
   WSlot slots[kSlots];
@@ -1277,7 +1283,8 @@ extern "C" zn_archive_writer* zn_archive_writer_create(zn_ctx* ctx, const char* 
   if (!ctx || !output_path) return nullptr;
   const bool envelope = (codec & ZN_CODEC_ENVELOPE) != 0;
   codec &= ~ZN_CODEC_ENVELOPE;
-  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4) return nullptr;
+  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4 && codec != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) return nullptr;
+  if ((codec & ZN_CODEC_SEEKABLE) && level >= 20) return nullptr;
   if (slot_bytes < 2 * kSliceSize) slot_bytes = 2 * kSliceSize;
   const int fd = open(output_path, O_CREAT | O_RDWR | O_TRUNC, 0644);
   if (fd < 0) return nullptr;
@@ -1348,6 +1355,7 @@ extern "C" int zn_archive_writer_finish(zn_archive_writer* w, zn_compression_rep
       zn_index_writer_metadata(iw, "compression_level", "19");
       zn_index_writer_metadata(iw, "zstd_output_buffer_size", "1048576");
       if (w->envelope) zn_index_writer_metadata(iw, "znippy_envelope", "ZNB1");  // readers resolve compressed rows through zn_envelope_parse
+      if (w->codec & ZN_CODEC_SEEKABLE) zn_index_writer_metadata(iw, "znippy_seekable", "zstd");  // range reads use the seek tables
     }
     for (auto& kv : groups) {
       const auto& rows = kv.second;
@@ -1420,6 +1428,10 @@ struct ReadJob {
 extern "C" int zn_archive_compress_dir(zn_ctx* ctx, const char* input_dir, const char* output_path, int no_skip, int level, int codec,
                                        size_t slot_bytes, int io_threads, zn_compression_report* report, char* err, size_t errcap) {
   if (!ctx || !input_dir || !output_path) return ZN_E_ARG;
+  if ((codec & ZN_CODEC_SEEKABLE) && ((codec & ~(ZN_CODEC_SEEKABLE | ZN_CODEC_ENVELOPE)) != ZN_CODEC_ZSTD || level >= 20)) {
+    set_err(err, errcap, "seekable archives need the zstd codec at a level <= 19");
+    return ZN_E_ARG;
+  }
   std::vector<DirFile> files;
   walk_dir(input_dir, "", &files);
   zn_archive_writer* w = zn_archive_writer_create(ctx, output_path, no_skip, level, codec, slot_bytes ? slot_bytes : (256u << 20));
@@ -1665,11 +1677,15 @@ extern "C" int zn_archive_extract_files(zn_ctx* ctx, zn_archive* a, const char* 
   return rc;
 }
 
+// envelope.cpp: zn_envelope_parse over the first `head` bytes of a blob of `len` bytes
+extern "C" int zn_envelope_parse_head(const uint8_t* blob, size_t head, size_t len, zn_envelope* e);
+
 // Windowed decode of znippy_cuda.cu (declared in host_api.h, which needs the CUDA headers this file is built without).
-extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
-                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
-                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
-                                 uint8_t* pack, uint32_t* status, uint64_t* produced);
+extern "C" int zn_decode_windows_checked(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                         const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                         const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                         const uint32_t* ck_row, const uint64_t* ck_off, const uint64_t* ck_len,
+                                         const uint32_t* ck_sum, uint32_t n_ck, uint8_t* pack, uint32_t* status, uint64_t* produced);
 
 namespace {
 struct PinnedBuf {  // pinned host buffer from the process-wide cache, returned on scope exit
@@ -1684,6 +1700,48 @@ bool pread_all(int fd, uint8_t* dst, uint64_t len, uint64_t off) {
     done += (uint64_t)r;
   }
   return true;
+}
+
+// One frame of a seekable zstd payload (ZN_CODEC_SEEKABLE): compressed bytes [c, c + cs) of the payload decode to
+// content bytes [d, d + ds) of the row, whose XXH64 has the low 32 bits `sum`.
+struct SeekFrame {
+  uint64_t c, d;
+  uint32_t cs, ds, sum;
+};
+constexpr uint64_t kSeekBlock = 128u << 10;  // frame size of this library's writer (cz::kZstdCBlock)
+uint32_t ld32(const uint8_t* p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
+
+// The seek table at the end of a zstd payload of plen bytes at archive offset po that decodes to ul bytes (the Zstandard
+// seekable format: skippable frame 0x184D2A5E, 12-byte entries with checksums, footer {N, 0x80, 0x8F92EAB1}).  The
+// writer's frame count is tried first, then the footer's.  False when the table is absent or inconsistent with the
+// payload or the index: the row is then decoded from its start.
+bool read_seek_table(int fd, uint64_t po, uint64_t plen, uint64_t ul, std::vector<SeekFrame>* fr, uint64_t* bytes_read) {
+  uint64_t nf = ul ? (ul + kSeekBlock - 1) / kSeekBlock : 1;
+  std::vector<uint8_t> t;
+  for (int attempt = 0;; attempt++) {
+    const uint64_t tl = 12 * nf + 17;
+    if (tl > plen) return false;
+    t.resize(tl);
+    if (!pread_all(fd, t.data(), tl, po + plen - tl)) return false;
+    *bytes_read += tl;
+    const uint8_t* f = t.data() + tl - 9;
+    if (ld32(f + 5) != 0x8F92EAB1u) return false;
+    if (ld32(f) == nf) break;
+    if (attempt == 1) return false;
+    nf = ld32(f);
+  }
+  const uint8_t desc = t[t.size() - 5];
+  if (!(desc & 0x80) || (desc & 0x7C)) return false;  // checksums present, reserved bits clear
+  if (ld32(t.data()) != 0x184D2A5Eu || ld32(t.data() + 4) != 12 * nf + 9) return false;
+  fr->resize(nf);
+  uint64_t c = 0, d = 0;
+  for (uint64_t k = 0; k < nf; k++) {
+    const uint8_t* e = t.data() + 8 + 12 * k;
+    (*fr)[k] = {c, d, ld32(e), ld32(e + 4), ld32(e + 8)};
+    c += ld32(e);
+    d += ld32(e + 4);
+  }
+  return c + t.size() == plen && d == ul;
 }
 }  // namespace
 
@@ -1702,6 +1760,7 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
     uint32_t req, row;     // row: index into `rows` below
     uint64_t s, e, dst;    // bytes [s, e) of the row go to out_base + dst
     uint64_t at;           // where the bytes wait: offset in `cached` or in the decode pack
+    uint32_t unit = 0;     // decode rows: the decode unit (below) that holds the bytes
   };
   struct Row {
     uint64_t r, need = 0;  // index row; bytes [0, need) of it are needed
@@ -1765,22 +1824,28 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
     R.payload_len = bl;
     R.flag = ce;
     if (ce == 4) {
-      // ZNB1 and bare frames are parsed from their first bytes (the parser reads no further for them, so it is told
-      // the blob's full length); a foreign envelope gets the whole blob
+      // ZNB1 and bare frames are parsed from their first bytes; a foreign envelope, and a bare zstd blob that ends in
+      // a seek table (its size is the table's sum), get the whole blob
       std::vector<uint8_t> head((size_t)std::min<uint64_t>(bl, 64));
       if (!pread_all(a->fd, head.data(), head.size(), bo)) return ZN_E_ARG;
       S.blob_bytes_read += head.size();
-      uint32_t magic = 0;
+      uint32_t magic = 0, tail = 0;
       if (head.size() >= 4) memcpy(&magic, head.data(), 4);
-      const bool header_only = magic == 0x31424E5Au /* "ZNB1" */ || magic == 0xFD2FB528u || magic == 0x184D2204u ||
-                               (magic & 0xFFFFFFF0u) == 0x184D2A50u;
+      if (magic == 0xFD2FB528u && bl > head.size()) {
+        uint8_t t[4];
+        if (!pread_all(a->fd, t, 4, bo + bl - 4)) return ZN_E_ARG;
+        S.blob_bytes_read += 4;
+        tail = ld32(t);
+      }
+      const bool header_only = magic == 0x31424E5Au /* "ZNB1" */ || (magic == 0xFD2FB528u && tail != 0x8F92EAB1u) ||
+                               magic == 0x184D2204u || (magic & 0xFFFFFFF0u) == 0x184D2A50u;
       if (!header_only && head.size() < bl) {
         head.resize(bl);
         if (!pread_all(a->fd, head.data(), bl, bo)) return ZN_E_ARG;
         S.blob_bytes_read += bl;
       }
       zn_envelope e;
-      const int erc = zn_envelope_parse(head.data(), header_only ? bl : head.size(), &e);
+      const int erc = zn_envelope_parse_head(head.data(), head.size(), bl, &e);
       if (erc != ZN_OK || (e.out_len != ~0ull && e.out_len != ul)) {
         R.kind = 3;
         R.status = erc != ZN_OK ? ZN_S_UNSUPPORTED : ZN_S_SIZE_MISMATCH;
@@ -1796,41 +1861,124 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
       R.raw_off = bo + R.payload_off;
     }
   }
-  // decode rows: whole blobs into pinned staging, 16 bytes apart (room for the magic of a magicless zstd payload)
-  std::vector<uint32_t> dec;
+  // decode units: a decode row whole, up to its `need` (the prefix path), or, for a seekable row read in part, each run
+  // of adjacent frames its pieces touch, decoded whole and checked frame by frame against the seek table
+  struct Unit {
+    uint32_t row;
+    uint64_t rd_off, rd_len;  // archive bytes pread for the unit
+    uint64_t in_off, in_len;  // decoder input: bytes [in_off, + in_len) of what was pread
+    uint64_t d_off, d_len;    // content bytes [d_off, + d_len) of the row
+    uint64_t stop;            // decode up to here (d_len: whole)
+    bool seek = false;
+  };
+  std::vector<Unit> units;
+  std::vector<uint32_t> ck_row, ck_sum;
+  std::vector<uint64_t> ck_off, ck_len;
+  std::vector<std::vector<uint32_t>> pieces_of(rows.size());
+  for (uint32_t p = 0; p < (uint32_t)pieces.size(); p++) pieces_of[pieces[p].row].push_back(p);
+  // the seek tables of the seekable zstd rows read in part (their pieces leave a byte uncovered), pread in parallel
+  std::vector<uint32_t> seek_rows;
+  for (uint32_t j = 0; I.seekable && j < (uint32_t)rows.size(); j++) {
+    const Row& R = rows[j];
+    if (R.kind != 0 || R.flag != 1) continue;
+    std::vector<std::pair<uint64_t, uint64_t>> iv;
+    for (uint32_t p : pieces_of[j]) iv.emplace_back(pieces[p].s, pieces[p].e);
+    std::sort(iv.begin(), iv.end());
+    uint64_t covered = 0;
+    for (auto& v : iv) if (v.first <= covered) covered = std::max(covered, v.second);
+    if (covered < I.col[3][R.r]) seek_rows.push_back(j);
+  }
+  std::vector<std::vector<SeekFrame>> tables(rows.size());
+  std::vector<uint8_t> has_table(rows.size(), 0);
+  {
+    std::atomic<size_t> next{0};
+    std::atomic<uint64_t> table_bytes{0};
+    auto body = [&] {
+      for (size_t k; (k = next.fetch_add(1)) < seek_rows.size();) {
+        const uint32_t j = seek_rows[k];
+        const Row& R = rows[j];
+        uint64_t got = 0;
+        has_table[j] = read_seek_table(a->fd, I.col[0][R.r] + R.payload_off, R.payload_len, I.col[3][R.r], &tables[j], &got);
+        table_bytes += got;
+      }
+    };
+    std::vector<std::thread> ts;
+    for (int t = 1; t < (seek_rows.size() >= 16 ? 4 : 1); t++) ts.emplace_back(body);
+    body();
+    for (auto& t : ts) t.join();
+    S.blob_bytes_read += table_bytes;
+  }
+  uint32_t rows_dec = 0;
+  for (uint32_t j = 0; j < (uint32_t)rows.size(); j++) {
+    Row& R = rows[j];
+    if (R.kind != 0) continue;
+    rows_dec++;
+    const uint64_t bo = I.col[0][R.r], ul = I.col[3][R.r];
+    const std::vector<SeekFrame>& fr = tables[j];
+    if (!has_table[j]) {
+      units.push_back({j, bo, I.col[1][R.r], R.payload_off, R.payload_len, 0, ul, R.need});
+      for (uint32_t p : pieces_of[j]) pieces[p].unit = (uint32_t)units.size() - 1;
+      continue;
+    }
+    std::vector<uint8_t> touched(fr.size(), 0);
+    auto frame_of = [&](uint64_t x) {  // the frame holding content byte x
+      return (size_t)(std::upper_bound(fr.begin(), fr.end(), x, [](uint64_t v, const SeekFrame& f) { return v < f.d; }) - fr.begin()) - 1;
+    };
+    for (uint32_t p : pieces_of[j])
+      for (size_t f = frame_of(pieces[p].s); f < fr.size() && fr[f].d < pieces[p].e; f++) touched[f] = 1;
+    const uint32_t first_unit = (uint32_t)units.size();
+    for (size_t f = 0; f < fr.size();) {
+      if (!touched[f]) { f++; continue; }
+      size_t g = f;
+      while (g < fr.size() && touched[g]) g++;
+      const uint64_t c0 = fr[f].c, c1 = fr[g - 1].c + fr[g - 1].cs, d0 = fr[f].d, d1 = fr[g - 1].d + fr[g - 1].ds;
+      const uint32_t u = (uint32_t)units.size();
+      units.push_back({j, bo + R.payload_off + c0, c1 - c0, 0, c1 - c0, d0, d1 - d0, d1 - d0, true});
+      for (size_t k = f; k < g; k++) {
+        ck_row.push_back(u); ck_off.push_back(fr[k].d - d0); ck_len.push_back(fr[k].ds); ck_sum.push_back(fr[k].sum);
+      }
+      f = g;
+    }
+    for (uint32_t p : pieces_of[j]) {  // every piece lies inside one run: the frames it touches are adjacent
+      uint32_t u = first_unit;
+      while (u + 1 < units.size() && units[u + 1].d_off <= pieces[p].s) u++;
+      pieces[p].unit = u;
+    }
+  }
+  // units into pinned staging, 16 bytes apart (room for the magic of a magicless zstd payload)
   uint64_t in_cur = 0;
-  for (uint32_t j = 0; j < (uint32_t)rows.size(); j++)
-    if (rows[j].kind == 0) { dec.push_back(j); in_cur += 16 + ((I.col[1][rows[j].r] + 15) & ~15ull); }
-  std::vector<uint8_t> full_row(rows.size(), 0);  // decoded in full (and so a candidate for the cache)
+  for (const Unit& U : units) in_cur += 16 + ((U.rd_len + 15) & ~15ull);
+  std::vector<uint8_t> full_row(units.size(), 0);  // a row decoded in full (and so a candidate for the cache)
+  std::vector<uint32_t> unit_status(units.size(), 0);
   PinnedBuf pack;  // the decoded bytes of every piece of a decode row
-  if (!dec.empty()) {
-    const uint32_t nd = (uint32_t)dec.size();
+  if (!units.empty()) {
+    const uint32_t nd = (uint32_t)units.size();
     std::vector<uint64_t> bo(nd), bl(nd), ol(nd), stop(nd), prod(nd), w_off, w_len;
     std::vector<uint8_t> cf(nd);
-    std::vector<uint32_t> st(nd), w_row, dec_at(rows.size(), 0);
+    std::vector<uint32_t> st(nd), w_row;
     PinnedBuf stage_buf;
     uint8_t* stage = stage_buf.p = (uint8_t*)zn_ctx_pinned_alloc(in_cur + 4096);
     if (!stage) return ZN_E_NOMEM;
+    std::vector<uint64_t> rd_at(nd);
     uint64_t cur = 0;
     for (uint32_t j = 0; j < nd; j++) {
-      Row& R = rows[dec[j]];
-      dec_at[dec[j]] = j;
-      bo[j] = cur + 16 + R.payload_off;
-      bl[j] = R.payload_len;
-      cf[j] = (uint8_t)R.flag;
-      ol[j] = I.col[3][R.r];
-      stop[j] = R.need;
-      full_row[dec[j]] = R.need >= ol[j] || R.flag == 2;
-      cur += 16 + ((I.col[1][R.r] + 15) & ~15ull);
+      const Unit& U = units[j];
+      const Row& R = rows[U.row];
+      rd_at[j] = cur + 16;
+      bo[j] = cur + 16 + U.in_off;
+      bl[j] = U.in_len;
+      cf[j] = U.seek ? 1 : (uint8_t)R.flag;
+      ol[j] = U.d_len;
+      stop[j] = U.stop;
+      full_row[j] = !U.seek && (R.need >= ol[j] || R.flag == 2);
+      cur += 16 + ((U.rd_len + 15) & ~15ull);
     }
     {
       std::atomic<size_t> next{0};
       std::atomic<int> io_err{0};
       auto body = [&] {
-        for (size_t j; (j = next.fetch_add(1)) < nd;) {
-          const Row& R = rows[dec[j]];
-          if (!pread_all(a->fd, stage + bo[j] - R.payload_off, I.col[1][R.r], I.col[0][R.r])) io_err = 1;
-        }
+        for (size_t j; (j = next.fetch_add(1)) < nd;)
+          if (!pread_all(a->fd, stage + rd_at[j], units[j].rd_len, units[j].rd_off)) io_err = 1;
       };
       std::vector<std::thread> ts;
       for (int t = 1; t < (nd >= 16 ? 4 : 1); t++) ts.emplace_back(body);
@@ -1839,7 +1987,7 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
       if (io_err) return ZN_E_ARG;
     }
     for (uint32_t j = 0; j < nd; j++) {
-      S.blob_bytes_read += I.col[1][rows[dec[j]].r];
+      S.blob_bytes_read += units[j].rd_len;
       if (cf[j] == 3) {  // magicless zstd payload: decoded as magic + payload
         static const uint8_t magic[4] = {0x28, 0xB5, 0x2F, 0xFD};
         bo[j] -= 4;
@@ -1852,31 +2000,32 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
     uint64_t packed = 0;
     for (Piece& P : pieces) {
       if (rows[P.row].kind != 0) continue;
-      w_row.push_back(dec_at[P.row]); w_off.push_back(P.s); w_len.push_back(P.e - P.s);
+      w_row.push_back(P.unit); w_off.push_back(P.s - units[P.unit].d_off); w_len.push_back(P.e - P.s);
       P.at = packed;
       packed += P.e - P.s;
     }
     std::vector<uint64_t> whole_at(nd, ~0ull);
     if (K.budget)
       for (uint32_t j = 0; j < nd; j++)
-        if (full_row[dec[j]] && ol[j] <= K.budget) {
+        if (full_row[j] && ol[j] <= K.budget) {
           w_row.push_back(j); w_off.push_back(0); w_len.push_back(ol[j]);
           whole_at[j] = packed;
           packed += ol[j];
         }
     if (!(pack.p = (uint8_t*)zn_ctx_pinned_alloc(packed + 64))) return ZN_E_NOMEM;
-    const int rc = zn_decode_windows(ctx, stage, bo.data(), bl.data(), cf.data(), ol.data(), stop.data(), nd, w_row.data(),
-                                     w_off.data(), w_len.data(), (uint32_t)w_row.size(), pack.p, st.data(), prod.data());
+    const int rc = zn_decode_windows_checked(ctx, stage, bo.data(), bl.data(), cf.data(), ol.data(), stop.data(), nd, w_row.data(),
+                                     w_off.data(), w_len.data(), (uint32_t)w_row.size(), ck_row.data(), ck_off.data(),
+                                     ck_len.data(), ck_sum.data(), (uint32_t)ck_row.size(), pack.p, st.data(), prod.data());
     if (rc != ZN_OK) return rc;
+    S.rows_decoded += rows_dec;
     for (uint32_t j = 0; j < nd; j++) {
-      rows[dec[j]].status = st[j];
-      S.rows_decoded++;
+      unit_status[j] = st[j];
       S.bytes_decoded += prod[j];
     }
     if (K.budget) {
       std::lock_guard<std::mutex> g(K.mu);
       for (uint32_t j = 0; j < nd; j++) {
-        const uint64_t r = rows[dec[j]].r;
+        const uint64_t r = rows[units[j].row].r;
         if (whole_at[j] == ~0ull || st[j] != ZN_S_OK || K.at.count(r)) continue;
         while (K.used + ol[j] > K.budget && !K.lru.empty()) {  // evict from the cold end
           K.used -= K.lru.back().second.size();
@@ -1890,11 +2039,12 @@ extern "C" int zn_archive_read_ranges(zn_ctx* ctx, zn_archive* a, const char* co
       }
     }
   }
-  // request statuses: the first failing row of each request, in file order
+  // request statuses: the first failing row (or decode unit) of each request, in file order
   for (const Piece& P : pieces) {
     const Row& R = rows[P.row];
-    if (R.status != ZN_S_OK && file_status[P.req] == 0) {
-      file_status[P.req] = 2u | (R.status << 16);
+    const uint32_t status = R.kind == 0 ? unit_status[P.unit] : R.status;
+    if (status != ZN_S_OK && file_status[P.req] == 0) {
+      file_status[P.req] = 2u | (status << 16);
       got[P.req] = 0;
     }
   }

@@ -18,40 +18,67 @@
 namespace {
 std::atomic<zn_envelope_parser> g_foreign{nullptr};
 inline uint32_t le32(const uint8_t* p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
+
+// Decoded size of a zstd blob that ends in a seek table of the Zstandard seekable format (ZN_CODEC_SEEKABLE writes
+// them): the sum of its entries' decompressed sizes.  False unless the footer magic, the descriptor's reserved bits,
+// the skippable frame's magic and size, and the entries' compressed sizes all agree with a blob of len bytes.
+bool seekable_content_size(const uint8_t* blob, size_t len, uint64_t* out) {
+  if (len < 17 || le32(blob + len - 4) != 0x8F92EAB1u) return false;
+  const uint64_t n = le32(blob + len - 9);
+  const uint8_t desc = blob[len - 5];
+  if (desc & 0x7C) return false;
+  const uint64_t esz = desc & 0x80 ? 12 : 8, tl = 8 + esz * n + 9;
+  if (tl > len) return false;
+  const uint8_t* t = blob + len - tl;
+  if (le32(t) != 0x184D2A5Eu || le32(t + 4) != esz * n + 9) return false;
+  uint64_t c = 0, d = 0;
+  for (uint64_t k = 0; k < n; k++) {
+    c += le32(t + 8 + esz * k);
+    d += le32(t + 8 + esz * k + 4);
+  }
+  if (c + tl != len) return false;
+  *out = d;
+  return true;
+}
 }  // namespace
 
 extern "C" void zn_envelope_register(zn_envelope_parser fn) { g_foreign.store(fn); }
 
-extern "C" int zn_envelope_parse(const uint8_t* blob, size_t len, zn_envelope* e) {
-  if (!e || (len && !blob)) return ZN_E_ARG;
+// zn_envelope_parse over the first `head` bytes of a blob of `len` bytes (the archive reader preads only a blob's head):
+// ZNB1 headers and frame headers are read from the head; a bare zstd blob is sized from its seek table, and a foreign
+// parser runs, only when the whole blob is given (head == len).
+extern "C" int zn_envelope_parse_head(const uint8_t* blob, size_t head, size_t len, zn_envelope* e) {
+  if (!e || (head && !blob) || head > len) return ZN_E_ARG;
   memset(e, 0, sizeof *e);
   e->out_len = ~0ull;
   e->payload_len = len;
-  if (len >= 4) {
+  if (head >= 4) {
     const uint32_t magic = le32(blob);
     if (magic == 0xFD2FB528u || (magic & 0xFFFFFFF0u) == 0x184D2A50u) {  // Zstandard frame (or a skippable frame before one)
       e->kind = ZN_ENV_BARE;
       e->codec = ZN_PAYLOAD_ZSTD;
       uint64_t sz = 0;
-      if (zn_frame_content_size(blob, len, &sz) == ZN_OK) e->out_len = sz;
+      if (zn_frame_content_size(blob, head, &sz) == ZN_OK) e->out_len = sz;
+      // concatenated frames with a seek table: the first frame holds only 128 KiB of the content
+      if (magic == 0xFD2FB528u && head == len && seekable_content_size(blob, len, &sz)) e->out_len = sz;
       return ZN_OK;
     }
     if (magic == 0x184D2204u) {
       e->kind = ZN_ENV_BARE;
       e->codec = ZN_PAYLOAD_LZ4_FRAME;
       uint64_t sz = 0;
-      if (zn_frame_content_size(blob, len, &sz) == ZN_OK) e->out_len = sz;
+      if (zn_frame_content_size(blob, head, &sz) == ZN_OK) e->out_len = sz;
       return ZN_OK;
     }
     if (memcmp(blob, "ZNB1", 4) == 0) {
       e->kind = ZN_ENV_ZNB1;
-      if (len < 6) return 1;
+      if (head < 6) return 1;
       const uint32_t codec = blob[4];
       if (codec > ZN_PAYLOAD_LZ4_BLOCK) return 1;
       uint64_t v = 0;
       size_t p = 5;
       for (uint32_t shift = 0;; shift += 7) {  // LEB128, at most 5 bytes: decoded sizes stay below 4 GiB
-        if (p >= len || shift > 28) return 1;
+        if (p >= head || shift > 28) return 1;
         const uint8_t b = blob[p++];
         v |= (uint64_t)(b & 0x7F) << shift;
         if (!(b & 0x80)) break;
@@ -65,7 +92,8 @@ extern "C" int zn_envelope_parse(const uint8_t* blob, size_t len, zn_envelope* e
       return ZN_OK;
     }
   }
-  if (zn_envelope_parser f = g_foreign.load()) {
+  zn_envelope_parser f = g_foreign.load();
+  if (f && head == len) {
     const int rc = f(blob, len, e);
     if (rc == ZN_OK) {
       if (e->payload_off > len || e->payload_len > len - e->payload_off || e->codec > ZN_PAYLOAD_LZ4_BLOCK) return 1;
@@ -79,6 +107,8 @@ extern "C" int zn_envelope_parse(const uint8_t* blob, size_t len, zn_envelope* e
   e->kind = ZN_ENV_UNKNOWN;
   return 1;
 }
+
+extern "C" int zn_envelope_parse(const uint8_t* blob, size_t len, zn_envelope* e) { return zn_envelope_parse_head(blob, len, len, e); }
 
 extern "C" size_t zn_envelope_znb1_header(uint32_t codec, uint64_t out_len, uint8_t* hdr, size_t cap) {
   if (!hdr || cap < ZN_ENVELOPE_ZNB1_MAX_HEADER || codec > ZN_PAYLOAD_LZ4_BLOCK || out_len >= (1ull << 32)) return 0;

@@ -51,18 +51,21 @@ struct CompressScratch {
   }
 };
 void compress_init_attrs();
+constexpr int kCodecSeekable = 0x400;        // ZN_CODEC_SEEKABLE, OR-ed into the codec of the functions below
 size_t compress_bound(size_t n, int codec);  // zn_compress_bound: raw-block fallback makes this exact
 struct SliceDesc;
 // What compress_prepare works out from the slice sizes alone: the effort, the grid, the device descriptors (inside the
 // scratch), and for the long effort the rounds of units, each with its block range and the kernels of its key sort.
 struct CompressPrep {
   bool lz4 = false;
+  bool seekable = false;  // zstd only, levels <= 19: one frame per block and a seek table (cz::zstd_seek_table)
   int effort = 0;
   uint32_t n = 0, nb = 0, grid = 0, sm_count = 0;
   SliceDesc* d_sl = nullptr;   // n slice descriptors
   uint32_t* d_meta = nullptr;  // per-block results: zstd {payload offset, size} pairs, LZ4 sizes
   uint64_t* d_len = nullptr;   // n frame lengths
   uint32_t* d_raw = nullptr;   // n RAW decisions of the packed layout
+  uint32_t* d_xxh = nullptr;   // seekable: nb block checksums (k_block_xxh); nullptr otherwise
   std::vector<uint32_t> round_first{0}, round_pos, round_blk0, round_nblk, round_sort_launches;
   uint32_t long_grid = 0;
   size_t sort_temp = 0;
@@ -118,3 +121,11 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
                                  const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
                                  const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
                                  uint8_t* pack, uint32_t* status, uint64_t* produced);
+// zn_decode_windows that also checks frames of seekable payloads (n_ck of them, nullable arrays when 0): bytes
+// [ck_off[k], + ck_len[k]) of row ck_row[k], decoded in full, must have the low 32 bits of XXH64 ck_sum[k]
+// (k_frame_xxh_check); a mismatch turns a good row's status into S_DECODE_ERROR.
+extern "C" int zn_decode_windows_checked(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                         const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                         const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                         const uint32_t* ck_row, const uint64_t* ck_off, const uint64_t* ck_len,
+                                         const uint32_t* ck_sum, uint32_t n_ck, uint8_t* pack, uint32_t* status, uint64_t* produced);

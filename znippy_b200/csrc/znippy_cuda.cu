@@ -24,6 +24,7 @@
 #include "decode_kernels.cuh"
 #include "par_kernel.cuh"
 #include "fused_ws.cuh"
+#include "xxh_verify.cuh"
 
 using namespace zn;
 
@@ -735,8 +736,9 @@ extern "C" zn_plan* zn_plan_compress(zn_ctx* c, uint32_t n, const uint64_t* h_sr
                                      int codec, int digests) {
   if (!c) return nullptr;
   const int base = codec & ~ZN_CODEC_ENVELOPE;
-  if (base != ZN_CODEC_ZSTD && base != ZN_CODEC_LZ4) {
-    c->err = "zn_plan_compress: codec must be ZN_CODEC_ZSTD or ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE";
+  if (base != ZN_CODEC_ZSTD && base != ZN_CODEC_LZ4 && base != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) {
+    c->err = "zn_plan_compress: codec must be ZN_CODEC_ZSTD (optionally | ZN_CODEC_SEEKABLE) or ZN_CODEC_LZ4, optionally | "
+             "ZN_CODEC_ENVELOPE";
     return nullptr;
   }
   if (n && (!h_src_off || !h_src_len)) { c->err = "zn_plan_compress: null size arrays"; return nullptr; }
@@ -1015,12 +1017,22 @@ extern "C" int zn_decode_verify_batch(zn_ctx* c, const uint8_t* blobs_base, cons
   return rc;
 }
 
-extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
-                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
-                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
-                                 uint8_t* pack, uint32_t* status, uint64_t* produced) {
+// Frames of seekable payloads decoded by a range read, one thread each: bad[k] = 1 when the low 32 bits of XXH64 of
+// out[tab[k] .. + tab[n + k]) differ from tab[2n + k], the frame's seek-table entry.
+__global__ void __launch_bounds__(32) k_frame_xxh_check(const uint64_t* __restrict__ tab, uint32_t n, const uint8_t* __restrict__ out,
+                                                        uint32_t* bad) {
+  for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x)
+    bad[k] = (uint32_t)xxh64_1(out + tab[k], tab[n + k]) != (uint32_t)tab[2 * (size_t)n + k];
+}
+
+extern "C" int zn_decode_windows_checked(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                         const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                         const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                         const uint32_t* ck_row, const uint64_t* ck_off, const uint64_t* ck_len,
+                                         const uint32_t* ck_sum, uint32_t n_ck, uint8_t* pack, uint32_t* status, uint64_t* produced) {
   if (!c || (n && (!blobs_base || !blob_off || !blob_len || !compressed || !out_len || !stop || !status || !produced))) return ZN_E_ARG;
   if (n_win && (!win_row || !win_off || !win_len || !pack)) return ZN_E_ARG;
+  if (n_ck && (!ck_row || !ck_off || !ck_len || !ck_sum)) return ZN_E_ARG;
   if (n == 0) return ZN_OK;
   cudaSetDevice(c->device);
   // every row decodes into scratch of its full size, so the block a prefix row writes past its stop lands in its own space
@@ -1043,6 +1055,15 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
     gtab[2 * (size_t)n_win + w] = packed;
     packed += win_len[w];
   }
+  std::vector<uint64_t> ctab(3 * (size_t)n_ck);  // frame checks: device offset, length, expected checksum
+  for (uint32_t k = 0; k < n_ck; k++) {
+    const uint32_t r = ck_row[k];
+    if (r >= n || compressed[r] != 1 || stop[r] < out_len[r] || ck_off[k] > out_len[r] || ck_len[k] > out_len[r] - ck_off[k])
+      return ZN_E_ARG;
+    ctab[k] = dev_out[r] + ck_off[k];
+    ctab[n_ck + k] = ck_len[k];
+    ctab[2 * (size_t)n_ck + k] = ck_sum[k];
+  }
   Layout Li = make_layout(blob_off, blob_len, n);
   int rc = ensure(c, &c->d_in, &c->d_in_cap, Li.total);
   if (rc) return rc;
@@ -1058,9 +1079,11 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
   });
   uint32_t n_small = 0;
   while (n_small < np && stop[part[n_small]] <= (64u << 10)) n_small++;
-  // one device block: descriptors, stops, list, statuses, produced, 2 work counters, gather table
+  // one device block: descriptors, stops, list, statuses, produced, 2 work counters, gather table, frame checks and
+  // their verdicts
   const size_t o_stop = sizeof(BlobDesc) * np, o_list = o_stop + 4ull * np, o_st = o_list + 4ull * np, o_pr = o_st + 4ull * np,
-               o_ctr = o_pr + 4ull * np, o_tab = (o_ctr + 8 + 7) & ~(size_t)7, o_end = o_tab + 8 * gtab.size();
+               o_ctr = o_pr + 4ull * np, o_tab = (o_ctr + 8 + 7) & ~(size_t)7, o_ck = o_tab + 8 * gtab.size(),
+               o_bad = o_ck + 8 * ctab.size(), o_end = o_bad + 4ull * n_ck;
   std::vector<uint8_t> h(o_end, 0);
   {
     BlobDesc* d = reinterpret_cast<BlobDesc*>(h.data());
@@ -1074,6 +1097,7 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
       l[j] = j;
     }
     if (!gtab.empty()) memcpy(h.data() + o_tab, gtab.data(), 8 * gtab.size());
+    if (!ctab.empty()) memcpy(h.data() + o_ck, ctab.data(), 8 * ctab.size());
   }
   uint8_t* dm = nullptr;
   uint8_t* d_pack = nullptr;
@@ -1125,6 +1149,11 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
                                                                               nullptr, 0u, d_stop);
     launches++;
   }
+  uint32_t* d_bad = reinterpret_cast<uint32_t*>(dm + o_bad);
+  if (n_ck) {  // after the decodes, on the same stream
+    k_frame_xxh_check<<<(n_ck + 31) / 32, 32, 0, c->stream>>>(reinterpret_cast<const uint64_t*>(dm + o_ck), n_ck, c->d_out, d_bad);
+    launches++;
+  }
   // the windows, packed back to back on the device and returned with one copy
   if (packed) {
     k_pack_frames<<<std::min<uint32_t>((n_win + 7) / 8, (uint32_t)c->sm_count * 8u), 256, 0, c->stream>>>(
@@ -1132,8 +1161,10 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
     launches++;
   }
   c->launches += launches;
-  std::vector<uint32_t> pst(np), ppr(np);
+  std::vector<uint32_t> pst(np), ppr(np), bad(n_ck);
   rc = cudaGetLastError() == cudaSuccess ? ZN_OK : ZN_E_CUDA;
+  if (rc == ZN_OK && n_ck && cudaMemcpyAsync(bad.data(), d_bad, 4ull * n_ck, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess)
+    rc = ZN_E_CUDA;
   if (rc == ZN_OK && packed && cudaMemcpyAsync(pack, d_pack, packed, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) rc = ZN_E_CUDA;
   if (rc == ZN_OK && np &&
       (cudaMemcpyAsync(pst.data(), d_st, 4ull * np, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
@@ -1152,7 +1183,17 @@ extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uin
   if (rc != ZN_OK) return rc;
   for (size_t j = 0; j < full.size(); j++) { status[full[j]] = fst[j]; produced[full[j]] = out_len[full[j]]; }
   for (uint32_t j = 0; j < np; j++) { status[part[j]] = pst[j]; produced[part[j]] = ppr[j]; }
+  for (uint32_t k = 0; k < n_ck; k++)
+    if (bad[k] && status[ck_row[k]] == S_OK) status[ck_row[k]] = S_DECODE_ERROR;  // as a content checksum mismatch
   return ZN_OK;
+}
+
+extern "C" int zn_decode_windows(zn_ctx* c, const uint8_t* blobs_base, const uint64_t* blob_off, const uint64_t* blob_len,
+                                 const uint8_t* compressed, const uint64_t* out_len, const uint64_t* stop, uint32_t n,
+                                 const uint32_t* win_row, const uint64_t* win_off, const uint64_t* win_len, uint32_t n_win,
+                                 uint8_t* pack, uint32_t* status, uint64_t* produced) {
+  return zn_decode_windows_checked(c, blobs_base, blob_off, blob_len, compressed, out_len, stop, n, win_row, win_off, win_len,
+                                   n_win, nullptr, nullptr, nullptr, nullptr, 0, pack, status, produced);
 }
 
 extern "C" int zn_frame_content_size(const uint8_t* blob, size_t len, uint64_t* size_out) {
@@ -1190,7 +1231,11 @@ extern "C" int zn_compress_batch(zn_ctx* c, const uint8_t* src_base, const uint6
                                  uint32_t n, int level, int codec, uint8_t* dst_base, const uint64_t* dst_off,
                                  uint64_t* dst_len_out, uint8_t* digest_out, uint32_t* status) {
   if (!c || (n && (!src_base || !src_off || !src_len || !dst_base || !dst_off || !dst_len_out || !status))) return ZN_E_ARG;
-  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4) return ZN_E_ARG;
+  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4 && codec != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) return ZN_E_ARG;
+  if ((codec & ZN_CODEC_SEEKABLE) && level >= 20) {
+    c->err = "zn_compress_batch: seekable frames need a zstd level <= 19";
+    return ZN_E_ARG;
+  }
   if (n == 0) return ZN_OK;
   cudaSetDevice(c->device);
   for (uint32_t i = 0; i < n; i++)
