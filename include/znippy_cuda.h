@@ -84,7 +84,15 @@ enum {
    * touches.  An empty slice is the 9-byte empty frame and a one-entry table.  The archive writer records
    * znippy_seekable = "zstd" in the index metadata.  LZ4 and levels >= 20 (whose matches reach up to 8 MiB back) are
    * refused. */
-  ZN_CODEC_SEEKABLE = 0x400 /* 0x200 | ZN_CODEC_ZSTD stays an unknown codec */
+  ZN_CODEC_SEEKABLE = 0x400, /* 0x200 | ZN_CODEC_ZSTD stays an unknown codec */
+  /* OR-ed into ZN_CODEC_ZSTD (levels 1-22) or ZN_CODEC_LZ4, optionally with ZN_CODEC_ENVELOPE (zn_compress_batch,
+   * compress plans, archive writer): every frame carries a content checksum, as the zstd and lz4 command-line tools
+   * write by default.  Zstandard: frame-header descriptor bit 2 set (0xE4) and the low 32 bits of XXH64(slice, 0) after
+   * the last block; the empty slice is the 13-byte frame 28 B5 2F FD 24 00 01 00 00 99 E9 D8 51.  LZ4: FLG bit 2 set
+   * (header checksum byte recomputed) and XXH32(slice, 0) after the EndMark; no block checksums.  A frame is 4 bytes
+   * longer than without the flag, and so is zn_compress_bound.  Refused with ZN_CODEC_SEEKABLE (ZN_E_ARG): the seek
+   * table already carries one XXH64 per frame. */
+  ZN_CODEC_CHECKSUM = 0x800
 };
 
 typedef struct zn_ctx zn_ctx;   /* one CUDA device + streams + scratch + pinned staging; not thread-safe */
@@ -140,14 +148,15 @@ int zn_decode_verify_batch(zn_ctx* ctx, const uint8_t* blobs_base, const uint64_
  * times longer.  A match never reaches into another slice, and a frame depends only on its slice's bytes.  LZ4 has
  * one effort.  The frame is always decodable by stock libzstd / liblz4.
  * codec ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE (levels <= 19): the blob is the seekable layout described at the codec enum;
- * ZN_E_ARG for LZ4 or a level >= 20 with the flag.
+ * ZN_E_ARG for LZ4 or a level >= 20 with the flag.  | ZN_CODEC_CHECKSUM (zstd or LZ4, not seekable): every frame ends
+ * in its content checksum.
  */
 int zn_compress_batch(zn_ctx* ctx, const uint8_t* src_base, const uint64_t* src_off, const uint64_t* src_len,
                       uint32_t n, int level, int codec, uint8_t* dst_base, const uint64_t* dst_off,
                       uint64_t* dst_len_out, uint8_t* digest_out /* nullable */, uint32_t* status);
 
 /* ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE: exact, per 128 KiB block 13 + 3 + the block's bytes + 12, plus 17 for the seek
- * table; 38 for an empty slice. */
+ * table; 38 for an empty slice.  ZN_CODEC_CHECKSUM adds 4 bytes. */
 size_t zn_compress_bound(size_t src_len, int codec);
 /* device time (ms, CUDA events) of the compression kernels of the most recent zn_compress_batch on this ctx */
 float zn_ctx_last_compress_ms(const zn_ctx* ctx);
@@ -304,7 +313,8 @@ const char* zn_archive_writer_error(const zn_archive_writer* w);
  * lets io_threads readers pread the bytes into place — the whole directory in one call.
  * codec ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE (levels <= 19) writes seekable blobs and the index metadata
  * znippy_seekable = "zstd"; with LZ4 or a level >= 20 zn_archive_writer_create returns NULL and zn_archive_compress_dir
- * returns ZN_E_ARG with a message. */
+ * returns ZN_E_ARG with a message.  codec | ZN_CODEC_CHECKSUM (zstd or LZ4, not seekable) writes a content checksum
+ * into every compressed row's frame. */
 int zn_archive_compress_dir(zn_ctx* ctx, const char* input_dir, const char* output_path, int no_skip, int level, int codec,
                             size_t slot_bytes, int io_threads, zn_compression_report* report, char* err, size_t errcap);
 /* pinned host memory (cudaHostAlloc) for callers that stage their own buffers */
@@ -371,11 +381,11 @@ int zn_plan_last_ms(zn_plan* plan, float ms[4]);
  * d_src[h_src_off[i] .. + h_src_len[i]) of every run.  `level` and `codec` as for zn_compress_batch; `digests` != 0 also
  * hashes the source slices (the zn_hash_batch kernels, on the run's stream).  All planning, uploads and allocation
  * happen here.  NULL, with zn_last_error set, for a slice of 4 GiB or more, a codec other than ZN_CODEC_ZSTD
- * (optionally | ZN_CODEC_SEEKABLE) / ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE, or ZN_CODEC_SEEKABLE at a level
- * >= 20.  Seekable plans also run the frame checksum kernel, counted in stage [1] of zn_plan_last_ms.  n = 0 is a valid
- * plan. */
+ * (optionally | ZN_CODEC_SEEKABLE or | ZN_CODEC_CHECKSUM) / ZN_CODEC_LZ4 (optionally | ZN_CODEC_CHECKSUM), optionally
+ * | ZN_CODEC_ENVELOPE, or ZN_CODEC_SEEKABLE at a level >= 20.  Seekable plans also run the frame checksum kernel, and
+ * checksummed plans the slice checksum kernel, counted in stage [1] of zn_plan_last_ms.  n = 0 is a valid plan. */
 zn_plan* zn_plan_compress(zn_ctx* ctx, uint32_t n, const uint64_t* h_src_off, const uint64_t* h_src_len, int level,
-                          int codec /* ZN_CODEC_ZSTD [| ZN_CODEC_SEEKABLE] | ZN_CODEC_LZ4, optionally | ZN_CODEC_ENVELOPE */,
+                          int codec /* ZN_CODEC_ZSTD [| ZN_CODEC_SEEKABLE] | ZN_CODEC_LZ4, optionally | ZN_CODEC_CHECKSUM, | ZN_CODEC_ENVELOPE */,
                           int digests);
 /* bytes d_dst must hold for any input of these sizes */
 uint64_t zn_plan_compress_capacity(const zn_plan* plan);

@@ -15,6 +15,7 @@ S_OK, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_UNSUPPORTED, S_SIZE_
 CODEC_ZSTD, CODEC_LZ4 = 1, 2
 CODEC_ENVELOPE = 0x100  # archive writer and compress plans: wrap compressed rows in ZNB1 (include/znippy_cuda.h)
 CODEC_SEEKABLE = 0x400  # OR-ed into CODEC_ZSTD (levels <= 19): one frame per 128 KiB block + a seek table
+CODEC_CHECKSUM = 0x800  # OR-ed into CODEC_ZSTD / CODEC_LZ4: every frame ends in its content checksum (not with SEEKABLE)
 
 EXPORTS = [
     "zn_abi_version", "zn_device_count", "zn_strerror", "zn_status_name", "zn_ctx_create", "zn_ctx_destroy",
@@ -261,13 +262,16 @@ class Plan:
 
     @classmethod
     def compress(cls, ctx: Ctx, src_off, src_len, level: int = 1, codec: int = CODEC_ZSTD, envelope: bool = False,
-                 digests: bool = True, seekable: bool = False) -> "Plan":
+                 digests: bool = True, seekable: bool = False, checksum: bool = False) -> "Plan":
         """Compress plan over slices resident on the device (zn_plan_compress): slice i = d_src[src_off[i] : + src_len[i]]
         of every run_compress.  envelope=True: ZNB1 blobs, RAW when the frame does not shrink the slice.
-        seekable=True (zstd, levels <= 19): every blob is the seekable layout (CODEC_SEEKABLE)."""
+        seekable=True (zstd, levels <= 19): every blob is the seekable layout (CODEC_SEEKABLE).  checksum=True: every
+        frame ends in its content checksum (CODEC_CHECKSUM); not together with seekable=True."""
+        if seekable and checksum:
+            raise ValueError("checksum=True cannot be combined with seekable=True: the seek table carries the checksums")
         o, l = u64(src_off), u64(src_len)
         assert l.size == o.size
-        flags = (CODEC_ENVELOPE if envelope else 0) | (CODEC_SEEKABLE if seekable else 0)
+        flags = (CODEC_ENVELOPE if envelope else 0) | (CODEC_SEEKABLE if seekable else 0) | (CODEC_CHECKSUM if checksum else 0)
         h = lib().zn_plan_compress(ctx.handle, o.size, ptr(o), ptr(l), level, codec | flags, 1 if digests else 0)
         return cls(ctx, h, o.size)
 

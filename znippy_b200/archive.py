@@ -488,19 +488,23 @@ class StreamCompressor:
 
     def __init__(self, output: str, no_skip: bool, level: int = 19, codec_id: int = codec.CODEC_ZSTD,
                  ctx: Ctx | None = None, batch_bytes: int = 256 << 20, native_index: bool = True, native: bool = True,
-                 envelope: bool = False, seekable: bool = False):
+                 envelope: bool = False, seekable: bool = False, checksum: bool = False):
         """level defaults to the reference's compression_level = 19 (common_config.rs:37); levels 20-22 select the
         long effort of the zstd match finder (smaller frames, slower writes; codec.CompressCtx).  envelope=True (native
         writer only): blobs of compressed rows are ZNB1 envelopes, incompressible slices are stored raw inside them.
         seekable=True (native writer, zstd at levels <= 19): compressed rows are seekable blobs, and range reads decode
-        only the 128 KiB frames they touch."""
+        only the 128 KiB frames they touch.  checksum=True: every compressed row's frame ends in its content checksum
+        (XXH64 for zstd, XXH32 for LZ4; codec.CompressCtx), which every read checks; not together with seekable=True."""
         if envelope and not native:
             raise ValueError("the ZNB1 envelope is written by the native pipeline only")
         if seekable and not native:
             raise ValueError("seekable archives are written by the native pipeline only")
         if seekable and (codec_id != codec.CODEC_ZSTD or level >= 20):
             raise ValueError("seekable archives need the zstd codec at a level <= 19")
+        if seekable and checksum:
+            raise ValueError("checksum=True cannot be combined with seekable=True: the seek table carries the checksums")
         self.envelope = envelope
+        self.checksum = checksum
         self.seekable = seekable
         self.native_index = native_index
         self.native = native
@@ -515,7 +519,8 @@ class StreamCompressor:
             self._ctx = self.ctx or default_ctx()
             self._w = N.lib().zn_archive_writer_create(self._ctx.handle, self.output.encode(), int(self.no_skip), self.level,
                                                        self.codec_id | (N.CODEC_ENVELOPE if self.envelope else 0) |
-                                                       (N.CODEC_SEEKABLE if self.seekable else 0), self.batch_bytes)
+                                                       (N.CODEC_SEEKABLE if self.seekable else 0) |
+                                                       (N.CODEC_CHECKSUM if self.checksum else 0), self.batch_bytes)
             if not self._w:
                 raise IOError(f"cannot create {self.output}")
         return self._w
@@ -583,7 +588,7 @@ class StreamCompressor:
                 payload, digest = [None] * len(batch), [None] * len(batch)
                 if ci:
                     bl, dg, st = codec.compress_batch(src, [offs[i] for i in ci], [lens[i] for i in ci], self.level,
-                                                      self.codec_id, self.ctx)
+                                                      self.codec_id | (codec.CODEC_CHECKSUM if self.checksum else 0), self.ctx)
                     for k, i in enumerate(ci):
                         if st[k] != codec.S_OK:
                             raise codec.CodecError(int(st[k]), "compress")  # `?` propagates, stream_packer.rs:230
@@ -668,20 +673,24 @@ def compress_stream(output: str, no_skip: bool, **kw) -> StreamCompressor:
 
 def compress_dir(input_dir: str, output: str, no_skip: bool = False, level: int = 19, codec_id: int = codec.CODEC_ZSTD,
                  ctx: Ctx | None = None, envelope: bool = False, io_threads: int = 8, slot_bytes: int = 256 << 20,
-                 seekable: bool = False) -> CompressionReport:
+                 seekable: bool = False, checksum: bool = False) -> CompressionReport:
     """znippy-compress `compress_dir` (walk -> readers -> Magazine slots -> workers -> writer, slot_packer.rs:329-609) in
     one native call: `zn_archive_compress_dir` walks the directory, places every round in a pinned slot, lets
     `io_threads` readers pread the bytes into place, and runs the same three-stage slot pipeline as compress_stream.
-    `level` as in compress_stream: 19 by default, 20-22 for the long effort; `seekable` as in compress_stream."""
+    `level` as in compress_stream: 19 by default, 20-22 for the long effort; `seekable` and `checksum` as in
+    compress_stream."""
     import ctypes as C
 
     from . import _native as N
+    if seekable and checksum:
+        raise ValueError("checksum=True cannot be combined with seekable=True: the seek table carries the checksums")
     ctx = ctx or default_ctx()
     out = os.path.splitext(output)[0] + ".znippy"
     rep8 = (C.c_uint64 * 8)()
     err = C.create_string_buffer(512)
     rc = N.lib().zn_archive_compress_dir(ctx.handle, input_dir.encode(), out.encode(), int(no_skip), level,
-                                         codec_id | (N.CODEC_ENVELOPE if envelope else 0) | (N.CODEC_SEEKABLE if seekable else 0),
+                                         codec_id | (N.CODEC_ENVELOPE if envelope else 0) | (N.CODEC_SEEKABLE if seekable else 0) |
+                                         (N.CODEC_CHECKSUM if checksum else 0),
                                          slot_bytes, io_threads, C.byref(rep8), err, 512)
     if rc != 0:
         raise N.NativeError(f"zn_archive_compress_dir: {err.value.decode(errors='replace')}")

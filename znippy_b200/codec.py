@@ -19,7 +19,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
-from ._native import (CODEC_LZ4, CODEC_SEEKABLE, CODEC_ZSTD, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_OK,  # noqa: F401
+from ._native import (CODEC_CHECKSUM, CODEC_LZ4, CODEC_SEEKABLE, CODEC_ZSTD, S_DECODE_ERROR, S_DIGEST_MISMATCH, S_DST_TOO_SMALL, S_OK,  # noqa: F401
                       S_SIZE_MISMATCH, S_UNSUPPORTED, Ctx, NativeError, default_ctx)
 
 
@@ -164,12 +164,17 @@ class CompressCtx:
     """codec.rs:8-55.  `level` follows the reference's meaning (higher = more effort); the GPU match finder has
     four efforts: three window geometries for levels <= 2, 3..9 and 10..19, and for levels >= 20 (zstd only) the long
     effort, whose matches reach back anywhere in the slice up to 8 MiB (DESIGN.md §4.3).  seekable=True (zstd, levels
-    <= 19): one independent frame per 128 KiB block and a seek table (CODEC_SEEKABLE, DESIGN.md §4.3)."""
+    <= 19): one independent frame per 128 KiB block and a seek table (CODEC_SEEKABLE, DESIGN.md §4.3).  checksum=True:
+    every frame ends in its content checksum, XXH64 for zstd and XXH32 for LZ4 (CODEC_CHECKSUM), as the zstd and lz4
+    tools write by default; not together with seekable=True, whose seek table already carries a checksum per frame."""
 
     def __init__(self, compression_level: int, codec: int = CODEC_ZSTD, ctx: Ctx | None = None, envelope: bool = False,
-                 seekable: bool = False):
+                 seekable: bool = False, checksum: bool = False):
+        if seekable and checksum:
+            raise ValueError("checksum=True cannot be combined with seekable=True: the seek table carries the checksums")
         self.level = int(compression_level)
-        self.codec = codec | (CODEC_SEEKABLE if seekable else 0)
+        self.base = codec
+        self.codec = codec | (CODEC_SEEKABLE if seekable else 0) | (CODEC_CHECKSUM if checksum else 0)
         self.ctx = ctx or default_ctx()
         self.envelope = envelope  # wrap every frame in ZNB1; incompressible input is then stored RAW (size + 6..10 bytes)
 
@@ -185,7 +190,7 @@ class CompressCtx:
         if self.envelope:
             if len(blobs[0]) >= b.size:
                 return envelope_wrap(PAYLOAD_RAW, b.size, b.tobytes())
-            return envelope_wrap(PAYLOAD_LZ4_FRAME if self.codec == CODEC_LZ4 else PAYLOAD_ZSTD, b.size, blobs[0])
+            return envelope_wrap(PAYLOAD_LZ4_FRAME if self.base == CODEC_LZ4 else PAYLOAD_ZSTD, b.size, blobs[0])
         return blobs[0]
 
     def compress_into(self, data, out: bytearray) -> int:

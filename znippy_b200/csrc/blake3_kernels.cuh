@@ -26,14 +26,6 @@ constexpr int kB3StageBytes = 32 * kB3RowStride;
 constexpr int kB3SmemPerWarp = kB3Stages * kB3StageBytes;
 constexpr int kB3RowsPerIssue = 32 / (kB3RowBytes / 16);  // rows covered by one warp-wide 16-byte copy (4)
 
-ZN_D void cp_async16(void* smem_dst, const void* gmem_src) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem_src) : "memory");
-}
-ZN_D void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N>
-ZN_D void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-
 // Stage `stage_idx` (bytes [stage_idx*128, +128) of each of the warp's 32 chunks) -> shared memory.
 // ptr/len are this lane's chunk; rows are other lanes' chunks, fetched by shuffle.  `regular` (warp-uniform) = the 32
 // chunks are full, 16-byte aligned and contiguous in memory (the common case inside a large blob): rows are then
@@ -174,13 +166,12 @@ __global__ void __launch_bounds__(kB3Warps * 32) k_b3_chunks(const BlobDesc* __r
   }
 }
 
-// digest = cv words little-endian; compare with expect and fold into status (decode errors win).
+// digest = cv words little-endian; compare with expect and fold into status (decode errors win).  xxh_bad: a checksum of
+// the row's frames disagrees with its bytes (xxh_verify.cuh), a decode error.
 ZN_D void finish_blob(const BlobDesc& d, uint32_t blob, const uint32_t (&cv)[8], uint32_t* __restrict__ digests,
-                      const uint32_t* __restrict__ expect, uint32_t* __restrict__ status, const uint8_t* blobs_base,
-                      const uint8_t* out_base) {
+                      const uint32_t* __restrict__ expect, uint32_t* __restrict__ status, bool xxh_bad) {
   b3::store_cv(digests + (uint64_t)blob * 8, cv);
-  // Zstandard content checksum (xxh_verify.cuh): a decoded row whose frame says XXH64 != content is a decode error
-  if (out_base && status[blob] == S_OK && xxh_row_bad(d, blobs_base, out_base)) status[blob] = S_DECODE_ERROR;
+  if (xxh_bad && status[blob] == S_OK) status[blob] = S_DECODE_ERROR;
   if ((d.flags & F_HAS_EXPECT) && status[blob] == S_OK) {
     bool eq = true;
 #pragma unroll
@@ -218,12 +209,59 @@ __global__ void __launch_bounds__(128) k_b3_tree_small(const BlobDesc* __restric
     n = pairs + (n & 1);
   }
   b3::load_cv(base, o);
-  finish_blob(d, blob, o, digests, expect, status, blobs_base, out_base);
+  finish_blob(d, blob, o, digests, expect, status, out_base && status[blob] == S_OK && xxh_row_bad(d, blobs_base, out_base));
+}
+
+// Checksums of one decoded row by a whole CTA (xxh_verify.cuh): thread 0 walks the frame and block headers into a list
+// of spans in shared memory, the warps hash the spans (xxh_warp).  A row with more spans than the list holds is walked
+// again for each further part of the list.
+constexpr uint32_t kRowSpans = 256;
+struct XxhSpan {
+  const uint8_t* p;
+  uint64_t len;
+  uint32_t bits, want;
+};
+struct XxhSpanList {  // emit() of xxh_row_walk: keeps spans [first, first + kRowSpans), counts them all
+  XxhSpan* list;
+  uint32_t first, total = 0;
+  ZN_D bool operator()(const uint8_t* p, uint64_t len, uint32_t bits, uint32_t want) {
+    if (total >= first && total - first < kRowSpans) list[total - first] = XxhSpan{p, len, bits, want};
+    total++;
+    return true;
+  }
+};
+template <int kThreads>
+ZN_D bool xxh_row_bad_cta(const BlobDesc& d, bool ok, const uint8_t* blobs_base, const uint8_t* out_base) {
+  __shared__ XxhSpan spans[kRowSpans];
+  __shared__ uint32_t n_spans, more, bad;
+  __shared__ __align__(16) uint8_t ring[kThreads / 32][kXxhRing];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  for (uint32_t first = 0;; first += kRowSpans) {
+    if (threadIdx.x == 0) {
+      XxhSpanList l{spans, first};
+      if (ok) xxh_row_walk(d, blobs_base, out_base, l);
+      n_spans = l.total > first ? min(l.total - first, kRowSpans) : 0u;
+      more = l.total > first + kRowSpans;
+      if (first == 0) bad = 0;
+    }
+    __syncthreads();
+    for (uint32_t k = warp; k < n_spans; k += kThreads / 32) {
+      const XxhSpan sp = spans[k];
+      const uint32_t h = sp.bits == 64 ? (uint32_t)xxh_warp<64>(sp.p, sp.len, ring[warp], lane)
+                                       : (uint32_t)xxh_warp<32>(sp.p, sp.len, ring[warp], lane);
+      if (lane == 0 && h != sp.want) bad = 1;
+    }
+    __syncthreads();
+    const bool stop = !more || bad;
+    __syncthreads();  // everyone has read `more` and `bad` before thread 0 walks again
+    if (stop) return bad;
+  }
 }
 
 // K3c: large blobs: one CTA per blob, every level spread over the CTA.  Levels ping-pong between the blob's slots in
 // `cvs` and in `cvs2` (same layout), so a level needs no barrier between its items — the 8 warps run their (load, load,
-// compress, store) items independently and hide each other's L2 round trips — only one barrier per level.
+// compress, store) items independently and hide each other's L2 round trips — only one barrier per level.  Then the
+// CTA checks the row's frame checksums.
 __global__ void __launch_bounds__(512) k_b3_tree_large(const BlobDesc* __restrict__ blobs,
                                                        const uint32_t* __restrict__ list,
                                                        uint32_t* cvs, uint32_t* cvs2, uint32_t* __restrict__ digests,
@@ -253,9 +291,10 @@ __global__ void __launch_bounds__(512) k_b3_tree_large(const BlobDesc* __restric
     uint32_t* t = src; src = dst; dst = t;
     n = items;
   }
+  const bool bad = out_base && xxh_row_bad_cta<512>(d, status[blob] == S_OK, blobs_base, out_base);
   if (threadIdx.x == 0) {
     b3::load_cv(src, o);
-    finish_blob(d, blob, o, digests, expect, status, blobs_base, out_base);
+    finish_blob(d, blob, o, digests, expect, status, bad);
   }
 }
 

@@ -49,6 +49,17 @@ struct BlobDesc {
   uint32_t flags;
 };
 
+#if defined(__CUDACC__)
+// 16-byte global -> shared copies that bypass L1 (the hash kernels stage their input through these)
+ZN_D void cp_async16(void* smem_dst, const void* gmem_src) {
+  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem_dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem_src) : "memory");
+}
+ZN_D void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
+template <int N>
+ZN_D void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
+#endif
+
 constexpr uint32_t kChunk = 1024;
 constexpr uint32_t kWarp = 32;
 constexpr uint32_t kZstdBlockMax = 128u * 1024u;

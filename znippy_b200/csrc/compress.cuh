@@ -243,10 +243,11 @@ ZN_HD uint32_t lz4_compress_block(const Warp& w, const uint8_t* in, uint32_t n, 
   return op;
 }
 
-// LZ4 frame header for a slice of `content` bytes (15 bytes): independent 64 KiB blocks, content size present.
-ZN_HD uint32_t lz4_frame_header(uint8_t* dst, uint64_t content) {
+// LZ4 frame header for a slice of `content` bytes (15 bytes): independent 64 KiB blocks, content size present, and
+// with `checksum` (ZN_CODEC_CHECKSUM) the content checksum flag.
+ZN_HD uint32_t lz4_frame_header(uint8_t* dst, uint64_t content, bool checksum = false) {
   dst[0] = 0x04; dst[1] = 0x22; dst[2] = 0x4D; dst[3] = 0x18;
-  dst[4] = 0x68;  // version 01, B.Indep, C.Size
+  dst[4] = checksum ? 0x6C : 0x68;  // version 01, B.Indep, C.Size[, C.Checksum]
   dst[5] = 0x40;  // 64 KiB blocks
   for (int i = 0; i < 8; i++) dst[6 + i] = (uint8_t)(content >> (8 * i));
   // XXH32 of the 10 descriptor bytes (len < 16 path)
@@ -1309,10 +1310,11 @@ ZN_HD uint32_t zstd_long_block(const Warp& w, const uint8_t* s, const LongIndex&
   return zstd_block_payload(w, stage, nlit, seqs, nseq, n, scratch, payload_off);
 }
 
-// Zstandard frame header: single segment, 8-byte content size (13 bytes); empty content uses the 1-byte form.
-ZN_HD uint32_t zstd_frame_header(uint8_t* dst, uint64_t content) {
+// Zstandard frame header: single segment, 8-byte content size (13 bytes), and with `checksum` (ZN_CODEC_CHECKSUM) the
+// content checksum flag; empty content uses the 1-byte form (zstd_empty_frame).
+ZN_HD uint32_t zstd_frame_header(uint8_t* dst, uint64_t content, bool checksum = false) {
   dst[0] = 0x28; dst[1] = 0xB5; dst[2] = 0x2F; dst[3] = 0xFD;
-  dst[4] = 0xE0;
+  dst[4] = checksum ? 0xE4 : 0xE0;
   for (int i = 0; i < 8; i++) dst[5 + i] = (uint8_t)(content >> (8 * i));
   return 13;
 }
@@ -1324,20 +1326,25 @@ ZN_HD void zstd_block_header(uint8_t* dst, uint32_t last, uint32_t type, uint32_
 // ---- sizes of what the assemble kernels (compress_kernels.cuh) write for a slice of n bytes, from the per-block
 // results alone: a packed layout is computed on the device before any frame byte exists.
 // zstd: meta = the slice's first {payload offset, size} pair (size 0 = raw block); the empty frame is 9 bytes.
-ZN_HD uint64_t zstd_frame_size(uint64_t n, const uint32_t* meta) {
-  if (n == 0) return 9;
-  uint64_t sz = 13;
+// `checksum`: 4 more bytes, the content checksum behind the last block.
+ZN_HD uint64_t zstd_frame_size(uint64_t n, const uint32_t* meta, bool checksum = false) {
+  if (n == 0) return checksum ? 13 : 9;
+  uint64_t sz = checksum ? 17 : 13;
   for (uint64_t o = 0, j = 0; o < n; o += kZstdCBlock, j++) {
     const uint32_t bn = (uint32_t)(n - o < kZstdCBlock ? n - o : kZstdCBlock), c = meta[2 * j + 1];
     sz += 3 + (c ? c : bn);
   }
   return sz;
 }
-// The empty frame, as libzstd writes it: single segment, 1-byte content size 0, empty raw last block (9 bytes).
-ZN_HD uint32_t zstd_empty_frame(uint8_t* dst) {
-  const uint8_t e[9] = {0x28, 0xB5, 0x2F, 0xFD, 0x20, 0x00, 0x01, 0x00, 0x00};
+// The empty frame, as libzstd writes it: single segment, 1-byte content size 0, empty raw last block (9 bytes); with
+// `checksum` as libzstd writes it with ZSTD_c_checksumFlag: descriptor 0x24 and XXH64("") behind the block (13 bytes).
+ZN_HD uint32_t zstd_empty_frame(uint8_t* dst, bool checksum = false) {
+  const uint8_t e[13] = {0x28, 0xB5, 0x2F, 0xFD, 0x20, 0x00, 0x01, 0x00, 0x00, 0x99, 0xE9, 0xD8, 0x51};
   for (int k = 0; k < 9; k++) dst[k] = e[k];
-  return 9;
+  if (!checksum) return 9;
+  dst[4] = 0x24;
+  for (int k = 9; k < 13; k++) dst[k] = e[k];
+  return 13;
 }
 
 // ---- seekable layout (ZN_CODEC_SEEKABLE): every kZstdCBlock block of the slice is a frame of its own (the 13-byte
@@ -1380,9 +1387,10 @@ ZN_HD uint32_t zstd_seek_table(uint8_t* dst, uint64_t n, const uint32_t* meta, c
   return kSeekFixed + kSeekEntry * nf;
 }
 
-// LZ4: csize = the slice's first block size (>= the block's input size means stored); 15-byte header, 4-byte EndMark
-ZN_HD uint64_t lz4_frame_size(uint64_t n, const uint32_t* csize) {
-  uint64_t sz = 15 + 4;
+// LZ4: csize = the slice's first block size (>= the block's input size means stored); 15-byte header, 4-byte EndMark,
+// and with `checksum` the 4-byte content checksum
+ZN_HD uint64_t lz4_frame_size(uint64_t n, const uint32_t* csize, bool checksum = false) {
+  uint64_t sz = 15 + 4 + (checksum ? 4 : 0);
   for (uint64_t o = 0, j = 0; o < n; o += kLz4Block, j++) {
     const uint32_t bn = (uint32_t)(n - o < kLz4Block ? n - o : kLz4Block), c = csize[j];
     sz += 4 + (c < bn ? c : bn);

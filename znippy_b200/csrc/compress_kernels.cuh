@@ -57,13 +57,14 @@ __global__ void __launch_bounds__(kLz4WarpsPerCta * 32) k_lz4_blocks(const Slice
   }
 }
 
-// ---- LZ4 frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_lz4_assemble: one CTA per slice)
+// ---- LZ4 frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_lz4_assemble: one CTA per slice).
+// csum: nullptr, or the slice checksums of a ZN_CODEC_CHECKSUM batch (k_slice_xxh), stored behind the EndMark.
 ZN_D void lz4_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base, const uint8_t* tmp,
-                       const uint32_t* __restrict__ csize, uint8_t* dst_base, uint64_t* dst_len) {
+                       const uint32_t* __restrict__ csize, const uint32_t* __restrict__ csum, uint8_t* dst_base, uint64_t* dst_len) {
   const SliceDesc s = slices[i];
   uint8_t* dst = dst_base + s.dst_off;
   const Team t{threadIdx.x, blockDim.x};
-  if (threadIdx.x == 0) cz::lz4_frame_header(dst, s.src_len);
+  if (threadIdx.x == 0) cz::lz4_frame_header(dst, s.src_len, csum != nullptr);
   uint64_t op = 15;
   for (uint32_t b = 0; b < s.n_blocks; b++) {
     const uint32_t j = s.blk_first + b;
@@ -81,13 +82,15 @@ ZN_D void lz4_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const u
   }
   if (threadIdx.x == 0) {
     dst[op] = dst[op + 1] = dst[op + 2] = dst[op + 3] = 0;  // EndMark
-    dst_len[i] = op + 4;
+    op += 4;
+    if (csum) { cz::put_le32(dst + op, csum[i]); op += 4; }
+    dst_len[i] = op;
   }
 }
 __global__ void __launch_bounds__(256) k_lz4_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
-                                                      const uint8_t* tmp, const uint32_t* __restrict__ csize, uint8_t* dst_base,
-                                                      uint64_t* dst_len) {
-  lz4_assemble(slices, blockIdx.x, src_base, tmp, csize, dst_base, dst_len);
+                                                      const uint8_t* tmp, const uint32_t* __restrict__ csize,
+                                                      const uint32_t* __restrict__ csum, uint8_t* dst_base, uint64_t* dst_len) {
+  lz4_assemble(slices, blockIdx.x, src_base, tmp, csize, csum, dst_base, dst_len);
 }
 
 // ---- zstd: every 128 KiB block of every slice -> staged payload; meta[2j] = payload offset in the slot, meta[2j+1] = size (0 = raw)
@@ -171,17 +174,18 @@ __global__ void __launch_bounds__(32) k_long_blocks(const LongUnit* __restrict__
   }
 }
 
-// ---- zstd frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_zstd_assemble: one CTA per slice)
+// ---- zstd frame assembly: the CTA writes slice i's frame at dst_base + dst_off (k_zstd_assemble: one CTA per slice).
+// csum: nullptr, or the slice checksums of a ZN_CODEC_CHECKSUM batch (k_slice_xxh), stored behind the last block.
 ZN_D void zstd_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base, const uint8_t* tmp,
-                        const uint32_t* __restrict__ meta, uint8_t* dst_base, uint64_t* dst_len) {
+                        const uint32_t* __restrict__ meta, const uint32_t* __restrict__ csum, uint8_t* dst_base, uint64_t* dst_len) {
   const SliceDesc s = slices[i];
   uint8_t* dst = dst_base + s.dst_off;
   const Team t{threadIdx.x, blockDim.x};
   if (s.src_len == 0) {
-    if (threadIdx.x == 0) dst_len[i] = cz::zstd_empty_frame(dst);
+    if (threadIdx.x == 0) dst_len[i] = cz::zstd_empty_frame(dst, csum != nullptr);
     return;
   }
-  if (threadIdx.x == 0) cz::zstd_frame_header(dst, s.src_len);
+  if (threadIdx.x == 0) cz::zstd_frame_header(dst, s.src_len, csum != nullptr);
   uint64_t op = 13;
   for (uint32_t b = 0; b < s.n_blocks; b++) {
     const uint32_t j = s.blk_first + b;
@@ -199,7 +203,10 @@ ZN_D void zstd_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const 
       op += 3 + c;
     }
   }
-  if (threadIdx.x == 0) dst_len[i] = op;
+  if (threadIdx.x == 0) {
+    if (csum) { cz::put_le32(dst + op, csum[i]); op += 4; }
+    dst_len[i] = op;
+  }
 }
 // Seekable slice (cz::zstd_seek_table): one frame per block, then the seek table; xxh[j] = checksum of global block j.
 ZN_D void zstd_seekable_assemble(const SliceDesc* __restrict__ slices, uint32_t i, const uint8_t* __restrict__ src_base,
@@ -224,12 +231,13 @@ ZN_D void zstd_seekable_assemble(const SliceDesc* __restrict__ slices, uint32_t 
   }
   if (threadIdx.x == 0) dst_len[i] = op + cz::zstd_seek_table(dst + op, s.src_len, meta + 2 * (size_t)s.blk_first, xxh + s.blk_first);
 }
-// xxh: nullptr, or the block checksums of a seekable batch (k_block_xxh)
+// xxh: nullptr, or the block checksums of a seekable batch (k_block_xxh); csum as for zstd_assemble
 __global__ void __launch_bounds__(256) k_zstd_assemble(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
                                                        const uint8_t* tmp, const uint32_t* __restrict__ meta,
-                                                       const uint32_t* __restrict__ xxh, uint8_t* dst_base, uint64_t* dst_len) {
+                                                       const uint32_t* __restrict__ xxh, const uint32_t* __restrict__ csum,
+                                                       uint8_t* dst_base, uint64_t* dst_len) {
   if (xxh) zstd_seekable_assemble(slices, blockIdx.x, src_base, tmp, meta, xxh, dst_base, dst_len);
-  else zstd_assemble(slices, blockIdx.x, src_base, tmp, meta, dst_base, dst_len);
+  else zstd_assemble(slices, blockIdx.x, src_base, tmp, meta, csum, dst_base, dst_len);
 }
 
 // ---- seekable batches: xxh[j] = low 32 bits of XXH64 of global block j's source bytes (one thread per block: XXH64 is
@@ -246,13 +254,28 @@ __global__ void __launch_bounds__(kXxhThreads) k_block_xxh(const SliceDesc* __re
   }
 }
 
+// ---- ZN_CODEC_CHECKSUM batches: csum[i] = XXH64 (zstd, low 32 bits) or XXH32 (LZ4) of slice i, seed 0; one warp per
+// slice (xxh_warp: the source staged through shared memory, one lane per accumulator chain)
+constexpr int kSliceXxhWarps = 4;
+template <int Bits>
+__global__ void __launch_bounds__(kSliceXxhWarps * 32) k_slice_xxh(const SliceDesc* __restrict__ slices, uint32_t n,
+                                                                   const uint8_t* __restrict__ src_base, uint32_t* csum) {
+  __shared__ __align__(16) uint8_t ring[kSliceXxhWarps][kXxhRing];
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  for (uint32_t i = blockIdx.x * kSliceXxhWarps + warp; i < n; i += gridDim.x * kSliceXxhWarps) {
+    const SliceDesc s = slices[i];
+    const uint32_t h = (uint32_t)xxh_warp<Bits>(src_base + s.src_off, s.src_len, ring[warp], lane);
+    if (lane == 0) csum[i] = h;
+  }
+}
+
 // ---- packed layout (device-resident compress plans): blob i = [ZNB1 header] + frame, or header + the slice's bytes when
 // the envelope stores it RAW; blobs back to back.  One CTA: per tile of slices, every thread sizes one slice from the
 // block results (cz::zstd_frame_size / zstd_seekable_size / lz4_frame_size), the CTA scans the sizes, and each thread writes its slice's
 // offset, its frame's destination (past the header) into slices[i].dst_off, the RAW decision and the header.
 constexpr int kLayoutThreads = 1024;
 __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slices, uint32_t n, const uint32_t* __restrict__ res,
-                                                                uint32_t lz4, uint32_t seekable, uint32_t envelope,
+                                                                uint32_t lz4, uint32_t seekable, uint32_t checksum, uint32_t envelope,
                                                                 uint8_t* dst_base, uint64_t* offsets, uint32_t* raw) {
   __shared__ uint64_t warp_sum[kLayoutThreads / 32];
   const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
@@ -264,9 +287,9 @@ __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slice
     if (i < n) {
       const SliceDesc s = slices[i];
       len = s.src_len;
-      sz = lz4        ? cz::lz4_frame_size(len, res + s.blk_first)
+      sz = lz4        ? cz::lz4_frame_size(len, res + s.blk_first, checksum != 0)
            : seekable ? cz::zstd_seekable_size(len, res + 2 * (size_t)s.blk_first)
-                      : cz::zstd_frame_size(len, res + 2 * (size_t)s.blk_first);
+                      : cz::zstd_frame_size(len, res + 2 * (size_t)s.blk_first, checksum != 0);
       if (envelope) {
         r = sz >= len;
         hl = cz::znb1_header_len(len);
@@ -301,20 +324,20 @@ __global__ void __launch_bounds__(kLayoutThreads) k_pack_layout(SliceDesc* slice
 }
 
 // Frames straight into the packed layout (one CTA per slice); a RAW row gets the slice's bytes instead of its frame.
-// dst_len receives the frame lengths, as from k_zstd_assemble / k_lz4_assemble; xxh as for k_zstd_assemble.
+// dst_len receives the frame lengths, as from k_zstd_assemble / k_lz4_assemble; xxh and csum as for k_zstd_assemble.
 template <bool LZ4>
 __global__ void __launch_bounds__(256) k_assemble_packed(const SliceDesc* __restrict__ slices, const uint8_t* __restrict__ src_base,
                                                          const uint8_t* tmp, const uint32_t* __restrict__ res,
-                                                         const uint32_t* __restrict__ xxh, const uint32_t* __restrict__ raw,
-                                                         uint8_t* dst_base, uint64_t* dst_len) {
+                                                         const uint32_t* __restrict__ xxh, const uint32_t* __restrict__ csum,
+                                                         const uint32_t* __restrict__ raw, uint8_t* dst_base, uint64_t* dst_len) {
   if (raw[blockIdx.x]) {
     const SliceDesc s = slices[blockIdx.x];
     team_copy(Team{threadIdx.x, blockDim.x}, dst_base + s.dst_off, src_base + s.src_off, (uint32_t)s.src_len);
     return;
   }
-  if (LZ4) lz4_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
+  if (LZ4) lz4_assemble(slices, blockIdx.x, src_base, tmp, res, csum, dst_base, dst_len);
   else if (xxh) zstd_seekable_assemble(slices, blockIdx.x, src_base, tmp, res, xxh, dst_base, dst_len);
-  else zstd_assemble(slices, blockIdx.x, src_base, tmp, res, dst_base, dst_len);
+  else zstd_assemble(slices, blockIdx.x, src_base, tmp, res, csum, dst_base, dst_len);
 }
 
 }  // namespace zn

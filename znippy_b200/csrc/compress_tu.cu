@@ -19,11 +19,13 @@ void compress_init_attrs() {
 }
 
 size_t compress_bound(size_t n, int codec) {
+  const CodecWord cw = codec_parts(codec);
   const size_t nb = (n + cz::kZstdCBlock - 1) / cz::kZstdCBlock;
-  if (codec & kCodecSeekable)  // exact: every block stored raw in a frame of its own (cz::zstd_seekable_size)
+  if (cw.seekable)  // exact: every block stored raw in a frame of its own (cz::zstd_seekable_size)
     return n ? n + (13 + 3 + cz::kSeekEntry) * nb + cz::kSeekFixed : 9 + cz::kSeekEntry + cz::kSeekFixed;
-  if (codec == 2) return n + 4 * ((n + cz::kLz4Block - 1) / cz::kLz4Block) + 32;
-  return n + 3 * nb + 32;
+  const size_t ck = cw.checksum ? 4 : 0;
+  if (cw.base == ZN_CODEC_LZ4) return n + 4 * ((n + cz::kLz4Block - 1) / cz::kLz4Block) + 32 + ck;
+  return n + 3 * nb + 32 + ck;
 }
 
 template <typename T>
@@ -142,17 +144,12 @@ static int long_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, cons
 }
 
 int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const uint64_t* src_off, const uint64_t* src_len,
-                     uint32_t n, int level, int codec, const uint64_t* dst_off, CompressPrep* P, uint32_t* status,
+                     uint32_t n, int level, const CodecWord& cw, const uint64_t* dst_off, CompressPrep* P, uint32_t* status,
                      std::string* err) {
   // zstd: the level picks the match finder: three window geometries, then (levels >= 20) the whole-slice long effort;
   // LZ4 has one effort
   const int effort = level <= 2 ? 0 : (level <= 9 ? 1 : (level <= 19 ? 2 : 3));
-  const bool seekable = (codec & kCodecSeekable) != 0;
-  const bool lz4 = (codec & ~kCodecSeekable) == 2;
-  if (seekable && (lz4 || effort == 3)) {  // the long effort reaches up to 8 MiB back, which a one-block frame rules out
-    *err = "seekable frames need the zstd codec at a level <= 19";
-    return -1;
-  }
+  const bool seekable = cw.seekable, lz4 = cw.base == ZN_CODEC_LZ4;
   const uint64_t bsz = lz4 ? cz::kLz4Block : cz::kZstdCBlock;
   std::vector<SliceDesc> sl(n);
   uint64_t total_blocks = 0;
@@ -174,7 +171,7 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
                                                                   : effort == 1 ? ZstdLaunch<cz::WinMid>::kCtasPerSm
                                                                                 : ZstdLaunch<cz::WinHigh>::kCtasPerSm))));
   const size_t small_bytes = (size_t)n * sizeof(SliceDesc) + (size_t)nb * 8 + (size_t)n * 8 + (size_t)n * 4 + 64 +
-                             (seekable ? (size_t)nb * 4 : 0);
+                             (seekable ? (size_t)nb * 4 : 0) + (cw.checksum ? (size_t)n * 4 : 0);
   if (!grow(&cs->tmp, &cs->tmp_cap, std::max<size_t>(1, (size_t)nb * slot)) ||
       !grow((uint8_t**)&cs->small, &cs->small_cap, small_bytes) ||
       (!lz4 && effort < 3 && !grow(&cs->seqs, &cs->seqs_cap, (size_t)grid * wpc * cz::kZstdMaxSeq * 8))) {
@@ -184,6 +181,7 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   *P = CompressPrep();
   P->lz4 = lz4;
   P->seekable = seekable;
+  P->checksum = cw.checksum;
   P->effort = effort;
   P->n = n;
   P->nb = nb;
@@ -195,16 +193,23 @@ int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const u
   P->d_len = (uint64_t*)(((uintptr_t)d_len + 7) & ~(uintptr_t)7);
   P->d_raw = (uint32_t*)(P->d_len + n);
   if (seekable) P->d_xxh = P->d_raw + n;
+  if (cw.checksum) P->d_csum = P->d_raw + n;
   if (cudaMemcpyAsync(P->d_sl, sl.data(), (size_t)n * sizeof(SliceDesc), cudaMemcpyHostToDevice, st) != cudaSuccess) {
     *err = "compress H2D failed";
     return -2;
   }
+  if (cw.checksum && n) P->launches = 1;  // k_slice_xxh
   if (nb && !lz4 && effort == 3) return long_prepare(cs, st, sm_count, sl, P, err);
-  if (nb) P->launches = seekable ? 2 : 1;
+  if (nb) P->launches += seekable ? 2 : 1;
   return 0;
 }
 
 int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, std::string* err) {
+  if (P.checksum && P.n) {
+    const uint32_t grid = std::min<uint32_t>((P.n + kSliceXxhWarps - 1) / kSliceXxhWarps, P.sm_count * 16u);
+    if (P.lz4) k_slice_xxh<32><<<grid, kSliceXxhWarps * 32, 0, st>>>(P.d_sl, P.n, d_src, P.d_csum);
+    else k_slice_xxh<64><<<grid, kSliceXxhWarps * 32, 0, st>>>(P.d_sl, P.n, d_src, P.d_csum);
+  }
   if (!P.nb) return 0;
   if (!P.lz4 && P.effort == 3) {
     const LongUnit* d_units = (const LongUnit*)cs->lunits;
@@ -251,27 +256,27 @@ int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st
 void compress_pack(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, uint8_t* d_dst,
                    uint64_t* d_offsets, bool envelope) {
   if (!P.n) return;
-  k_pack_layout<<<1, kLayoutThreads, 0, st>>>(P.d_sl, P.n, P.d_meta, P.lz4 ? 1u : 0u, P.seekable ? 1u : 0u, envelope ? 1u : 0u, d_dst,
-                                              d_offsets, P.d_raw);
-  if (P.lz4) k_assemble_packed<true><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, nullptr, P.d_raw, d_dst, P.d_len);
-  else k_assemble_packed<false><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, P.d_raw, d_dst, P.d_len);
+  k_pack_layout<<<1, kLayoutThreads, 0, st>>>(P.d_sl, P.n, P.d_meta, P.lz4 ? 1u : 0u, P.seekable ? 1u : 0u, P.checksum ? 1u : 0u,
+                                              envelope ? 1u : 0u, d_dst, d_offsets, P.d_raw);
+  if (P.lz4) k_assemble_packed<true><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, nullptr, P.d_csum, P.d_raw, d_dst, P.d_len);
+  else k_assemble_packed<false><<<P.n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, P.d_csum, P.d_raw, d_dst, P.d_len);
 }
 
 // Compresses n slices resident on the device into frames at d_dst + dst_off[i]; synchronises `st` before returning.
 int compress_run(CompressScratch* cs, cudaStream_t st, int sm_count, const uint8_t* d_src, const uint64_t* src_off,
-                        const uint64_t* src_len, uint32_t n, int level, int codec, uint8_t* d_dst, const uint64_t* dst_off,
+                        const uint64_t* src_len, uint32_t n, int level, const CodecWord& cw, uint8_t* d_dst, const uint64_t* dst_off,
                         const uint64_t* /*dst_cap*/, uint64_t* out_len, uint32_t* status, uint32_t* launches, std::string* err) {
   CompressPrep P;
   *launches = 0;
-  int rc = compress_prepare(cs, st, sm_count, src_off, src_len, n, level, codec, dst_off, &P, status, err);
+  int rc = compress_prepare(cs, st, sm_count, src_off, src_len, n, level, cw, dst_off, &P, status, err);
   if (rc) return rc;
   if (!cs->ev[0]) { cudaEventCreate(&cs->ev[0]); cudaEventCreate(&cs->ev[1]); }
   cudaEventRecord(cs->ev[0], st);
   rc = compress_enqueue(cs, P, st, d_src, err);
   if (rc) return rc;
   *launches = P.launches;
-  if (P.lz4) k_lz4_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, d_dst, P.d_len);
-  else k_zstd_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, d_dst, P.d_len);
+  if (P.lz4) k_lz4_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_csum, d_dst, P.d_len);
+  else k_zstd_assemble<<<n, 256, 0, st>>>(P.d_sl, d_src, cs->tmp, P.d_meta, P.d_xxh, P.d_csum, d_dst, P.d_len);
   (*launches)++;
   cudaEventRecord(cs->ev[1], st);
   if (cudaMemcpyAsync(out_len, P.d_len, (size_t)n * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||

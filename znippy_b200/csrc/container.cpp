@@ -37,6 +37,7 @@
 #include <vector>
 
 #include "../../include/znippy_cuda.h"
+#include "codec_word.h"
 
 namespace {
 constexpr uint64_t kMaxRowBytes = 1ull << 32;  // blobs / slices of 4 GiB or more are unsupported (include/znippy_cuda.h)
@@ -1066,8 +1067,8 @@ struct zn_archive_writer {
   zn_ctx* ctx;
   int fd;
   bool no_skip;
-  int level, codec;       // codec: ZN_CODEC_ZSTD [| ZN_CODEC_SEEKABLE] or ZN_CODEC_LZ4, as zn_compress_batch takes it
-  bool envelope = false;  // ZN_CODEC_ENVELOPE: blobs of compressed rows are ZNB1 envelopes (store-if-incompressible)
+  int level, codec;       // codec: the word without ZN_CODEC_ENVELOPE, as zn_compress_batch takes it
+  zn::CodecWord cw;       // its parts; cw.envelope: blobs of compressed rows are ZNB1 envelopes (store-if-incompressible)
   uint64_t slot_bytes, out_cursor = 0;
   WSlot slots[kSlots];
   WSlot* cur = nullptr;  // the slot being filled
@@ -1151,10 +1152,10 @@ int slot_write(zn_archive_writer* w, WSlot* s) {
     if (r.skip) { payload = s->stage + r.stage_off; m.blob_size = r.len; memcpy(m.checksum, s->s_dig.data() + 32 * si, 32); si++; }
     else {
       payload = s->outb + s->d_off[ci]; m.blob_size = s->c_out[ci]; memcpy(m.checksum, s->c_dig.data() + 32 * ci, 32); ci++;
-      if (w->envelope) {
+      if (w->cw.envelope) {
         // store-if-incompressible (deferred in the reference, TODO_NOW.md:37-38): a frame that did not shrink the slice
         // is dropped for the raw bytes; the row stays `compressed` and the envelope says RAW
-        uint32_t pc = w->codec == ZN_CODEC_LZ4 ? ZN_PAYLOAD_LZ4_FRAME : ZN_PAYLOAD_ZSTD;
+        uint32_t pc = w->cw.base == ZN_CODEC_LZ4 ? ZN_PAYLOAD_LZ4_FRAME : ZN_PAYLOAD_ZSTD;
         if (m.blob_size >= r.len) { pc = ZN_PAYLOAD_RAW; payload = s->stage + r.stage_off; m.blob_size = r.len; }
         hl = zn_envelope_znb1_header(pc, r.len, hdr, sizeof hdr);
       }
@@ -1281,16 +1282,15 @@ uint64_t writer_new_entry(zn_archive_writer* w, const char* relative_path, int h
 extern "C" zn_archive_writer* zn_archive_writer_create(zn_ctx* ctx, const char* output_path, int no_skip, int level, int codec,
                                                        size_t slot_bytes) {
   if (!ctx || !output_path) return nullptr;
-  const bool envelope = (codec & ZN_CODEC_ENVELOPE) != 0;
-  codec &= ~ZN_CODEC_ENVELOPE;
-  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4 && codec != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) return nullptr;
-  if ((codec & ZN_CODEC_SEEKABLE) && level >= 20) return nullptr;
+  zn::CodecWord cw;
+  if (zn::codec_split(codec, level, true, &cw)) return nullptr;
   if (slot_bytes < 2 * kSliceSize) slot_bytes = 2 * kSliceSize;
   const int fd = open(output_path, O_CREAT | O_RDWR | O_TRUNC, 0644);
   if (fd < 0) return nullptr;
   zn_archive_writer* w = new zn_archive_writer();
-  w->ctx = ctx; w->fd = fd; w->no_skip = no_skip != 0; w->level = level; w->codec = codec; w->slot_bytes = slot_bytes;
-  w->envelope = envelope;
+  w->ctx = ctx; w->fd = fd; w->no_skip = no_skip != 0; w->level = level; w->codec = codec & ~ZN_CODEC_ENVELOPE;
+  w->slot_bytes = slot_bytes;
+  w->cw = cw;
   memset(&w->rep, 0, sizeof w->rep);
   for (auto& s : w->slots) {
     s.stage = (uint8_t*)zn_ctx_pinned_alloc(slot_bytes + 4096);
@@ -1354,8 +1354,8 @@ extern "C" int zn_archive_writer_finish(zn_archive_writer* w, zn_compression_rep
       zn_index_writer_metadata(iw, "max_chunks", "128");
       zn_index_writer_metadata(iw, "compression_level", "19");
       zn_index_writer_metadata(iw, "zstd_output_buffer_size", "1048576");
-      if (w->envelope) zn_index_writer_metadata(iw, "znippy_envelope", "ZNB1");  // readers resolve compressed rows through zn_envelope_parse
-      if (w->codec & ZN_CODEC_SEEKABLE) zn_index_writer_metadata(iw, "znippy_seekable", "zstd");  // range reads use the seek tables
+      if (w->cw.envelope) zn_index_writer_metadata(iw, "znippy_envelope", "ZNB1");  // readers resolve compressed rows through zn_envelope_parse
+      if (w->cw.seekable) zn_index_writer_metadata(iw, "znippy_seekable", "zstd");  // range reads use the seek tables
     }
     for (auto& kv : groups) {
       const auto& rows = kv.second;
@@ -1428,8 +1428,9 @@ struct ReadJob {
 extern "C" int zn_archive_compress_dir(zn_ctx* ctx, const char* input_dir, const char* output_path, int no_skip, int level, int codec,
                                        size_t slot_bytes, int io_threads, zn_compression_report* report, char* err, size_t errcap) {
   if (!ctx || !input_dir || !output_path) return ZN_E_ARG;
-  if ((codec & ZN_CODEC_SEEKABLE) && ((codec & ~(ZN_CODEC_SEEKABLE | ZN_CODEC_ENVELOPE)) != ZN_CODEC_ZSTD || level >= 20)) {
-    set_err(err, errcap, "seekable archives need the zstd codec at a level <= 19");
+  zn::CodecWord cw;
+  if (const char* why = zn::codec_split(codec, level, true, &cw)) {
+    set_err(err, errcap, why);
     return ZN_E_ARG;
   }
   std::vector<DirFile> files;

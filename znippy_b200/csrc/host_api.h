@@ -9,6 +9,7 @@
 #include <string>
 #include <vector>
 
+#include "codec_word.h"
 #include "zpipe.cuh"
 
 namespace zn {
@@ -51,7 +52,6 @@ struct CompressScratch {
   }
 };
 void compress_init_attrs();
-constexpr int kCodecSeekable = 0x400;        // ZN_CODEC_SEEKABLE, OR-ed into the codec of the functions below
 size_t compress_bound(size_t n, int codec);  // zn_compress_bound: raw-block fallback makes this exact
 struct SliceDesc;
 // What compress_prepare works out from the slice sizes alone: the effort, the grid, the device descriptors (inside the
@@ -59,6 +59,7 @@ struct SliceDesc;
 struct CompressPrep {
   bool lz4 = false;
   bool seekable = false;  // zstd only, levels <= 19: one frame per block and a seek table (cz::zstd_seek_table)
+  bool checksum = false;  // ZN_CODEC_CHECKSUM: every frame ends in its content checksum
   int effort = 0;
   uint32_t n = 0, nb = 0, grid = 0, sm_count = 0;
   SliceDesc* d_sl = nullptr;   // n slice descriptors
@@ -66,15 +67,16 @@ struct CompressPrep {
   uint64_t* d_len = nullptr;   // n frame lengths
   uint32_t* d_raw = nullptr;   // n RAW decisions of the packed layout
   uint32_t* d_xxh = nullptr;   // seekable: nb block checksums (k_block_xxh); nullptr otherwise
+  uint32_t* d_csum = nullptr;  // checksum: n slice checksums (k_slice_xxh); nullptr otherwise
   std::vector<uint32_t> round_first{0}, round_pos, round_blk0, round_nblk, round_sort_launches;
   uint32_t long_grid = 0;
   size_t sort_temp = 0;
   uint32_t launches = 0;  // kernels compress_enqueue launches
 };
 // Plans a batch: grows `cs` to fit, uploads the descriptors on `st` (dst_off[i]: where slice i's frame goes; nullable
-// for a packed layout, which places the frames on the device).  No kernel runs.
+// for a packed layout, which places the frames on the device).  No kernel runs.  `cw` has passed codec_split.
 int compress_prepare(CompressScratch* cs, cudaStream_t st, int sm_count, const uint64_t* src_off, const uint64_t* src_len,
-                     uint32_t n, int level, int codec, const uint64_t* dst_off, CompressPrep* P, uint32_t* status,
+                     uint32_t n, int level, const CodecWord& cw, const uint64_t* dst_off, CompressPrep* P, uint32_t* status,
                      std::string* err);
 // Enqueues the block kernels of a prepared batch on `st` (P.launches kernels): fills the per-block results.
 int compress_enqueue(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, const uint8_t* d_src, std::string* err);
@@ -84,7 +86,7 @@ void compress_pack(CompressScratch* cs, const CompressPrep& P, cudaStream_t st, 
                    uint64_t* d_offsets, bool envelope);
 // Compresses n slices resident on the device into frames at d_dst + dst_off[i]; synchronises `st` before returning.
 int compress_run(CompressScratch* cs, cudaStream_t st, int sm_count, const uint8_t* d_src, const uint64_t* src_off,
-                 const uint64_t* src_len, uint32_t n, int level, int codec, uint8_t* d_dst, const uint64_t* dst_off,
+                 const uint64_t* src_len, uint32_t n, int level, const CodecWord& cw, uint8_t* d_dst, const uint64_t* dst_off,
                  const uint64_t* dst_cap, uint64_t* out_len, uint32_t* status, uint32_t* launches, std::string* err);
 
 // ---------------------------------------------------------------------------------------------- zpipe_tu.cu

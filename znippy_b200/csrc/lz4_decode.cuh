@@ -4,8 +4,8 @@
 // README.md:10).  Written from the public format descriptions.  Thread 0 walks the token stream of a block and emits
 // sequences {literal offset, ll, ml, distance} into the shared batch; the team executes them with the same
 // cooperative copy engine as the Zstandard path (zstd_decode.cuh: exec_batch).  Linked blocks need nothing special:
-// the whole output of the blob is the window.  Block / content checksums (XXH32) are skipped, not verified; the
-// header checksum byte is verified.
+// the whole output of the blob is the window.  The header checksum byte is verified here; block / content checksums
+// (XXH32) are stepped over and verified where the row's digest is compared (xxh_verify.cuh).
 #pragma once
 #include "zstd_decode.cuh"
 

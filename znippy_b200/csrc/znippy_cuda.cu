@@ -676,7 +676,7 @@ extern "C" int zn_plan_run(zn_plan* p, const uint8_t* d_blobs, uint8_t* d_out, v
     launches++;
   }
   ZN_CUDA(c, cudaEventRecord(p->ev[2], st));
-  // Zstandard content checksums are checked where a row's digest is compared (xxh_verify.cuh)
+  // frame checksums (zstd content, LZ4 block and content) are checked where a row's digest is compared (xxh_verify.cuh)
   const uint8_t* xxh_out = p->n_dec ? d_out : nullptr;
   if (p->n_small) {
     k_b3_tree_small<<<(p->n_small + 127) / 128, 128, 0, st>>>(p->d_blobs, p->d_list_small, p->n_small, p->d_cvs, p->d_digests,
@@ -735,19 +735,19 @@ extern "C" int zn_plan_last_ms(zn_plan* p, float ms[4]) {
 extern "C" zn_plan* zn_plan_compress(zn_ctx* c, uint32_t n, const uint64_t* h_src_off, const uint64_t* h_src_len, int level,
                                      int codec, int digests) {
   if (!c) return nullptr;
-  const int base = codec & ~ZN_CODEC_ENVELOPE;
-  if (base != ZN_CODEC_ZSTD && base != ZN_CODEC_LZ4 && base != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) {
-    c->err = "zn_plan_compress: codec must be ZN_CODEC_ZSTD (optionally | ZN_CODEC_SEEKABLE) or ZN_CODEC_LZ4, optionally | "
-             "ZN_CODEC_ENVELOPE";
+  CodecWord cw;
+  if (const char* why = codec_split(codec, level, true, &cw)) {
+    c->err = std::string("zn_plan_compress: ") + why;
     return nullptr;
   }
+  const int base = codec & ~ZN_CODEC_ENVELOPE;
   if (n && (!h_src_off || !h_src_len)) { c->err = "zn_plan_compress: null size arrays"; return nullptr; }
   cudaSetDevice(c->device);
   zn_plan* p = new zn_plan();
   p->ctx = c;
   p->kind = PLAN_COMPRESS;
   p->n = n;
-  p->envelope = (codec & ZN_CODEC_ENVELOPE) != 0;
+  p->envelope = cw.envelope;
   p->h_status.assign(n, 0);
   for (uint32_t i = 0; i < n; i++) {
     uint8_t hdr[ZN_ENVELOPE_ZNB1_MAX_HEADER];
@@ -755,7 +755,7 @@ extern "C" zn_plan* zn_plan_compress(zn_ctx* c, uint32_t n, const uint64_t* h_sr
                                : compress_bound(h_src_len[i], base);
   }
   std::string err;
-  if (compress_prepare(&p->cs, c->stream, c->sm_count, h_src_off, h_src_len, n, level, base, nullptr, &p->cp, p->h_status.data(),
+  if (compress_prepare(&p->cs, c->stream, c->sm_count, h_src_off, h_src_len, n, level, cw, nullptr, &p->cp, p->h_status.data(),
                        &err) != 0) {
     c->err = "zn_plan_compress: " + err;
     zn_plan_destroy(p);
@@ -1231,9 +1231,9 @@ extern "C" int zn_compress_batch(zn_ctx* c, const uint8_t* src_base, const uint6
                                  uint32_t n, int level, int codec, uint8_t* dst_base, const uint64_t* dst_off,
                                  uint64_t* dst_len_out, uint8_t* digest_out, uint32_t* status) {
   if (!c || (n && (!src_base || !src_off || !src_len || !dst_base || !dst_off || !dst_len_out || !status))) return ZN_E_ARG;
-  if (codec != ZN_CODEC_ZSTD && codec != ZN_CODEC_LZ4 && codec != (ZN_CODEC_ZSTD | ZN_CODEC_SEEKABLE)) return ZN_E_ARG;
-  if ((codec & ZN_CODEC_SEEKABLE) && level >= 20) {
-    c->err = "zn_compress_batch: seekable frames need a zstd level <= 19";
+  CodecWord cw;
+  if (const char* why = codec_split(codec, level, false, &cw)) {
+    c->err = std::string("zn_compress_batch: ") + why;
     return ZN_E_ARG;
   }
   if (n == 0) return ZN_OK;
@@ -1267,7 +1267,7 @@ extern "C" int zn_compress_batch(zn_ctx* c, const uint8_t* src_base, const uint6
   }
   std::vector<uint64_t> out_len(n, 0);
   uint32_t launches = 0;
-  rc = compress_run(&c->cs, c->stream, c->sm_count, c->d_in, Li.dev_off.data(), src_len, n, level, codec, c->d_out, doff.data(),
+  rc = compress_run(&c->cs, c->stream, c->sm_count, c->d_in, Li.dev_off.data(), src_len, n, level, cw, c->d_out, doff.data(),
                     cap.data(), out_len.data(), status, &launches, &c->err);
   c->launches += launches;
   if (rc == ZN_OK) {
